@@ -2,7 +2,7 @@
 """bench.py — polynomial-commitment throughput (BASELINE.json metric: LDE+Merkle commit cells/s; block-proof-shaped
 commit latency in ms).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -24,6 +24,8 @@ barriers and the max over ranks.
 --impl reference: times the CPU restatement only (the reference's Rust prover cannot be built here: DESIGN.md), with every
 host thread, on a bounded row sample of the same workload sized so that W + K steps end within a few minutes.
 B200ZKP_BENCH_CONFIG=5: BASELINE.json configs[4] (2^24 x 256, needs 8 GPUs) with per-rank opening checks.
+--dump-outputs DIR: after the timed steps, what the last one returned (cap, and a fixed sample of coefficients, leaves and
+digests) as float64 .npy files (dump_outputs), so that two builds can be compared output for output on the same input.
 """
 import argparse
 import hashlib
@@ -237,6 +239,30 @@ def xor_all(t):
 def np_xor(a):
     import numpy as np
     return int(np.bitwise_xor.reduce(a.reshape(-1).view(np.uint64)))
+
+
+def dump_indices(sizes, k, rows=4096):
+    """the fixed sample of --dump-outputs: for each name -> length in `sizes`, sorted indices from one seeded generator, first
+    and last included; at most `rows` of them, fewer for wide matrices so that a sampled (rows, k) matrix stays under 24 MB"""
+    import numpy as np
+    rows = max(3, min(rows, (24 << 20) // (16 * k)))
+    rng = np.random.default_rng(20)
+    return {name: np.unique(np.concatenate([[0, size - 1], rng.integers(0, size, rows - 2)])).astype(np.int64)
+            for name, size in sizes.items()}
+
+
+def dump_outputs(path, outputs, index):
+    """--dump-outputs: each uint64 array of `outputs` (numpy or torch int64) as path/<name>.npy in float64, with a last axis of
+    2 holding the low and the high 32 bits of every word (a field element does not fit the 53-bit mantissa, its halves do), and
+    each array of `index` (the rows a sample holds) as float64.  At 2^20 x 135 the files come to 18 MB."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        w = np.ascontiguousarray(a.cpu().numpy() if hasattr(a, "cpu") else a).view(np.uint64)
+        limbs = np.stack([w & np.uint64(0xFFFFFFFF), w >> np.uint64(32)], axis=-1).astype(np.float64)
+        np.save(os.path.join(path, name + ".npy"), limbs)
+    for name, a in index.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def parity_full_single_gpu(torch, np, host_vals, out, n_log, k):
@@ -599,6 +625,22 @@ def run_b200(args):
     ms_step = float(t.item()) / args.steps
     value = cells / (ms_step * 1e-3)
 
+    if args.dump_outputs:
+        if world == 1:
+            idx = dump_indices({"coeffs_index": n, "leaves_index": N, "digests_index": out.digests.shape[0]}, k)
+            at = {name: torch.as_tensor(i, device=dev) for name, i in idx.items()}
+            dump_outputs(args.dump_outputs, {"cap": out.cap, "coeffs": out.coeffs[:, at["coeffs_index"]].t(),
+                                             "leaves": out.lde[:, at["leaves_index"]].t(),
+                                             "digests": out.digests[at["digests_index"]]}, idx)
+        else:
+            # every rank holds its own leaf range and subtree: the sampled leaves are opened through the collective
+            # b200zkp_sharded_rows, and the digests, split over the ranks, are not written
+            idx = dump_indices({"coeffs_index": n, "leaves_index": N}, k)
+            leaves, _ = sh.rows(idx["leaves_index"])
+            if rank == 0:
+                cols = sh.coeffs_all[:k][:, torch.as_tensor(idx["coeffs_index"], device=dev)].t()
+                dump_outputs(args.dump_outputs, {"cap": sh.cap, "coeffs": cols, "leaves": leaves}, idx)
+
     # ---- end to end through the host-buffer API (pinned host input, H2D + commit + cap D2H per step)
     cap_host = torch.empty((1 << CAP_HEIGHT, 4), dtype=torch.int64).pin_memory()
     if world == 1:
@@ -770,7 +812,13 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (cap, sampled coefficients, leaves, digests) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

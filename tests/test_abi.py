@@ -107,3 +107,29 @@ def test_bench_profile_blocks_are_keyed_to_the_kernel_sources():
     json.dumps(blk)
     if "profile" in blk:
         assert 0.5 < blk["profile"]["alu_pipe_busy"] <= 1.0 and len(blk["profile"]["lde_passes"]) == 3
+
+
+def test_bench_dump_outputs_are_exact_and_bounded(tmp_path):
+    """bench.py --dump-outputs: the sample is the same on every call, the float64 limbs give back every uint64 word, and the
+    files of the benchmarked shape stay under 64 MB."""
+    import sys
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    n_log, k = 20, 135
+    N = 1 << (n_log + bench.RATE_BITS)
+    sizes = {"coeffs_index": 1 << n_log, "leaves_index": N, "digests_index": 2 * (N - (1 << bench.CAP_HEIGHT))}
+    idx = bench.dump_indices(sizes, k)
+    again = bench.dump_indices(sizes, k)
+    for name, size in sizes.items():
+        i = idx[name]
+        assert (i == again[name]).all() and i[0] == 0 and i[-1] == size - 1 and (np.diff(i) > 0).all()
+    rows = len(idx["coeffs_index"]) + len(idx["leaves_index"])
+    total = 16 * (rows * k + 4 * len(idx["digests_index"]) + (4 << bench.CAP_HEIGHT)) + 8 * sum(len(i) for i in idx.values())
+    assert total < 64 << 20
+    w = np.array([[0, 1, bench.P - 1], [2**32 - 1, 2**32, 2**64 - 1]], dtype=np.uint64)
+    bench.dump_outputs(str(tmp_path), {"w": w}, {"w_index": np.array([0, 7])})
+    got = np.load(tmp_path / "w.npy")
+    assert got.dtype == np.float64 and got.shape == (2, 3, 2)
+    assert (got[..., 0].astype(np.uint64) + (got[..., 1].astype(np.uint64) << np.uint64(32)) == w).all()
+    assert (np.load(tmp_path / "w_index.npy") == [0, 7]).all()
