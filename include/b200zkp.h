@@ -76,8 +76,6 @@ uint64_t b200zkp_ctx_launch_count(const b200zkp_ctx* ctx);
 enum { B200ZKP_STAGE_INTT = 0, B200ZKP_STAGE_LDE = 1, B200ZKP_STAGE_LEAF_HASH = 2, B200ZKP_STAGE_TREE = 3,
        B200ZKP_N_STAGES = 4 };
 int b200zkp_ctx_set_timing(b200zkp_ctx* ctx, int enabled);
-/* LDE / leaf-hash overlap on two streams (off by default: no gain measured on B200); 0 = strictly sequential stages */
-int b200zkp_ctx_set_overlap(b200zkp_ctx* ctx, int enabled);
 int b200zkp_ctx_stage_ms(b200zkp_ctx* ctx, double ms[B200ZKP_N_STAGES], uint32_t counts[B200ZKP_N_STAGES]);
 /* pinned host memory for callers that want full-speed H2D/D2H */
 int b200zkp_host_alloc(size_t bytes, void** out);

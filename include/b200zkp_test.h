@@ -23,6 +23,9 @@ int b200zkp_field_op(b200zkp_ctx* ctx, int op, const uint64_t* a, const uint64_t
  *       16 three-input IADD3 with a uniform operand, 17 alternating three-input IADD3/IMAD,
  *       18 IMAD.WIDE : IMAD : LOP3 : IADD3 = 1 : 2 : 2 : 3, 19 IMAD.WIDE : LOP3 : IMAD = 1 : 2 : 1 */
 int b200zkp_int_pipe_bench(b200zkp_ctx* ctx, int kind, uint32_t iters, double* out_gips);
+/* device memory of the ctx's buffer pool: *live = bytes handed out and not yet returned (scratch of a call in flight and the
+ * buffers of live handles), *cached = bytes kept for reuse (b200zkp_ctx_trim returns them to the driver).  A leak check. */
+int b200zkp_ctx_buffer_bytes(b200zkp_ctx* ctx, uint64_t* live, uint64_t* cached);
 
 #ifdef __cplusplus
 }

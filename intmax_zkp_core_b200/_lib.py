@@ -86,7 +86,6 @@ _SIGS = {
     "b200zkp_ctx_launch_count": (C.c_uint64, [C.c_void_p]),
     "b200zkp_ctx_trim": (C.c_int, [C.c_void_p]),
     "b200zkp_ctx_set_pool_limit": (C.c_int, [C.c_void_p, C.c_uint64]),
-    "b200zkp_ctx_set_overlap": (C.c_int, [C.c_void_p, C.c_int]),
     "b200zkp_ctx_set_timing": (C.c_int, [C.c_void_p, C.c_int]),
     "b200zkp_ctx_stage_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), u32p]),
     "b200zkp_host_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p)]),
@@ -168,6 +167,7 @@ _SIGS = {
     "b200zkp_sharded_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "b200zkp_field_op": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "b200zkp_int_pipe_bench": (C.c_int, [C.c_void_p, C.c_int, C.c_uint32, C.POINTER(C.c_double)]),
+    "b200zkp_ctx_buffer_bytes": (C.c_int, [C.c_void_p, u64p, u64p]),
 }
 
 EXPORTED_SYMBOLS = tuple(_SIGS)

@@ -10,7 +10,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
+#include <optional>
 #include <string>
 #include <vector>
 
@@ -66,13 +68,13 @@ struct b200zkp_ctx {
     void* mailbox = nullptr;
     void* mailbox_dev = nullptr;
     u64* round_add = nullptr;                           // poseidon_tables::ROUND_ADD in global memory (latency-form kernels)
-    std::multimap<size_t, void*> pool;                  // cached device allocations (dev_release), at most pool_max_bytes
+    std::multimap<size_t, void*> pool;                  // cached device allocations (DevBuf::reset), at most pool_max_bytes
     size_t pool_bytes = 0;
+    size_t live_bytes = 0;                              // handed out by DevBuf::alloc and not yet returned (b200zkp_ctx_buffer_bytes)
     size_t pool_max_bytes = (size_t)16 << 30;         // reset to 1/8 of the device memory in ctx_create
     std::vector<void*> table_allocs;
-    // second, higher-priority stream: coset transforms run here while finished blocks are hashed on `stream`
+    // second, higher-priority stream: host uploads and copy-back beside the main stream (ensure_stream2)
     cudaStream_t stream2 = nullptr;
-    bool overlap = false;   // measured on B200: no gain (both kernels are issue/I-cache limited when co-resident)
     std::vector<cudaEvent_t> sync_events;
     // optional per-stage timing (bench.py): CUDA event pairs recorded on the ctx stream
     bool timing = false;
@@ -108,19 +110,12 @@ struct Guard {
     ~Guard() { c->mu.unlock(); }
 };
 
-struct b200zkp_batch {
-    b200zkp_ctx* ctx;
-    u32 n_log, k, rate_bits, cap_height, salt;
-    u64 *coeffs, *lde, *digests, *cap;
-    size_t coeffs_b, lde_b, digests_b, cap_b;
-};
-
-struct b200zkp_tree {
-    b200zkp_ctx* ctx;
-    u64 n_leaves;
-    u32 leaf_len, cap_height;
-    u64 *digests, *cap;
-    size_t digests_b, cap_b;
+// Sets ctx->stream for the life of the scope and puts the previous stream back on every exit.
+struct StreamScope {
+    b200zkp_ctx* c;
+    cudaStream_t saved;
+    StreamScope(b200zkp_ctx* ctx, cudaStream_t s) : c(ctx), saved(ctx->stream) { c->stream = s; }
+    ~StreamScope() { c->stream = saved; }
 };
 
 #define CUDA_TRY(ctx, expr)                                                                   \
@@ -141,36 +136,122 @@ static void pool_drop(b200zkp_ctx* ctx) {
     ctx->pool_bytes = 0;
 }
 
-static int dev_alloc(b200zkp_ctx* ctx, size_t bytes, void** out) {
-    *out = nullptr;
-    if (bytes == 0) return 0;
-    auto it = ctx->pool.find(bytes);
-    if (it != ctx->pool.end()) { *out = it->second; ctx->pool_bytes -= it->first; ctx->pool.erase(it); return 0; }
-    cudaError_t e = cudaMalloc(out, bytes);
-    if (e == cudaErrorMemoryAllocation) {
-        // drop the cache and retry once
-        (void)cudaGetLastError();
-        pool_drop(ctx);
-        e = cudaMalloc(out, bytes);
+// One pooled device allocation, returned to the ctx's cache when its owner goes away; take the ctx lock around both.
+// A returned buffer may be handed to later work on ctx->stream without a synchronisation, so a buffer that another stream
+// touched (stream2, the communicator's side or hash stream, NCCL) must have that stream drained or joined into ctx->stream
+// before its owner is destroyed.
+class DevBuf {
+  public:
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : ctx_(o.ctx_), p_(o.p_), bytes_(o.bytes_) { o.p_ = nullptr; o.bytes_ = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) { reset(); ctx_ = o.ctx_; p_ = o.p_; bytes_ = o.bytes_; o.p_ = nullptr; o.bytes_ = 0; }
+        return *this;
     }
-    if (e != cudaSuccess) {
-        ctx->err = std::string("cudaMalloc: ") + cudaGetErrorString(e);
+    ~DevBuf() { reset(); }
+
+    u64* get() const { return (u64*)p_; }
+    size_t bytes() const { return bytes_; }
+
+    // 0 bytes: nullptr and success
+    int alloc(b200zkp_ctx* ctx, size_t bytes) {
+        reset();
+        ctx_ = ctx;
+        if (bytes == 0) return 0;
+        void* p = nullptr;
+        auto it = ctx->pool.find(bytes);
+        if (it != ctx->pool.end()) {
+            p = it->second; ctx->pool_bytes -= it->first; ctx->pool.erase(it);
+        } else {
+            cudaError_t e = cudaMalloc(&p, bytes);
+            if (e == cudaErrorMemoryAllocation) {
+                // drop the cache and retry once
+                (void)cudaGetLastError();
+                pool_drop(ctx);
+                e = cudaMalloc(&p, bytes);
+            }
+            if (e != cudaSuccess) {
+                ctx->err = std::string("cudaMalloc: ") + cudaGetErrorString(e);
+                (void)cudaGetLastError();
+                return e == cudaErrorMemoryAllocation ? B200ZKP_ERR_OOM : B200ZKP_ERR_CUDA;
+            }
+        }
+        p_ = p; bytes_ = bytes;
+        ctx->live_bytes += bytes;
+        return 0;
+    }
+    // grows only (the contents are not kept)
+    int ensure(b200zkp_ctx* ctx, size_t bytes) { return bytes_ >= bytes ? 0 : alloc(ctx, bytes); }
+
+    void reset() {
+        if (!p_) return;
+        ctx_->live_bytes -= bytes_;
+        // cached for the next request of the same size; an opening proof cycles through ~40 distinct sizes.  The cache is
+        // capped by bytes so that a freed 2^20 x 135 batch (10.7 GB) goes back to the driver instead of starving torch or a
+        // second ctx on the same GPU; b200zkp_ctx_trim empties it on request
+        if (ctx_->pool.size() < 256 && ctx_->pool_bytes + bytes_ <= ctx_->pool_max_bytes) {
+            ctx_->pool.emplace(bytes_, p_);
+            ctx_->pool_bytes += bytes_;
+        } else {
+            cudaFree(p_);    // (cudaFree synchronises the device: pending work on the buffer has finished when it returns)
+        }
+        p_ = nullptr; bytes_ = 0;
+    }
+
+  private:
+    b200zkp_ctx* ctx_ = nullptr;
+    void* p_ = nullptr;
+    size_t bytes_ = 0;
+};
+
+struct b200zkp_batch {
+    b200zkp_ctx* ctx;
+    u32 n_log, k, rate_bits, cap_height, salt;
+    DevBuf coeffs, lde, digests, cap;
+};
+
+struct b200zkp_tree {
+    b200zkp_ctx* ctx;
+    u64 n_leaves;
+    u32 leaf_len, cap_height;
+    DevBuf digests, cap;
+};
+
+static int d2h(b200zkp_ctx* ctx, void* dst, const void* src, size_t bytes) {
+    if (!bytes) return 0;
+    CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+static int h2d(b200zkp_ctx* ctx, void* dst, const void* src, size_t bytes) {
+    if (!bytes) return 0;
+    CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+// the second stream of the ctx, created on first use at the highest priority
+static int ensure_stream2(b200zkp_ctx* ctx) {
+    if (ctx->stream2) return 0;
+    int lo = 0, hi = 0;
+    if (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess ||
+        cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, hi) != cudaSuccess) {
         (void)cudaGetLastError();
-        return e == cudaErrorMemoryAllocation ? B200ZKP_ERR_OOM : B200ZKP_ERR_CUDA;
+        ctx->stream2 = nullptr;
+        ctx->err = "cannot create the copy stream";
+        return B200ZKP_ERR_CUDA;
     }
     return 0;
 }
-static void dev_release(b200zkp_ctx* ctx, void* p, size_t bytes) {
-    if (!p) return;
-    // cached for the next request of the same size (stream order makes reuse on the same ctx safe); an opening proof
-    // cycles through ~40 distinct sizes.  The cache is capped by bytes so that a freed 2^20 x 135 batch (10.7 GB) goes back
-    // to the driver instead of starving torch or a second ctx on the same GPU; b200zkp_ctx_trim empties it on request
-    if (ctx->pool.size() < 256 && ctx->pool_bytes + bytes <= ctx->pool_max_bytes) {
-        ctx->pool.emplace(bytes, p);
-        ctx->pool_bytes += bytes;
-    } else {
-        cudaFree(p);    // (cudaFree synchronises the device: pending work on the buffer has finished when it returns)
-    }
+
+// *lg = log2(n); false unless n is a power of two
+static bool log2_exact(u64 n, u32* lg) {
+    if (n == 0 || (n & (n - 1))) return false;
+    u32 l = 0;
+    while (((u64)1 << l) < n) l++;
+    *lg = l;
+    return true;
 }
 
 static int upload(b200zkp_ctx* ctx, const std::vector<u64>& h, u64** d) {
@@ -386,12 +467,12 @@ static int launch_ct_b(b200zkp_ctx* ctx, int kind, const ntc::PassParams& p, u64
 static int run_ct_plan(b200zkp_ctx* ctx, ntc::Plan& plan, cudaStream_t later_stream = nullptr, cudaEvent_t first_done = nullptr,
                        u32 pull_ctas_per_sm = 4) {
     cudaStream_t const first_stream = ctx->stream;
-    struct Restore { b200zkp_ctx* c; cudaStream_t s; ~Restore() { c->stream = s; } } restore{ctx, first_stream};
+    std::optional<StreamScope> later;
     for (u32 pi = 0; pi < plan.n_passes; pi++) {
         if (pi == 1 && later_stream && later_stream != first_stream) {
             CUDA_TRY(ctx, cudaEventRecord(first_done, first_stream));
             CUDA_TRY(ctx, cudaStreamWaitEvent(later_stream, first_done, 0));
-            ctx->stream = later_stream;
+            later.emplace(ctx, later_stream);
         }
         ntc::PassParams& p = plan.pass[pi];
         const u32 B = plan.bits[pi];
@@ -607,10 +688,11 @@ extern "C" int b200zkp_ctx_trim(b200zkp_ctx* ctx) {
     return 0;
 }
 
-extern "C" int b200zkp_ctx_set_overlap(b200zkp_ctx* ctx, int enabled) {
-    if (!ctx) return B200ZKP_ERR_BAD_ARG;
+extern "C" int b200zkp_ctx_buffer_bytes(b200zkp_ctx* ctx, uint64_t* live, uint64_t* cached) {
+    if (!ctx || !live || !cached) return B200ZKP_ERR_BAD_ARG;
     Guard g(ctx);
-    ctx->overlap = enabled != 0;
+    *live = ctx->live_bytes;
+    *cached = ctx->pool_bytes;
     return 0;
 }
 
@@ -762,9 +844,8 @@ extern "C" int b200zkp_dev_salt(b200zkp_ctx* ctx, const uint64_t* salt, uint64_t
 
 static int merkle_shape(b200zkp_ctx* ctx, u64 n_leaves, u32 cap_height, const void* leaves, const void* digests, const void* cap,
                         merkle::TreeShape* shape) {
-    if (n_leaves == 0 || (n_leaves & (n_leaves - 1))) BAD(ctx, "number of leaves must be a power of two");
     u32 lg = 0;
-    while (((u64)1 << lg) < n_leaves) lg++;
+    if (!log2_exact(n_leaves, &lg)) BAD(ctx, "number of leaves must be a power of two");
     if (cap_height > lg) BAD(ctx, "cap_height exceeds log2(number of leaves)");
     if (!leaves || !cap) BAD(ctx, "null buffer");
     shape->sub_log = lg - cap_height;
@@ -848,53 +929,16 @@ static int get_sync_event(b200zkp_ctx* ctx, size_t i, cudaEvent_t* out) {
     return 0;
 }
 
-// Coset LDE of leaf blocks [b0, b1) + Merkle forest over those leaves, software-pipelined: the transforms of block b+1
-// (ALU-pipe bound) run on a second stream while block b is hashed (multiplier bound) on the main stream.
+// Coset LDE of leaf blocks [b0, b1) + Merkle forest over those leaves
 static int dev_lde_merkle_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 coeff_stride, u64* lde, u64 lde_stride, u32 n_log,
                                  u32 k, u32 rate_bits, u32 b0, u32 b1, u32 leaf_len, u32 cap_height, u64* digests, u64* cap) {
     if (rate_bits > 8 || n_log + rate_bits > 32) BAD(ctx, "rate_bits / n_log out of range");
     if (b0 >= b1 || b1 > (1u << rate_bits)) BAD(ctx, "bad coset block range");
-    u64 n = (u64)1 << n_log;
     u64 n_leaves = (u64)(b1 - b0) << n_log;
     merkle::TreeShape shape;
     TRY(merkle_shape(ctx, n_leaves, cap_height, lde, digests, cap, &shape));
-    if (!ctx->overlap || b1 - b0 < 2) {
-        TRY(dev_lde_locked(ctx, coeffs, coeff_stride, lde, lde_stride, n_log, k, rate_bits, b0, b1));
-        TRY(launch_leaf_hash(ctx, lde, 1, lde_stride, leaf_len, 0, n_leaves, shape, digests, cap));
-        return launch_tree_levels(ctx, n_leaves, shape, digests, cap);
-    }
-    if (!ctx->stream2) {
-        int lo = 0, hi = 0;
-        CUDA_TRY(ctx, cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CUDA_TRY(ctx, cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, hi));
-    }
-    const u64* cs = nullptr;
-    TRY(get_coset_scale(ctx, n_log, rate_bits, &cs));          // (table build, if any, happens on the main stream)
-    b200zkp_ctx::Images im;
-    TRY(get_twiddle_images(ctx, n_log, 0, true, &im));
-    cudaStream_t main_stream = ctx->stream;
-    cudaEvent_t e0;
-    TRY(get_sync_event(ctx, 0, &e0));
-    CUDA_TRY(ctx, cudaEventRecord(e0, main_stream));
-    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, e0, 0));   // coefficients (and tables) are ready
-    int rc = 0;
-    for (u32 b = b0; b < b1 && !rc; b++) {
-        u64 off = (u64)(b - b0) << n_log;
-        ctx->stream = ctx->stream2;
-        {
-            StageTimer tm(ctx, B200ZKP_STAGE_LDE);
-            rc = run_transform(ctx, coeffs, coeff_stride, lde + off, lde_stride, nullptr, n_log, k, /*dir=*/0, /*bitrev_out=*/true,
-                               cs + (u64)b * n, n, /*inverse_scale=*/false, /*canon_in=*/true, 1, n);
-        }
-        cudaEvent_t eb = nullptr;
-        if (!rc) rc = get_sync_event(ctx, 1 + (b - b0), &eb);
-        if (!rc && cudaEventRecord(eb, ctx->stream2) != cudaSuccess) rc = B200ZKP_ERR_CUDA;
-        ctx->stream = main_stream;
-        if (!rc && cudaStreamWaitEvent(main_stream, eb, 0) != cudaSuccess) rc = B200ZKP_ERR_CUDA;
-        if (!rc) rc = launch_leaf_hash(ctx, lde, 1, lde_stride, leaf_len, off, n, shape, digests, cap);
-    }
-    ctx->stream = main_stream;
-    if (rc) { if (rc == B200ZKP_ERR_CUDA) ctx->err = "stream/event error in the LDE/hash pipeline"; (void)cudaGetLastError(); return rc; }
+    TRY(dev_lde_locked(ctx, coeffs, coeff_stride, lde, lde_stride, n_log, k, rate_bits, b0, b1));
+    TRY(launch_leaf_hash(ctx, lde, 1, lde_stride, leaf_len, 0, n_leaves, shape, digests, cap));
     return launch_tree_levels(ctx, n_leaves, shape, digests, cap);
 }
 
@@ -958,14 +1002,6 @@ extern "C" int b200zkp_dev_transpose_to_rows(b200zkp_ctx* ctx, const uint64_t* c
 }
 
 // ------------------------------------------------------------------------------------------------ PolynomialBatch
-static void batch_release(b200zkp_batch* b) {
-    dev_release(b->ctx, b->coeffs, b->coeffs_b);
-    dev_release(b->ctx, b->lde, b->lde_b);
-    dev_release(b->ctx, b->digests, b->digests_b);
-    dev_release(b->ctx, b->cap, b->cap_b);
-    delete b;
-}
-
 // host destinations of a copy-back commit (any may be null)
 struct CopyBack {
     u64* coeffs = nullptr;   // k * n
@@ -984,119 +1020,91 @@ static int commit_host(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log
     if (!in) BAD(ctx, "null input");
     u64 n = (u64)1 << n_log, N = n << rate_bits;
     u32 row = k + (salt ? B200ZKP_SALT_SIZE : 0);
-    b200zkp_batch* b = new (std::nothrow) b200zkp_batch();
+    std::unique_ptr<b200zkp_batch> b(new (std::nothrow) b200zkp_batch());
     if (!b) return B200ZKP_ERR_OOM;
     b->ctx = ctx; b->n_log = n_log; b->k = k; b->rate_bits = rate_bits; b->cap_height = cap_height;
     b->salt = salt ? B200ZKP_SALT_SIZE : 0;
-    b->coeffs_b = (size_t)k * n * 8;
-    b->lde_b = (size_t)row * N * 8;
-    b->digests_b = (size_t)2 * (N - ((u64)1 << cap_height)) * 32;
-    b->cap_b = ((size_t)32) << cap_height;
-    int rc = 0;
-    void* d_in = nullptr; size_t in_b = (size_t)k * n * 8;
-    void* d_salt = nullptr; size_t salt_b = salt ? (size_t)B200ZKP_SALT_SIZE * N * 8 : 0;
-    if ((rc = dev_alloc(ctx, b->coeffs_b, (void**)&b->coeffs)) || (rc = dev_alloc(ctx, b->lde_b, (void**)&b->lde)) ||
-        (rc = dev_alloc(ctx, b->digests_b, (void**)&b->digests)) || (rc = dev_alloc(ctx, b->cap_b, (void**)&b->cap)) ||
-        (rc = dev_alloc(ctx, in_b, &d_in)) || (rc = dev_alloc(ctx, salt_b, &d_salt))) {
-        dev_release(ctx, d_in, in_b); dev_release(ctx, d_salt, salt_b);
-        batch_release(b);
-        return rc;
-    }
-    auto fail = [&](int code) {
-        cudaStreamSynchronize(ctx->stream);
-        if (ctx->stream2) cudaStreamSynchronize(ctx->stream2);   // nothing may still be writing the buffers we recycle
-        (void)cudaGetLastError();
-        dev_release(ctx, d_in, in_b); dev_release(ctx, d_salt, salt_b); batch_release(b); return code;
-    };
+    DevBuf d_in, d_salt, stage;
+    TRY(b->coeffs.alloc(ctx, (size_t)k * n * 8));
+    TRY(b->lde.alloc(ctx, (size_t)row * N * 8));
+    TRY(b->digests.alloc(ctx, (size_t)2 * (N - ((u64)1 << cap_height)) * 32));
+    TRY(b->cap.alloc(ctx, ((size_t)32) << cap_height));
+    TRY(d_in.alloc(ctx, (size_t)k * n * 8));
+    TRY(d_salt.alloc(ctx, salt ? (size_t)B200ZKP_SALT_SIZE * N * 8 : 0));
+    // declared after the buffers, so it runs before they go back to the pool on every exit: nothing may still be writing them
+    struct Drain {
+        b200zkp_ctx* c;
+        ~Drain() { cudaStreamSynchronize(c->stream); if (c->stream2) cudaStreamSynchronize(c->stream2); (void)cudaGetLastError(); }
+    } drain{ctx};
     // Column-chunked upload pipeline: chunk c+1 crosses PCIe on the copy stream while chunk c is inverse-transformed
     // and extended on the main stream (columns are independent until the leaf hash), so the 8nk-byte H2D hides behind
     // the transforms when the caller's buffer is pinned.
-    if (!ctx->stream2) {
-        int lo = 0, hi = 0;
-        if (cudaDeviceGetStreamPriorityRange(&lo, &hi) != cudaSuccess ||
-            cudaStreamCreateWithPriority(&ctx->stream2, cudaStreamNonBlocking, hi) != cudaSuccess) {
-            (void)cudaGetLastError();
-            ctx->err = "cannot create the copy stream";
-            return fail(B200ZKP_ERR_CUDA);
-        }
-    }
+    TRY(ensure_stream2(ctx));
     cudaError_t e = cudaSuccess;
-    const u32 n_chunks = (k >= 16 && in_b >= ((size_t)64 << 20)) ? 8 : 1;
+    const u32 n_chunks = (k >= 16 && d_in.bytes() >= ((size_t)64 << 20)) ? 8 : 1;
     const u32 per = (k + n_chunks - 1) / n_chunks;
     cudaEvent_t e_free;
-    if ((rc = get_sync_event(ctx, 0, &e_free))) return fail(rc);
+    TRY(get_sync_event(ctx, 0, &e_free));
     // d_in / lde may be recycled buffers still in use by earlier work on the main stream
     if (cudaEventRecord(e_free, ctx->stream) != cudaSuccess || cudaStreamWaitEvent(ctx->stream2, e_free, 0) != cudaSuccess) {
-        (void)cudaGetLastError(); ctx->err = "event error"; return fail(B200ZKP_ERR_CUDA);
+        (void)cudaGetLastError(); ctx->err = "event error"; return B200ZKP_ERR_CUDA;
     }
-    if (salt) e = cudaMemcpyAsync(d_salt, salt, salt_b, cudaMemcpyHostToDevice, ctx->stream2);
+    if (salt) e = cudaMemcpyAsync(d_salt.get(), salt, d_salt.bytes(), cudaMemcpyHostToDevice, ctx->stream2);
     std::vector<cudaEvent_t> up(n_chunks);
     for (u32 c = 0; c < n_chunks && e == cudaSuccess; c++) {
         u32 c0 = std::min(k, c * per), c1 = std::min(k, (c + 1) * per);
-        if ((rc = get_sync_event(ctx, 1 + c, &up[c]))) return fail(rc);
-        if (c1 > c0) e = cudaMemcpyAsync((u64*)d_in + (u64)c0 * n, in + (u64)c0 * n, (size_t)(c1 - c0) * n * 8, cudaMemcpyHostToDevice, ctx->stream2);
+        TRY(get_sync_event(ctx, 1 + c, &up[c]));
+        if (c1 > c0) e = cudaMemcpyAsync(d_in.get() + (u64)c0 * n, in + (u64)c0 * n, (size_t)(c1 - c0) * n * 8, cudaMemcpyHostToDevice, ctx->stream2);
         if (e == cudaSuccess) e = cudaEventRecord(up[c], ctx->stream2);
     }
-    if (e != cudaSuccess) { ctx->err = std::string("H2D: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return fail(B200ZKP_ERR_CUDA); }
+    if (e != cudaSuccess) { ctx->err = std::string("H2D: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
     for (u32 c = 0; c < n_chunks; c++) {
         u32 c0 = std::min(k, c * per), c1 = std::min(k, (c + 1) * per);
-        if (cudaStreamWaitEvent(ctx->stream, up[c], 0) != cudaSuccess) { (void)cudaGetLastError(); ctx->err = "event error"; return fail(B200ZKP_ERR_CUDA); }
+        if (cudaStreamWaitEvent(ctx->stream, up[c], 0) != cudaSuccess) { (void)cudaGetLastError(); ctx->err = "event error"; return B200ZKP_ERR_CUDA; }
         if (c1 == c0) continue;
-        const u64* src = (const u64*)d_in + (u64)c0 * n;
-        u64* cf = b->coeffs + (u64)c0 * n;
-        u64* ld = b->lde + (u64)c0 * N;
-        if (is_coeffs) rc = launch_canon_copy(ctx, src, cf, (u64)(c1 - c0) * n);
-        else rc = dev_intt_locked(ctx, src, n, cf, n, /*scratch=*/ld, n_log, c1 - c0);     // this chunk's LDE columns are still free
-        if (!rc && cb && cb->coeffs) {
+        const u64* src = d_in.get() + (u64)c0 * n;
+        u64* cf = b->coeffs.get() + (u64)c0 * n;
+        u64* ld = b->lde.get() + (u64)c0 * N;
+        if (is_coeffs) TRY(launch_canon_copy(ctx, src, cf, (u64)(c1 - c0) * n));
+        else TRY(dev_intt_locked(ctx, src, n, cf, n, /*scratch=*/ld, n_log, c1 - c0));     // this chunk's LDE columns are still free
+        if (cb && cb->coeffs) {
             // copy-back: this chunk's coefficients go home while the later chunks are still being transformed
             cudaEvent_t e_cf;
-            if ((rc = get_sync_event(ctx, 2 + n_chunks + c, &e_cf))) return fail(rc);
+            TRY(get_sync_event(ctx, 2 + n_chunks + c, &e_cf));
             e = cudaEventRecord(e_cf, ctx->stream);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream2, e_cf, 0);
             if (e == cudaSuccess) e = cudaMemcpyAsync(cb->coeffs + (u64)c0 * n, cf, (size_t)(c1 - c0) * n * 8, cudaMemcpyDeviceToHost, ctx->stream2);
-            if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return fail(B200ZKP_ERR_CUDA); }
+            if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
         }
-        if (!rc) rc = dev_lde_locked(ctx, cf, n, ld, N, n_log, c1 - c0, rate_bits, 0, 1u << rate_bits);
-        if (rc) return fail(rc);
+        TRY(dev_lde_locked(ctx, cf, n, ld, N, n_log, c1 - c0, rate_bits, 0, 1u << rate_bits));
     }
-    if (salt) rc = dev_salt_locked(ctx, (const u64*)d_salt, b->lde + (u64)k * N, N, n_log, rate_bits, 0, 1u << rate_bits);
-    if (rc) return fail(rc);
+    if (salt) TRY(dev_salt_locked(ctx, d_salt.get(), b->lde.get() + (u64)k * N, N, n_log, rate_bits, 0, 1u << rate_bits));
     // Copy-back (strict drop-in) mode: coefficients and row-major leaves leave the device on the copy stream while the
     // main stream hashes — the 8N(k+salt)-byte D2H (PCIe bound) overlaps the leaf hash instead of following it.
-    void* stage = nullptr; size_t stage_b = 0;
     if (cb && (cb->coeffs || cb->leaves)) {
         cudaEvent_t e_lde;
-        if ((rc = get_sync_event(ctx, 1 + n_chunks, &e_lde))) return fail(rc);
+        TRY(get_sync_event(ctx, 1 + n_chunks, &e_lde));
         e = cudaEventRecord(e_lde, ctx->stream);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream2, e_lde, 0);
         if (e == cudaSuccess && cb->leaves) {
             u64 chunk_rows = std::min<u64>(N, std::max<u64>(1, ((u64)256 << 20) / ((u64)row * 8)));
-            stage_b = (size_t)chunk_rows * row * 8;
-            if ((rc = dev_alloc(ctx, stage_b, &stage))) return fail(rc);
-            cudaStream_t main_stream = ctx->stream;
-            ctx->stream = ctx->stream2;     // transposes are issued on the copy stream (same order as their D2H)
-            for (u64 r0 = 0; r0 < N && !rc && e == cudaSuccess; r0 += chunk_rows) {
+            TRY(stage.alloc(ctx, (size_t)chunk_rows * row * 8));
+            StreamScope on_copy(ctx, ctx->stream2);     // transposes are issued on the copy stream (same order as their D2H)
+            for (u64 r0 = 0; r0 < N && e == cudaSuccess; r0 += chunk_rows) {
                 u64 nr = std::min(chunk_rows, N - r0);
-                rc = dev_transpose_rows_locked(ctx, b->lde, N, row, r0, nr, (u64*)stage);
-                if (!rc) e = cudaMemcpyAsync(cb->leaves + r0 * row, stage, (size_t)nr * row * 8, cudaMemcpyDeviceToHost, ctx->stream2);
+                TRY(dev_transpose_rows_locked(ctx, b->lde.get(), N, row, r0, nr, stage.get()));
+                e = cudaMemcpyAsync(cb->leaves + r0 * row, stage.get(), (size_t)nr * row * 8, cudaMemcpyDeviceToHost, ctx->stream2);
             }
-            ctx->stream = main_stream;
-            if (rc) { dev_release(ctx, stage, stage_b); return fail(rc); }
         }
-        if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); dev_release(ctx, stage, stage_b); return fail(B200ZKP_ERR_CUDA); }
+        if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
     }
-    rc = dev_merkle_locked(ctx, b->lde, /*row_stride=*/1, /*col_stride=*/N, row, N, cap_height, b->digests, b->cap);
-    if (rc) { dev_release(ctx, stage, stage_b); return fail(rc); }
-    if (cb && cb->digests && b->digests_b) e = cudaMemcpyAsync(cb->digests, b->digests, b->digests_b, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && cb && cb->cap) e = cudaMemcpyAsync(cb->cap, b->cap, b->cap_b, cudaMemcpyDeviceToHost, ctx->stream);
+    TRY(dev_merkle_locked(ctx, b->lde.get(), /*row_stride=*/1, /*col_stride=*/N, row, N, cap_height, b->digests.get(), b->cap.get()));
+    if (cb && cb->digests && b->digests.bytes()) e = cudaMemcpyAsync(cb->digests, b->digests.get(), b->digests.bytes(), cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && cb && cb->cap) e = cudaMemcpyAsync(cb->cap, b->cap.get(), b->cap.bytes(), cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream2);
-    dev_release(ctx, stage, stage_b);
-    if (e != cudaSuccess) { ctx->err = std::string("commit: ") + cudaGetErrorString(e); return fail(B200ZKP_ERR_CUDA); }
-    dev_release(ctx, d_in, in_b);
-    dev_release(ctx, d_salt, salt_b);
-    if (out) *out = b;
-    else batch_release(b);
+    if (e != cudaSuccess) { ctx->err = std::string("commit: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    if (out) *out = b.release();
     return 0;
 }
 
@@ -1129,7 +1137,7 @@ extern "C" void b200zkp_batch_free(b200zkp_batch* b) {
     if (!b) return;
     Guard g(b->ctx);
     cudaStreamSynchronize(b->ctx->stream);
-    batch_release(b);
+    delete b;
 }
 
 extern "C" int b200zkp_batch_shape(const b200zkp_batch* b, uint32_t shape[5]) {
@@ -1138,33 +1146,21 @@ extern "C" int b200zkp_batch_shape(const b200zkp_batch* b, uint32_t shape[5]) {
     return 0;
 }
 
-static int d2h(b200zkp_ctx* ctx, void* dst, const void* src, size_t bytes) {
-    if (!bytes) return 0;
-    CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-    return 0;
-}
-static int h2d(b200zkp_ctx* ctx, void* dst, const void* src, size_t bytes) {
-    if (!bytes) return 0;
-    CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    return 0;
-}
-
 extern "C" int b200zkp_batch_cap(b200zkp_batch* b, uint64_t* out) {
     if (!b || !out) return B200ZKP_ERR_BAD_ARG;
     Guard g(b->ctx);
-    return d2h(b->ctx, out, b->cap, b->cap_b);
+    return d2h(b->ctx, out, b->cap.get(), b->cap.bytes());
 }
 extern "C" int b200zkp_batch_coeffs(b200zkp_batch* b, uint64_t* out) {
     if (!b || !out) return B200ZKP_ERR_BAD_ARG;
     Guard g(b->ctx);
-    return d2h(b->ctx, out, b->coeffs, b->coeffs_b);
+    return d2h(b->ctx, out, b->coeffs.get(), b->coeffs.bytes());
 }
 extern "C" int b200zkp_batch_digests(b200zkp_batch* b, uint64_t* out) {
     if (!b) return B200ZKP_ERR_BAD_ARG;
     Guard g(b->ctx);
-    if (b->digests_b && !out) BAD(b->ctx, "null out");
-    return d2h(b->ctx, out, b->digests, b->digests_b);
+    if (b->digests.bytes() && !out) BAD(b->ctx, "null out");
+    return d2h(b->ctx, out, b->digests.get(), b->digests.bytes());
 }
 
 // leaves leave the device row-major: transpose in chunks through a bounded staging buffer
@@ -1175,47 +1171,41 @@ extern "C" int b200zkp_batch_leaves(b200zkp_batch* b, uint64_t* out) {
     u64 N = (u64)1 << (b->n_log + b->rate_bits);
     u32 row = b->k + b->salt;
     u64 chunk_rows = std::min<u64>(N, std::max<u64>(1, ((u64)256 << 20) / ((u64)row * 8)));
-    void* stage = nullptr; size_t stage_b = (size_t)chunk_rows * row * 8;
-    TRY(dev_alloc(ctx, stage_b, &stage));
-    int rc = 0;
-    for (u64 r0 = 0; r0 < N && !rc; r0 += chunk_rows) {
+    DevBuf stage;
+    TRY(stage.alloc(ctx, (size_t)chunk_rows * row * 8));
+    for (u64 r0 = 0; r0 < N; r0 += chunk_rows) {
         u64 nr = std::min(chunk_rows, N - r0);
-        rc = dev_transpose_rows_locked(ctx, b->lde, N, row, r0, nr, (u64*)stage);
-        if (!rc) rc = d2h(ctx, out + r0 * row, stage, (size_t)nr * row * 8);
+        TRY(dev_transpose_rows_locked(ctx, b->lde.get(), N, row, r0, nr, stage.get()));
+        TRY(d2h(ctx, out + r0 * row, stage.get(), (size_t)nr * row * 8));
     }
-    dev_release(ctx, stage, stage_b);
-    return rc;
+    return 0;
 }
 
 static int gather_locked(b200zkp_ctx* ctx, const u64* lde, u64 N, u32 row, const u64* digests, u32 sub_log,
                          const u64* idx, u64 n_idx, u64* rows, u64* siblings) {
     if (!n_idx) return 0;
     for (u64 i = 0; i < n_idx; i++) if (idx[i] >= N) BAD(ctx, "leaf index out of range");
-    void *d_idx = nullptr, *d_rows = nullptr, *d_sib = nullptr;
-    size_t idx_b = n_idx * 8, rows_b = rows ? n_idx * row * 8 : 0, sib_b = siblings ? n_idx * sub_log * 32 : 0;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, idx_b, &d_idx)) || (rc = dev_alloc(ctx, rows_b, &d_rows)) || (rc = dev_alloc(ctx, sib_b, &d_sib))) {
-        dev_release(ctx, d_idx, idx_b); dev_release(ctx, d_rows, rows_b); dev_release(ctx, d_sib, sib_b);
-        return rc;
-    }
-    auto done = [&](int code) { dev_release(ctx, d_idx, idx_b); dev_release(ctx, d_rows, rows_b); dev_release(ctx, d_sib, sib_b); return code; };
-    if ((rc = h2d(ctx, d_idx, idx, idx_b))) return done(rc);
-    if (rows_b) {
+    DevBuf d_idx, d_rows, d_sib;
+    TRY(d_idx.alloc(ctx, n_idx * 8));
+    TRY(d_rows.alloc(ctx, rows ? n_idx * row * 8 : 0));
+    TRY(d_sib.alloc(ctx, siblings ? n_idx * sub_log * 32 : 0));
+    TRY(h2d(ctx, d_idx.get(), idx, d_idx.bytes()));
+    if (d_rows.bytes()) {
         u64 cnt = n_idx * row;
-        merkle::gather_rows_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(lde, N, row, (const u64*)d_idx, n_idx, (u64*)d_rows, N - 1);
+        merkle::gather_rows_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(lde, N, row, d_idx.get(), n_idx, d_rows.get(), N - 1);
         ctx->launches++;
-        if ((rc = d2h(ctx, rows, d_rows, rows_b))) return done(rc);
+        TRY(d2h(ctx, rows, d_rows.get(), d_rows.bytes()));
     }
-    if (sib_b) {
+    if (d_sib.bytes()) {
         merkle::TreeShape shape; shape.sub_log = sub_log; shape.sub_digests = 2 * (((u64)1 << sub_log) - 1);
         u64 cnt = n_idx * sub_log;
-        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(digests, shape, (const u64*)d_idx, n_idx, (u64*)d_sib, N - 1);
+        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(digests, shape, d_idx.get(), n_idx, d_sib.get(), N - 1);
         ctx->launches++;
-        if ((rc = d2h(ctx, siblings, d_sib, sib_b))) return done(rc);
+        TRY(d2h(ctx, siblings, d_sib.get(), d_sib.bytes()));
     }
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return done(B200ZKP_ERR_CUDA); }
-    return done(0);
+    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    return 0;
 }
 
 extern "C" int b200zkp_batch_rows(b200zkp_batch* b, const uint64_t* idx, uint64_t n_idx, uint64_t* rows,
@@ -1223,7 +1213,7 @@ extern "C" int b200zkp_batch_rows(b200zkp_batch* b, const uint64_t* idx, uint64_
     if (!b || (!idx && n_idx)) return B200ZKP_ERR_BAD_ARG;
     Guard g(b->ctx);
     u32 N_log = b->n_log + b->rate_bits;
-    return gather_locked(b->ctx, b->lde, (u64)1 << N_log, b->k + b->salt, b->digests, N_log - b->cap_height,
+    return gather_locked(b->ctx, b->lde.get(), (u64)1 << N_log, b->k + b->salt, b->digests.get(), N_log - b->cap_height,
                          (const u64*)idx, n_idx, (u64*)rows, (u64*)siblings);
 }
 
@@ -1237,16 +1227,16 @@ extern "C" int b200zkp_batch_lde_values(b200zkp_batch* b, uint64_t index, uint64
     u64 leaf = 0;
     for (u32 i = 0; i < N_log; i++) leaf |= ((nat >> i) & 1) << (N_log - 1 - i);
     // salt columns are last, so the first k entries of the row are the polynomial values
-    return gather_locked(b->ctx, b->lde, N, b->k, b->digests, 0, &leaf, 1, (u64*)out, nullptr);
+    return gather_locked(b->ctx, b->lde.get(), N, b->k, b->digests.get(), 0, &leaf, 1, (u64*)out, nullptr);
 }
 
 extern "C" int b200zkp_batch_device_ptrs(b200zkp_batch* b, const uint64_t** coeffs, const uint64_t** lde,
                                          const uint64_t** digests, const uint64_t** cap) {
     if (!b) return B200ZKP_ERR_BAD_ARG;
-    if (coeffs) *coeffs = (const uint64_t*)b->coeffs;
-    if (lde) *lde = (const uint64_t*)b->lde;
-    if (digests) *digests = (const uint64_t*)b->digests;
-    if (cap) *cap = (const uint64_t*)b->cap;
+    if (coeffs) *coeffs = (const uint64_t*)b->coeffs.get();
+    if (lde) *lde = (const uint64_t*)b->lde.get();
+    if (digests) *digests = (const uint64_t*)b->digests.get();
+    if (cap) *cap = (const uint64_t*)b->cap.get();
     return 0;
 }
 
@@ -1258,9 +1248,8 @@ extern "C" int b200zkp_dev_gather(b200zkp_ctx* ctx, const uint64_t* lde, uint64_
     Guard g(ctx);
     if (!n_idx) return 0;
     if (!idx_dev) BAD(ctx, "null index buffer");
-    if (n_leaves == 0 || (n_leaves & (n_leaves - 1))) BAD(ctx, "number of leaves must be a power of two");
     u32 lg = 0;
-    while (((u64)1 << lg) < n_leaves) lg++;
+    if (!log2_exact(n_leaves, &lg)) BAD(ctx, "number of leaves must be a power of two");
     if (cap_height > lg) BAD(ctx, "cap_height exceeds log2(number of leaves)");
     if (rows_dev) {
         if (!lde) BAD(ctx, "null leaf buffer");
@@ -1293,15 +1282,14 @@ static int dev_eval_ext2_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 col_str
     u64 n_seg = 1;
     while (n_seg < want && (n / (n_seg * 2)) >= 1024) n_seg *= 2;
     u64 seg_len = n / n_seg;
-    void* d_part = nullptr; size_t part_b = (size_t)k * n_seg * sizeof(evalk::Ext2);
-    TRY(dev_alloc(ctx, part_b, &d_part));
+    DevBuf d_part;
+    TRY(d_part.alloc(ctx, (size_t)k * n_seg * sizeof(evalk::Ext2)));
     dim3 grid((unsigned)n_seg, k);
-    evalk::eval_segments_kernel<<<grid, evalk::EVAL_THREADS, 0, ctx->stream>>>(coeffs, col_stride, n, seg_len, z, (evalk::Ext2*)d_part);
+    evalk::eval_segments_kernel<<<grid, evalk::EVAL_THREADS, 0, ctx->stream>>>(coeffs, col_stride, n, seg_len, z, (evalk::Ext2*)d_part.get());
     ctx->launches++;
-    evalk::eval_combine_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>((const evalk::Ext2*)d_part, (u32)n_seg, seg_len, k, z, (evalk::Ext2*)d_out);
+    evalk::eval_combine_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>((const evalk::Ext2*)d_part.get(), (u32)n_seg, seg_len, k, z, (evalk::Ext2*)d_out);
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
-    dev_release(ctx, d_part, part_b);    // stream-ordered reuse on the same ctx
     if (e != cudaSuccess) { ctx->err = std::string("eval: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
     return 0;
 }
@@ -1318,12 +1306,10 @@ extern "C" int b200zkp_batch_eval_ext2(b200zkp_batch* b, const uint64_t zeta[2],
     if (!b || !zeta || !out) return B200ZKP_ERR_BAD_ARG;
     b200zkp_ctx* ctx = b->ctx;
     Guard g(ctx);
-    void* d_out = nullptr; size_t out_b = (size_t)b->k * 16;
-    TRY(dev_alloc(ctx, out_b, &d_out));
-    int rc = dev_eval_ext2_locked(ctx, b->coeffs, (u64)1 << b->n_log, b->n_log, b->k, (const u64*)zeta, (u64*)d_out);
-    if (!rc) rc = d2h(ctx, out, d_out, out_b);
-    dev_release(ctx, d_out, out_b);
-    return rc;
+    DevBuf d_out;
+    TRY(d_out.alloc(ctx, (size_t)b->k * 16));
+    TRY(dev_eval_ext2_locked(ctx, b->coeffs.get(), (u64)1 << b->n_log, b->n_log, b->k, (const u64*)zeta, d_out.get()));
+    return d2h(ctx, out, d_out.get(), d_out.bytes());
 }
 
 // ------------------------------------------------------------------------------------------------ opening proof (N2 + N3)
@@ -1343,8 +1329,7 @@ static inline HostExt host_ext_pow(HostExt x, u64 e) {
 static inline evalk::Ext2 to_dev(HostExt x) { evalk::Ext2 r; r.a = x.a; r.b = x.b; return r; }
 
 struct FriLayer {
-    u64 *rows = nullptr, *digests = nullptr, *cap = nullptr;
-    size_t rows_b = 0, digests_b = 0, cap_b = 0;
+    DevBuf rows, digests, cap;
     u32 arity_bits = 0, cap_height = 0;
     u64 n_leaves = 0;
 };
@@ -1354,48 +1339,28 @@ struct b200zkp_fri {
     u32 n_log = 0, rate_bits = 0;
     u32 cur_log = 0;          // log2 of the current (folded) LDE size
     u64 shift = 7;            // coset shift of the current values
-    u64* coef[2] = {};        // ping-pong coefficient planes; coef[i] = [2][cap_i], plane stride cap_i
-    size_t coef_b[2] = {};
+    DevBuf coef[2];           // ping-pong coefficient planes; coef[i] = [2][cap_i], plane stride cap_i
     u64 coef_stride[2] = {};
     int cur = 0;
-    u64* values = nullptr;    // [2][N] planes, bit-reversed values of the current layer
-    size_t values_b = 0;
+    DevBuf values;            // [2][N] planes, bit-reversed values of the current layer
     u64 N = 0;
     bool values_ready = false;
     int pending_arity_bits = -1;
     std::vector<FriLayer> layers;
 };
 
-static void fri_release(b200zkp_fri* f) {
-    b200zkp_ctx* ctx = f->ctx;
-    for (int i = 0; i < 2; i++) dev_release(ctx, f->coef[i], f->coef_b[i]);
-    dev_release(ctx, f->values, f->values_b);
-    for (auto& L : f->layers) {
-        dev_release(ctx, L.rows, L.rows_b);
-        dev_release(ctx, L.digests, L.digests_b);
-        dev_release(ctx, L.cap, L.cap_b);
-    }
-    delete f;
-}
-
-static int fri_alloc_state(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, b200zkp_fri** out) {
+static int fri_alloc_state(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, std::unique_ptr<b200zkp_fri>* out) {
     if (rate_bits > 8 || n_log + rate_bits > 32) BAD(ctx, "n_log + rate_bits exceeds two-adicity");
-    b200zkp_fri* f = new (std::nothrow) b200zkp_fri();
+    std::unique_ptr<b200zkp_fri> f(new (std::nothrow) b200zkp_fri());
     if (!f) return B200ZKP_ERR_OOM;
     f->ctx = ctx; f->n_log = n_log; f->rate_bits = rate_bits; f->cur_log = n_log + rate_bits;
     f->N = (u64)1 << f->cur_log;
     f->coef_stride[0] = f->N; f->coef_stride[1] = std::max<u64>(f->N / 2, 1);
-    for (int i = 0; i < 2; i++) f->coef_b[i] = (size_t)2 * f->coef_stride[i] * 8;
-    f->values_b = (size_t)2 * f->N * 8;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, f->coef_b[0], (void**)&f->coef[0])) || (rc = dev_alloc(ctx, f->coef_b[1], (void**)&f->coef[1])) ||
-        (rc = dev_alloc(ctx, f->values_b, (void**)&f->values))) {
-        fri_release(f);
-        return rc;
-    }
-    cudaError_t e = cudaMemsetAsync(f->coef[0], 0, f->coef_b[0], ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("fri: ") + cudaGetErrorString(e); fri_release(f); return B200ZKP_ERR_CUDA; }
-    *out = f;
+    for (int i = 0; i < 2; i++) TRY(f->coef[i].alloc(ctx, (size_t)2 * f->coef_stride[i] * 8));
+    TRY(f->values.alloc(ctx, (size_t)2 * f->N * 8));
+    cudaError_t e = cudaMemsetAsync(f->coef[0].get(), 0, f->coef[0].bytes(), ctx->stream);
+    if (e != cudaSuccess) { ctx->err = std::string("fri: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    *out = std::move(f);
     return 0;
 }
 
@@ -1423,7 +1388,7 @@ static int fri_compute_values(b200zkp_fri* f) {
     u64 M = (u64)1 << f->cur_log;
     const u64* scale = nullptr;
     TRY(get_power_scale(ctx, f->shift, f->cur_log, &scale));
-    TRY(run_transform(ctx, f->coef[f->cur], f->coef_stride[f->cur], f->values, M, nullptr, f->cur_log, 2, /*dir=*/0,
+    TRY(run_transform(ctx, f->coef[f->cur].get(), f->coef_stride[f->cur], f->values.get(), M, nullptr, f->cur_log, 2, /*dir=*/0,
                       /*bitrev_out=*/true, scale, 0, /*inverse_scale=*/false, /*canon_in=*/false));
     f->values_ready = true;
     return 0;
@@ -1451,55 +1416,53 @@ extern "C" int b200zkp_fri_begin(b200zkp_ctx* ctx, b200zkp_batch* const* oracles
         if (poly_index[i] >= oracles[poly_oracle[i]]->k) BAD(ctx, "polynomial index out of range");
     }
     if (!max_k) BAD(ctx, "no polynomial to open");
-    b200zkp_fri* f = nullptr;
+    std::unique_ptr<b200zkp_fri> f;
     TRY(fri_alloc_state(ctx, n_log, rate_bits, &f));
     HostExt alpha{gl_host_canon(alpha_in[0]), gl_host_canon(alpha_in[1])};
     u32 n_seg = (u32)((n + frik::SCAN_SEG - 1) / frik::SCAN_SEG);
-    void *d_ptrs = nullptr, *d_pw = nullptr, *d_comp = nullptr, *d_tot = nullptr, *d_carry = nullptr;
-    size_t ptrs_b = (size_t)max_k * 8, pw_b = (size_t)max_k * 16, comp_b = (size_t)2 * n * 8, seg_b = (size_t)n_seg * 16;
-    int rc = 0;
-    auto done = [&](int code) {
-        dev_release(ctx, d_ptrs, ptrs_b); dev_release(ctx, d_pw, pw_b); dev_release(ctx, d_comp, comp_b);
-        dev_release(ctx, d_tot, seg_b); dev_release(ctx, d_carry, seg_b);
-        if (code) fri_release(f); else *out = f;
-        return code;
-    };
-    if ((rc = dev_alloc(ctx, ptrs_b, &d_ptrs)) || (rc = dev_alloc(ctx, pw_b, &d_pw)) || (rc = dev_alloc(ctx, comp_b, &d_comp)) ||
-        (rc = dev_alloc(ctx, seg_b, &d_tot)) || (rc = dev_alloc(ctx, seg_b, &d_carry)))
-        return done(rc);
-    u64* fin_a = f->coef[0];
-    u64* fin_b = f->coef[0] + f->coef_stride[0];
-    u64* comp_a = (u64*)d_comp;
-    u64* comp_im = (u64*)d_comp + n;
+    DevBuf d_ptrs, d_pw, d_comp, d_tot, d_carry;
+    TRY(d_ptrs.alloc(ctx, (size_t)max_k * 8));
+    TRY(d_pw.alloc(ctx, (size_t)max_k * 16));
+    TRY(d_comp.alloc(ctx, (size_t)2 * n * 8));
+    TRY(d_tot.alloc(ctx, (size_t)n_seg * 16));
+    TRY(d_carry.alloc(ctx, (size_t)n_seg * 16));
+    u64* fin_a = f->coef[0].get();
+    u64* fin_b = f->coef[0].get() + f->coef_stride[0];
+    u64* comp_a = d_comp.get();
+    u64* comp_im = d_comp.get() + n;
+    evalk::Ext2* pw = (evalk::Ext2*)d_pw.get();
+    evalk::Ext2* tot = (evalk::Ext2*)d_tot.get();
+    evalk::Ext2* carry = (evalk::Ext2*)d_carry.get();
     std::vector<const u64*> ptrs(max_k);
     u32 off = 0;
     for (u32 b = 0; b < n_points; b++) {
         u32 k = point_n_polys[b];
         if (!k) continue;       // an empty batch contributes the zero polynomial and alpha^0
-        for (u32 i = 0; i < k; i++) ptrs[i] = oracles[poly_oracle[off + i]]->coeffs + (u64)poly_index[off + i] * n;
+        for (u32 i = 0; i < k; i++) ptrs[i] = oracles[poly_oracle[off + i]]->coeffs.get() + (u64)poly_index[off + i] * n;
         off += k;
-        if ((rc = h2d(ctx, d_ptrs, ptrs.data(), (size_t)k * 8))) return done(rc);
-        frik::ext_powers_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>(to_dev(alpha), k, (evalk::Ext2*)d_pw);
+        TRY(h2d(ctx, d_ptrs.get(), ptrs.data(), (size_t)k * 8));
+        frik::ext_powers_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>(to_dev(alpha), k, pw);
         ctx->launches++;
         frik::reduce_polys_base_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(
-            (const u64* const*)d_ptrs, k, n, (const evalk::Ext2*)d_pw, comp_a, comp_im);
+            (const u64* const*)d_ptrs.get(), k, n, pw, comp_a, comp_im);
         ctx->launches++;
         HostExt z{gl_host_canon(points[2 * b]), gl_host_canon(points[2 * b + 1])};
-        frik::scan_totals_kernel<<<n_seg, frik::SCAN_THREADS, 0, ctx->stream>>>(comp_a, comp_im, n, to_dev(z), (evalk::Ext2*)d_tot);
+        frik::scan_totals_kernel<<<n_seg, frik::SCAN_THREADS, 0, ctx->stream>>>(comp_a, comp_im, n, to_dev(z), tot);
         ctx->launches++;
-        frik::scan_carries_kernel<<<1, frik::SCAN_THREADS, 0, ctx->stream>>>((const evalk::Ext2*)d_tot, n_seg, to_dev(z), (evalk::Ext2*)d_carry);
+        frik::scan_carries_kernel<<<1, frik::SCAN_THREADS, 0, ctx->stream>>>(tot, n_seg, to_dev(z), carry);
         ctx->launches++;
         // alpha.shift_poly(&mut final_poly): final_poly *= alpha^count, count = polynomials of this batch
         frik::divide_by_linear_kernel<<<n_seg, frik::SCAN_THREADS, 0, ctx->stream>>>(
-            comp_a, comp_im, n, to_dev(z), (const evalk::Ext2*)d_carry, to_dev(host_ext_pow(alpha, k)),
+            comp_a, comp_im, n, to_dev(z), carry, to_dev(host_ext_pow(alpha, k)),
             (flags & B200ZKP_FRI_MUL_BY_X) ? 1u : 0u, fin_a, fin_b);
         ctx->launches++;
         cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { ctx->err = std::string("fri_begin: ") + cudaGetErrorString(e); return done(B200ZKP_ERR_CUDA); }
+        if (e != cudaSuccess) { ctx->err = std::string("fri_begin: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
         // the pointer table is reused by the next batch: the copy above is stream-ordered after these kernels
     }
-    if ((rc = fri_compute_values(f))) return done(rc);
-    return done(0);
+    TRY(fri_compute_values(f.get()));
+    *out = f.release();
+    return 0;
 }
 
 extern "C" int b200zkp_fri_begin_from_coeffs(b200zkp_ctx* ctx, const uint64_t* coeffs, uint32_t n_log, uint32_t rate_bits,
@@ -1509,19 +1472,16 @@ extern "C" int b200zkp_fri_begin_from_coeffs(b200zkp_ctx* ctx, const uint64_t* c
     if (!out) BAD(ctx, "null out");
     *out = nullptr;
     if (!coeffs) BAD(ctx, "null buffer");
-    b200zkp_fri* f = nullptr;
+    std::unique_ptr<b200zkp_fri> f;
     TRY(fri_alloc_state(ctx, n_log, rate_bits, &f));
     u64 n = (u64)1 << n_log;
     // stage the interleaved input in the (still unused) values buffer
-    int rc = h2d(ctx, f->values, coeffs, (size_t)n * 16);
-    if (!rc) {
-        frik::deinterleave_kernel<<<(unsigned)((2 * n + 255) / 256), 256, 0, ctx->stream>>>(f->values, n, f->coef[0], f->coef[0] + f->coef_stride[0]);
-        ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: deinterleave launch failed"; rc = B200ZKP_ERR_CUDA; }
-    }
-    if (!rc) rc = fri_compute_values(f);
-    if (rc) { fri_release(f); return rc; }
-    *out = f;
+    TRY(h2d(ctx, f->values.get(), coeffs, (size_t)n * 16));
+    frik::deinterleave_kernel<<<(unsigned)((2 * n + 255) / 256), 256, 0, ctx->stream>>>(f->values.get(), n, f->coef[0].get(), f->coef[0].get() + f->coef_stride[0]);
+    ctx->launches++;
+    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: deinterleave launch failed"; return B200ZKP_ERR_CUDA; }
+    TRY(fri_compute_values(f.get()));
+    *out = f.release();
     return 0;
 }
 
@@ -1529,7 +1489,7 @@ extern "C" void b200zkp_fri_free(b200zkp_fri* f) {
     if (!f) return;
     Guard g(f->ctx);
     cudaStreamSynchronize(f->ctx->stream);
-    fri_release(f);
+    delete f;
 }
 
 extern "C" int b200zkp_fri_shape(const b200zkp_fri* f, uint32_t shape[4]) {
@@ -1541,16 +1501,13 @@ extern "C" int b200zkp_fri_shape(const b200zkp_fri* f, uint32_t shape[4]) {
 static int fri_copy_coeffs(b200zkp_fri* f, u64 len, u64* out) {
     b200zkp_ctx* ctx = f->ctx;
     if (!len) return 0;
-    void* d = nullptr; size_t bytes = (size_t)len * 16;
-    TRY(dev_alloc(ctx, bytes, &d));
-    const u64* pa = f->coef[f->cur];
-    frik::interleave_kernel<<<(unsigned)((2 * len + 255) / 256), 256, 0, ctx->stream>>>(pa, pa + f->coef_stride[f->cur], len, (u64*)d);
+    DevBuf d;
+    TRY(d.alloc(ctx, (size_t)len * 16));
+    const u64* pa = f->coef[f->cur].get();
+    frik::interleave_kernel<<<(unsigned)((2 * len + 255) / 256), 256, 0, ctx->stream>>>(pa, pa + f->coef_stride[f->cur], len, d.get());
     ctx->launches++;
-    int rc = cudaGetLastError() == cudaSuccess ? 0 : B200ZKP_ERR_CUDA;
-    if (rc) ctx->err = "fri: interleave launch failed";
-    if (!rc) rc = d2h(ctx, out, d, bytes);
-    dev_release(ctx, d, bytes);
-    return rc;
+    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: interleave launch failed"; return B200ZKP_ERR_CUDA; }
+    return d2h(ctx, out, d.get(), d.bytes());
 }
 
 extern "C" int b200zkp_fri_coeffs(b200zkp_fri* f, uint64_t* out) {
@@ -1577,23 +1534,16 @@ extern "C" int b200zkp_fri_commit_layer(b200zkp_fri* f, uint32_t arity_bits, uin
     u64 M = (u64)1 << f->cur_log;
     FriLayer L;
     L.arity_bits = arity_bits; L.cap_height = cap_height; L.n_leaves = M >> arity_bits;
-    L.rows_b = (size_t)M * 16;
-    L.digests_b = (size_t)2 * (L.n_leaves - ((u64)1 << cap_height)) * 32;
-    L.cap_b = ((size_t)32) << cap_height;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, L.rows_b, (void**)&L.rows)) || (rc = dev_alloc(ctx, L.digests_b, (void**)&L.digests)) ||
-        (rc = dev_alloc(ctx, L.cap_b, (void**)&L.cap))) {
-        dev_release(ctx, L.rows, L.rows_b); dev_release(ctx, L.digests, L.digests_b); dev_release(ctx, L.cap, L.cap_b);
-        return rc;
-    }
-    auto fail = [&](int code) { dev_release(ctx, L.rows, L.rows_b); dev_release(ctx, L.digests, L.digests_b); dev_release(ctx, L.cap, L.cap_b); return code; };
-    frik::interleave_kernel<<<(unsigned)((2 * M + 255) / 256), 256, 0, ctx->stream>>>(f->values, f->values + M, M, L.rows);
+    TRY(L.rows.alloc(ctx, (size_t)M * 16));
+    TRY(L.digests.alloc(ctx, (size_t)2 * (L.n_leaves - ((u64)1 << cap_height)) * 32));
+    TRY(L.cap.alloc(ctx, ((size_t)32) << cap_height));
+    frik::interleave_kernel<<<(unsigned)((2 * M + 255) / 256), 256, 0, ctx->stream>>>(f->values.get(), f->values.get() + M, M, L.rows.get());
     ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: interleave launch failed"; return fail(B200ZKP_ERR_CUDA); }
+    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: interleave launch failed"; return B200ZKP_ERR_CUDA; }
     u32 leaf_len = 2u << arity_bits;
-    if ((rc = dev_merkle_locked(ctx, L.rows, leaf_len, 1, leaf_len, L.n_leaves, cap_height, L.digests, L.cap))) return fail(rc);
-    if ((rc = d2h(ctx, cap_out, L.cap, L.cap_b))) return fail(rc);
-    f->layers.push_back(L);
+    TRY(dev_merkle_locked(ctx, L.rows.get(), leaf_len, 1, leaf_len, L.n_leaves, cap_height, L.digests.get(), L.cap.get()));
+    TRY(d2h(ctx, cap_out, L.cap.get(), L.cap.bytes()));
+    f->layers.push_back(std::move(L));
     f->pending_arity_bits = (int)arity_bits;
     return 0;
 }
@@ -1608,8 +1558,8 @@ extern "C" int b200zkp_fri_fold(b200zkp_fri* f, const uint64_t beta_in[2]) {
     u64 out_len = ((u64)1 << f->cur_log) >> ab;
     int nxt = f->cur ^ 1;
     HostExt beta{gl_host_canon(beta_in[0]), gl_host_canon(beta_in[1])};
-    const u64* ia = f->coef[f->cur];
-    u64* oa = f->coef[nxt];
+    const u64* ia = f->coef[f->cur].get();
+    u64* oa = f->coef[nxt].get();
     frik::fold_kernel<<<(unsigned)((out_len + 127) / 128), 128, 0, ctx->stream>>>(
         ia, ia + f->coef_stride[f->cur], out_len, 1u << ab, to_dev(beta), oa, oa + f->coef_stride[nxt]);
     LAUNCH_CHECK(ctx);
@@ -1631,30 +1581,29 @@ extern "C" int b200zkp_fri_query(b200zkp_fri* f, uint32_t layer, const uint64_t*
     if (!n_idx) return 0;
     for (u64 i = 0; i < n_idx; i++) if (idx[i] >= L.n_leaves) BAD(ctx, "leaf index out of range");
     u32 lg = 0;
-    while (((u64)1 << lg) < L.n_leaves) lg++;
+    log2_exact(L.n_leaves, &lg);
     u32 depth = lg - L.cap_height, row_len = 2u << L.arity_bits;
-    void *d_idx = nullptr, *d_rows = nullptr, *d_sib = nullptr;
-    size_t idx_b = n_idx * 8, rows_b = evals ? n_idx * row_len * 8 : 0, sib_b = (siblings && depth) ? n_idx * depth * 32 : 0;
-    int rc = 0;
-    auto done = [&](int code) { dev_release(ctx, d_idx, idx_b); dev_release(ctx, d_rows, rows_b); dev_release(ctx, d_sib, sib_b); return code; };
-    if ((rc = dev_alloc(ctx, idx_b, &d_idx)) || (rc = dev_alloc(ctx, rows_b, &d_rows)) || (rc = dev_alloc(ctx, sib_b, &d_sib))) return done(rc);
-    if ((rc = h2d(ctx, d_idx, idx, idx_b))) return done(rc);
-    if (rows_b) {
+    DevBuf d_idx, d_rows, d_sib;
+    TRY(d_idx.alloc(ctx, n_idx * 8));
+    TRY(d_rows.alloc(ctx, evals ? n_idx * row_len * 8 : 0));
+    TRY(d_sib.alloc(ctx, (siblings && depth) ? n_idx * depth * 32 : 0));
+    TRY(h2d(ctx, d_idx.get(), idx, d_idx.bytes()));
+    if (d_rows.bytes()) {
         u64 cnt = n_idx * row_len;
-        frik::gather_rows_rm_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.rows, row_len, (const u64*)d_idx, n_idx, (u64*)d_rows);
+        frik::gather_rows_rm_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.rows.get(), row_len, d_idx.get(), n_idx, d_rows.get());
         ctx->launches++;
-        if ((rc = d2h(ctx, evals, d_rows, rows_b))) return done(rc);
+        TRY(d2h(ctx, evals, d_rows.get(), d_rows.bytes()));
     }
-    if (sib_b) {
+    if (d_sib.bytes()) {
         merkle::TreeShape shape; shape.sub_log = depth; shape.sub_digests = 2 * (((u64)1 << depth) - 1);
         u64 cnt = n_idx * depth;
-        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.digests, shape, (const u64*)d_idx, n_idx, (u64*)d_sib, ~0ull);
+        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.digests.get(), shape, d_idx.get(), n_idx, d_sib.get(), ~0ull);
         ctx->launches++;
-        if ((rc = d2h(ctx, siblings, d_sib, sib_b))) return done(rc);
+        TRY(d2h(ctx, siblings, d_sib.get(), d_sib.bytes()));
     }
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return done(B200ZKP_ERR_CUDA); }
-    return done(0);
+    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    return 0;
 }
 
 extern "C" int b200zkp_pow_grind(b200zkp_ctx* ctx, const uint64_t state[12], uint32_t witness_pos, uint32_t response_pos,
@@ -1664,26 +1613,24 @@ extern "C" int b200zkp_pow_grind(b200zkp_ctx* ctx, const uint64_t state[12], uin
     if (!state || !witness) BAD(ctx, "null buffer");
     if (witness_pos >= 12 || response_pos >= 12 || min_leading_zeros > 64) BAD(ctx, "bad argument");
     if (max_candidates == 0 || max_candidates > hostgl::P) max_candidates = hostgl::P;
-    void* d = nullptr; size_t bytes = 13 * 8;      // 12 state words + the running minimum
-    TRY(dev_alloc(ctx, bytes, &d));
+    DevBuf d;
+    TRY(d.alloc(ctx, 13 * 8));      // 12 state words + the running minimum
     u64 h[13];
     for (int i = 0; i < 12; i++) h[i] = gl_host_canon(state[i]);
     h[12] = ~(u64)0;
-    int rc = h2d(ctx, d, h, bytes);
+    TRY(h2d(ctx, d.get(), h, d.bytes()));
     u64 start = 0, window = (u64)1 << 18, best = ~(u64)0;
-    while (!rc && start < max_candidates) {
+    while (start < max_candidates) {
         u64 count = std::min(window, max_candidates - start);
         frik::pow_grind_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(
-            (const u64*)d, witness_pos, response_pos, min_leading_zeros, start, count, (unsigned long long*)d + 12);
+            d.get(), witness_pos, response_pos, min_leading_zeros, start, count, (unsigned long long*)d.get() + 12);
         ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) { ctx->err = "pow_grind launch failed"; rc = B200ZKP_ERR_CUDA; break; }
-        rc = d2h(ctx, &best, (u64*)d + 12, 8);
-        if (rc || best != ~(u64)0) break;
+        if (cudaGetLastError() != cudaSuccess) { ctx->err = "pow_grind launch failed"; return B200ZKP_ERR_CUDA; }
+        TRY(d2h(ctx, &best, d.get() + 12, 8));
+        if (best != ~(u64)0) break;
         start += count;
         if (window < ((u64)1 << 24)) window <<= 2;
     }
-    dev_release(ctx, d, bytes);
-    if (rc) return rc;
     if (best == ~(u64)0) { ctx->err = "proof of work: no witness below the bound"; return B200ZKP_ERR_UNSUPPORTED; }
     *witness = best;
     return 0;
@@ -1696,62 +1643,52 @@ extern "C" int b200zkp_merkle_new(b200zkp_ctx* ctx, const uint64_t* leaves, uint
     Guard g(ctx);
     if (!out) BAD(ctx, "null out");
     *out = nullptr;
-    if (n_leaves == 0 || (n_leaves & (n_leaves - 1))) BAD(ctx, "number of leaves must be a power of two");
     u32 lg = 0;
-    while (((u64)1 << lg) < n_leaves) lg++;
+    if (!log2_exact(n_leaves, &lg)) BAD(ctx, "number of leaves must be a power of two");
     if (cap_height > lg) BAD(ctx, "cap_height exceeds log2(number of leaves)");
     if (!leaves && leaf_len) BAD(ctx, "null leaves");
-    b200zkp_tree* t = new (std::nothrow) b200zkp_tree();
+    std::unique_ptr<b200zkp_tree> t(new (std::nothrow) b200zkp_tree());
     if (!t) return B200ZKP_ERR_OOM;
     t->ctx = ctx; t->n_leaves = n_leaves; t->leaf_len = leaf_len; t->cap_height = cap_height;
-    t->digests_b = (size_t)2 * (n_leaves - ((u64)1 << cap_height)) * 32;
-    t->cap_b = ((size_t)32) << cap_height;
-    void* d_leaves = nullptr; size_t leaves_b = std::max<size_t>((size_t)n_leaves * leaf_len * 8, 8);
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, t->digests_b, (void**)&t->digests)) || (rc = dev_alloc(ctx, t->cap_b, (void**)&t->cap)) ||
-        (rc = dev_alloc(ctx, leaves_b, &d_leaves))) {
-        dev_release(ctx, d_leaves, leaves_b); dev_release(ctx, t->digests, t->digests_b); dev_release(ctx, t->cap, t->cap_b);
-        delete t; return rc;
-    }
-    auto fail = [&](int code) { dev_release(ctx, d_leaves, leaves_b); dev_release(ctx, t->digests, t->digests_b); dev_release(ctx, t->cap, t->cap_b); delete t; return code; };
-    if ((rc = h2d(ctx, d_leaves, leaves, (size_t)n_leaves * leaf_len * 8))) return fail(rc);
-    if ((rc = dev_merkle_locked(ctx, (const u64*)d_leaves, leaf_len, 1, leaf_len, n_leaves, cap_height, t->digests, t->cap))) return fail(rc);
+    DevBuf d_leaves;
+    TRY(t->digests.alloc(ctx, (size_t)2 * (n_leaves - ((u64)1 << cap_height)) * 32));
+    TRY(t->cap.alloc(ctx, ((size_t)32) << cap_height));
+    TRY(d_leaves.alloc(ctx, std::max<size_t>((size_t)n_leaves * leaf_len * 8, 8)));
+    TRY(h2d(ctx, d_leaves.get(), leaves, (size_t)n_leaves * leaf_len * 8));
+    TRY(dev_merkle_locked(ctx, d_leaves.get(), leaf_len, 1, leaf_len, n_leaves, cap_height, t->digests.get(), t->cap.get()));
     cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("merkle_new: ") + cudaGetErrorString(e); return fail(B200ZKP_ERR_CUDA); }
-    dev_release(ctx, d_leaves, leaves_b);
-    *out = t;
+    if (e != cudaSuccess) { ctx->err = std::string("merkle_new: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    *out = t.release();
     return 0;
 }
 extern "C" void b200zkp_tree_free(b200zkp_tree* t) {
     if (!t) return;
     Guard g(t->ctx);
     cudaStreamSynchronize(t->ctx->stream);
-    dev_release(t->ctx, t->digests, t->digests_b);
-    dev_release(t->ctx, t->cap, t->cap_b);
     delete t;
 }
 extern "C" int b200zkp_tree_cap(b200zkp_tree* t, uint64_t* out) {
     if (!t || !out) return B200ZKP_ERR_BAD_ARG;
     Guard g(t->ctx);
-    return d2h(t->ctx, out, t->cap, t->cap_b);
+    return d2h(t->ctx, out, t->cap.get(), t->cap.bytes());
 }
 extern "C" int b200zkp_tree_digests(b200zkp_tree* t, uint64_t* out) {
     if (!t) return B200ZKP_ERR_BAD_ARG;
     Guard g(t->ctx);
-    if (t->digests_b && !out) BAD(t->ctx, "null out");
-    return d2h(t->ctx, out, t->digests, t->digests_b);
+    if (t->digests.bytes() && !out) BAD(t->ctx, "null out");
+    return d2h(t->ctx, out, t->digests.get(), t->digests.bytes());
 }
 extern "C" int b200zkp_tree_prove(b200zkp_tree* t, const uint64_t* idx, uint64_t n_idx, uint64_t* siblings) {
     if (!t || (!idx && n_idx)) return B200ZKP_ERR_BAD_ARG;
     Guard g(t->ctx);
     u32 lg = 0;
-    while (((u64)1 << lg) < t->n_leaves) lg++;
+    log2_exact(t->n_leaves, &lg);
     if (lg == t->cap_height) {
         for (u64 i = 0; i < n_idx; i++) if (idx[i] >= t->n_leaves) BAD(t->ctx, "leaf index out of range");
         return 0;  // empty proofs
     }
     if (!siblings && n_idx) BAD(t->ctx, "null out");
-    return gather_locked(t->ctx, nullptr, t->n_leaves, 0, t->digests, lg - t->cap_height, (const u64*)idx, n_idx,
+    return gather_locked(t->ctx, nullptr, t->n_leaves, 0, t->digests.get(), lg - t->cap_height, (const u64*)idx, n_idx,
                          nullptr, (u64*)siblings);
 }
 
@@ -1769,40 +1706,33 @@ static int dev_partial_products_locked(b200zkp_ctx* ctx, const u64* wires, u64 w
     std::vector<u64> small((size_t)R + 2 * C);
     for (u32 j = 0; j < R; j++) small[j] = k_is[j] % hostgl::P;
     for (u32 c = 0; c < C; c++) { small[R + c] = betas[c] % hostgl::P; small[R + C + c] = gammas[c] % hostgl::P; }
-    void *d_small = nullptr, *d_run = nullptr, *d_tot = nullptr;
-    const size_t small_b = small.size() * 8, run_b = (size_t)C * chunks * n * 8;
     const u32 per = 4;
     const u32 n_blocks = (u32)((n + (u64)perm::SCAN_THREADS * per - 1) / ((u64)perm::SCAN_THREADS * per));
-    const size_t tot_b = (size_t)C * n_blocks * 8;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, small_b, &d_small))) return rc;
-    if ((rc = dev_alloc(ctx, run_b, &d_run))) { dev_release(ctx, d_small, small_b); return rc; }
-    if ((rc = dev_alloc(ctx, tot_b, &d_tot))) { dev_release(ctx, d_small, small_b); dev_release(ctx, d_run, run_b); return rc; }
-    auto done = [&](int code) {
-        if (code == 0) { cudaError_t e = cudaStreamSynchronize(ctx->stream); if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); code = B200ZKP_ERR_CUDA; } }
-        dev_release(ctx, d_small, small_b); dev_release(ctx, d_run, run_b); dev_release(ctx, d_tot, tot_b);
-        return code;
-    };
-    if ((rc = h2d(ctx, d_small, small.data(), small_b))) return done(rc);
+    DevBuf d_small, d_run, d_tot;
+    TRY(d_small.alloc(ctx, small.size() * 8));
+    TRY(d_run.alloc(ctx, (size_t)C * chunks * n * 8));
+    TRY(d_tot.alloc(ctx, (size_t)C * n_blocks * 8));
+    TRY(h2d(ctx, d_small.get(), small.data(), d_small.bytes()));
     {   // `small` is a pageable host vector
         cudaError_t e0 = cudaStreamSynchronize(ctx->stream);
-        if (e0 != cudaSuccess) { ctx->err = cudaGetErrorString(e0); return done(B200ZKP_ERR_CUDA); }
+        if (e0 != cudaSuccess) { ctx->err = cudaGetErrorString(e0); return B200ZKP_ERR_CUDA; }
     }
     perm::Params p;
     p.wires = wires; p.wires_stride = wires_stride; p.sigmas = sigmas; p.sigmas_stride = sigmas_stride;
-    p.k_is = (const u64*)d_small; p.betas = (const u64*)d_small + R; p.gammas = (const u64*)d_small + R + C;
+    p.k_is = d_small.get(); p.betas = d_small.get() + R; p.gammas = d_small.get() + R + C;
     p.omega = hostgl::root(n_log); p.n = n; p.R = R; p.degree = degree; p.chunks = chunks; p.C = C;
-    perm::chunk_products_kernel<<<dim3((unsigned)((n + 127) / 128), C), 128, 0, ctx->stream>>>(p, (u64*)d_run);
+    perm::chunk_products_kernel<<<dim3((unsigned)((n + 127) / 128), C), 128, 0, ctx->stream>>>(p, d_run.get());
     ctx->launches++;
-    perm::block_totals_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>((const u64*)d_run, n, chunks, per, (u64*)d_tot);
+    perm::block_totals_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>(d_run.get(), n, chunks, per, d_tot.get());
     ctx->launches++;
-    perm::scan_totals_kernel<<<C, perm::SCAN_THREADS, 0, ctx->stream>>>((u64*)d_tot, n_blocks);
+    perm::scan_totals_kernel<<<C, perm::SCAN_THREADS, 0, ctx->stream>>>(d_tot.get(), n_blocks);
     ctx->launches++;
-    perm::finish_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>((const u64*)d_run, (const u64*)d_tot, n, chunks, per, C, out, out_stride);
+    perm::finish_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>(d_run.get(), d_tot.get(), n, chunks, per, C, out, out_stride);
     ctx->launches++;
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return done(B200ZKP_ERR_CUDA); }
-    return done(0);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    return 0;
 }
 
 extern "C" int b200zkp_dev_partial_products_and_zs(b200zkp_ctx* ctx, const uint64_t* wires_dev, uint64_t wires_col_stride,
@@ -1828,17 +1758,15 @@ extern "C" int b200zkp_partial_products_and_zs(b200zkp_ctx* ctx, const uint64_t*
     const u64 n = (u64)1 << n_log;
     const u32 chunks = (num_routed + degree - 1) / degree;
     const size_t in_b = (size_t)num_routed * n * 8, out_b = (size_t)num_challenges * chunks * n * 8;
-    void *d_w = nullptr, *d_s = nullptr, *d_o = nullptr;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, in_b, &d_w))) return rc;
-    if ((rc = dev_alloc(ctx, in_b, &d_s))) { dev_release(ctx, d_w, in_b); return rc; }
-    if ((rc = dev_alloc(ctx, out_b, &d_o))) { dev_release(ctx, d_w, in_b); dev_release(ctx, d_s, in_b); return rc; }
-    auto done = [&](int code) { dev_release(ctx, d_w, in_b); dev_release(ctx, d_s, in_b); dev_release(ctx, d_o, out_b); return code; };
-    if ((rc = h2d(ctx, d_w, wires, in_b)) || (rc = h2d(ctx, d_s, sigmas, in_b))) return done(rc);
-    rc = dev_partial_products_locked(ctx, (const u64*)d_w, n, (const u64*)d_s, n, n_log, num_routed, degree, (const u64*)k_is,
-                                     (const u64*)betas, (const u64*)gammas, num_challenges, (u64*)d_o, n);
-    if (!rc) rc = d2h(ctx, out, d_o, out_b);
-    return done(rc);
+    DevBuf d_w, d_s, d_o;
+    TRY(d_w.alloc(ctx, in_b));
+    TRY(d_s.alloc(ctx, in_b));
+    TRY(d_o.alloc(ctx, out_b));
+    TRY(h2d(ctx, d_w.get(), wires, in_b));
+    TRY(h2d(ctx, d_s.get(), sigmas, in_b));
+    TRY(dev_partial_products_locked(ctx, d_w.get(), n, d_s.get(), n, n_log, num_routed, degree, (const u64*)k_is,
+                                    (const u64*)betas, (const u64*)gammas, num_challenges, d_o.get(), n));
+    return d2h(ctx, out, d_o.get(), out_b);
 }
 
 // ------------------------------------------------------------------------------------------------ Hasher / field helpers
@@ -1867,17 +1795,12 @@ static int with_io(b200zkp_ctx* ctx, const void* in, size_t in_b, void* out, siz
         if (out_b) memcpy(out, (char*)ctx->mailbox + in_pad, out_b);
         return 0;
     }
-    void *d_in = nullptr, *d_out = nullptr;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, std::max<size_t>(in_b, 8), &d_in)) || (rc = dev_alloc(ctx, std::max<size_t>(out_b, 8), &d_out))) {
-        dev_release(ctx, d_in, std::max<size_t>(in_b, 8));
-        return rc;
-    }
-    auto done = [&](int code) { dev_release(ctx, d_in, std::max<size_t>(in_b, 8)); dev_release(ctx, d_out, std::max<size_t>(out_b, 8)); return code; };
-    if ((rc = h2d(ctx, d_in, in, in_b))) return done(rc);
-    if ((rc = body((u64*)d_in, (u64*)d_out))) return done(rc);
-    if ((rc = d2h(ctx, out, d_out, out_b))) return done(rc);
-    return done(0);
+    DevBuf d_in, d_out;
+    TRY(d_in.alloc(ctx, std::max<size_t>(in_b, 8)));
+    TRY(d_out.alloc(ctx, std::max<size_t>(out_b, 8)));
+    TRY(h2d(ctx, d_in.get(), in, in_b));
+    TRY(body(d_in.get(), d_out.get()));
+    return d2h(ctx, out, d_out.get(), out_b);
 }
 
 extern "C" int b200zkp_poseidon_permute(b200zkp_ctx* ctx, const uint64_t* in, uint64_t count, uint64_t* out) {
@@ -1945,19 +1868,17 @@ extern "C" int b200zkp_two_to_one(b200zkp_ctx* ctx, const uint64_t* left, const 
     Guard g(ctx);
     if (!count) return 0;
     if (!left || !right || !out) BAD(ctx, "null buffer");
-    void* d_r = nullptr;
-    TRY(dev_alloc(ctx, count * 32, &d_r));
-    int rc = h2d(ctx, d_r, right, count * 32);
-    if (!rc) rc = with_io(ctx, left, count * 32, out, count * 32, [&](u64* dl, u64* dout) -> int {
+    DevBuf d_r;
+    TRY(d_r.alloc(ctx, count * 32));
+    TRY(h2d(ctx, d_r.get(), right, count * 32));
+    return with_io(ctx, left, count * 32, out, count * 32, [&](u64* dl, u64* dout) -> int {
         if (count <= COOP_MAX_NODES)
-            merkle::permute_coop_kernel<<<(unsigned)((count * 16 + 127) / 128), 128, 0, ctx->stream>>>(dl, (const u64*)d_r, dout, count, 1u, ctx->round_add);
+            merkle::permute_coop_kernel<<<(unsigned)((count * 16 + 127) / 128), 128, 0, ctx->stream>>>(dl, d_r.get(), dout, count, 1u, ctx->round_add);
         else
-            merkle::two_to_one_kernel<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(dl, (const u64*)d_r, dout, count);
+            merkle::two_to_one_kernel<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(dl, d_r.get(), dout, count);
         LAUNCH_CHECK(ctx);
         return 0;
     });
-    dev_release(ctx, d_r, count * 32);
-    return rc;
 }
 
 static int transform_host(b200zkp_ctx* ctx, u64* data, u32 n_log, u32 k, int dir) {
@@ -1965,19 +1886,15 @@ static int transform_host(b200zkp_ctx* ctx, u64* data, u32 n_log, u32 k, int dir
     if (!data) BAD(ctx, "null buffer");
     if (n_log > 32) BAD(ctx, "n_log exceeds two-adicity");
     size_t bytes = ((size_t)k << n_log) * 8;
-    void *d = nullptr, *scratch = nullptr, *dout = nullptr;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, bytes, &d)) || (rc = dev_alloc(ctx, bytes, &scratch)) || (rc = dev_alloc(ctx, bytes, &dout))) {
-        dev_release(ctx, d, bytes); dev_release(ctx, scratch, bytes);
-        return rc;
-    }
-    auto done = [&](int code) { dev_release(ctx, d, bytes); dev_release(ctx, scratch, bytes); dev_release(ctx, dout, bytes); return code; };
-    if ((rc = h2d(ctx, d, data, bytes))) return done(rc);
+    DevBuf d, scratch, dout;
+    TRY(d.alloc(ctx, bytes));
+    TRY(scratch.alloc(ctx, bytes));
+    TRY(dout.alloc(ctx, bytes));
+    TRY(h2d(ctx, d.get(), data, bytes));
     u64 n = (u64)1 << n_log;
-    if (dir) rc = dev_intt_locked(ctx, (const u64*)d, n, (u64*)dout, n, (u64*)scratch, n_log, k);
-    else rc = run_transform(ctx, (const u64*)d, n, (u64*)dout, n, (u64*)scratch, n_log, k, 0, false, nullptr, 0, false, true);
-    if (rc) return done(rc);
-    return done(d2h(ctx, data, dout, bytes));
+    if (dir) TRY(dev_intt_locked(ctx, d.get(), n, dout.get(), n, scratch.get(), n_log, k));
+    else TRY(run_transform(ctx, d.get(), n, dout.get(), n, scratch.get(), n_log, k, 0, false, nullptr, 0, false, true));
+    return d2h(ctx, data, dout.get(), bytes);
 }
 extern "C" int b200zkp_ntt(b200zkp_ctx* ctx, uint64_t* data, uint32_t n_log, uint32_t k) {
     if (!ctx) return B200ZKP_ERR_BAD_ARG;
@@ -2025,17 +1942,14 @@ extern "C" int b200zkp_coset_intt(b200zkp_ctx* ctx, uint64_t* data, uint32_t n_l
     if (!data) BAD(ctx, "null buffer");
     if (n_log > 32) BAD(ctx, "n_log exceeds two-adicity");
     size_t bytes = ((size_t)k << n_log) * 8;
-    void *d = nullptr, *scratch = nullptr, *dout = nullptr;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, bytes, &d)) || (rc = dev_alloc(ctx, bytes, &scratch)) || (rc = dev_alloc(ctx, bytes, &dout))) {
-        dev_release(ctx, d, bytes); dev_release(ctx, scratch, bytes);
-        return rc;
-    }
-    auto done = [&](int code) { dev_release(ctx, d, bytes); dev_release(ctx, scratch, bytes); dev_release(ctx, dout, bytes); return code; };
-    if ((rc = h2d(ctx, d, data, bytes))) return done(rc);
+    DevBuf d, scratch, dout;
+    TRY(d.alloc(ctx, bytes));
+    TRY(scratch.alloc(ctx, bytes));
+    TRY(dout.alloc(ctx, bytes));
+    TRY(h2d(ctx, d.get(), data, bytes));
     u64 n = (u64)1 << n_log;
-    if ((rc = dev_coset_intt_locked(ctx, (const u64*)d, n, (u64*)dout, n, (u64*)scratch, n_log, k, shift))) return done(rc);
-    return done(d2h(ctx, data, dout, bytes));
+    TRY(dev_coset_intt_locked(ctx, d.get(), n, dout.get(), n, scratch.get(), n_log, k, shift));
+    return d2h(ctx, data, dout.get(), bytes);
 }
 
 // natural-order coset LDE (an independent route from the leaf-order dev_lde: zero-pad, scale by 7^i,
@@ -2060,19 +1974,15 @@ extern "C" int b200zkp_coset_lde(b200zkp_ctx* ctx, const uint64_t* coeffs, uint3
         it = ctx->shift7_scale.emplace(N_log, d).first;
     }
     size_t big = (size_t)k * N * 8;
-    void *d_pad = nullptr, *d_scr = nullptr, *d_out = nullptr;
-    int rc = 0;
-    if ((rc = dev_alloc(ctx, big, &d_pad)) || (rc = dev_alloc(ctx, big, &d_scr)) || (rc = dev_alloc(ctx, big, &d_out))) {
-        dev_release(ctx, d_pad, big); dev_release(ctx, d_scr, big);
-        return rc;
-    }
-    auto done = [&](int code) { dev_release(ctx, d_pad, big); dev_release(ctx, d_scr, big); dev_release(ctx, d_out, big); return code; };
-    cudaError_t e = cudaMemsetAsync(d_pad, 0, big, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpy2DAsync(d_pad, N * 8, coeffs, n * 8, n * 8, k, cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("coset_lde H2D: ") + cudaGetErrorString(e); return done(B200ZKP_ERR_CUDA); }
-    rc = run_transform(ctx, (const u64*)d_pad, N, (u64*)d_out, N, (u64*)d_scr, N_log, k, 0, false, it->second, 0, false, true);
-    if (rc) return done(rc);
-    return done(d2h(ctx, out, d_out, big));
+    DevBuf d_pad, d_scr, d_out;
+    TRY(d_pad.alloc(ctx, big));
+    TRY(d_scr.alloc(ctx, big));
+    TRY(d_out.alloc(ctx, big));
+    cudaError_t e = cudaMemsetAsync(d_pad.get(), 0, big, ctx->stream);
+    if (e == cudaSuccess) e = cudaMemcpy2DAsync(d_pad.get(), N * 8, coeffs, n * 8, n * 8, k, cudaMemcpyHostToDevice, ctx->stream);
+    if (e != cudaSuccess) { ctx->err = std::string("coset_lde H2D: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    TRY(run_transform(ctx, d_pad.get(), N, d_out.get(), N, d_scr.get(), N_log, k, 0, false, it->second, 0, false, true));
+    return d2h(ctx, out, d_out.get(), big);
 }
 
 // ------------------------------------------------------------------------------------------------ field primitive probe
@@ -2100,16 +2010,14 @@ extern "C" int b200zkp_field_op(b200zkp_ctx* ctx, int op, const uint64_t* a, con
     Guard g(ctx);
     if (!count) return 0;
     if (!a || !b || !out || op < 0 || op > 7) BAD(ctx, "bad argument");
-    void* d_b = nullptr;
-    TRY(dev_alloc(ctx, count * 8, &d_b));
-    int rc = h2d(ctx, d_b, b, count * 8);
-    if (!rc) rc = with_io(ctx, a, count * 8, out, count * 8, [&](u64* da, u64* dout) -> int {
-        field_op_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(op, da, (const u64*)d_b, dout, count);
+    DevBuf d_b;
+    TRY(d_b.alloc(ctx, count * 8));
+    TRY(h2d(ctx, d_b.get(), b, count * 8));
+    return with_io(ctx, a, count * 8, out, count * 8, [&](u64* da, u64* dout) -> int {
+        field_op_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(op, da, d_b.get(), dout, count);
         LAUNCH_CHECK(ctx);
         return 0;
     });
-    dev_release(ctx, d_b, count * 8);
-    return rc;
 }
 
 // ------------------------------------------------------------------------------------------------ integer-pipe roof
@@ -2202,12 +2110,16 @@ extern "C" int b200zkp_int_pipe_bench(b200zkp_ctx* ctx, int kind, uint32_t iters
     if (!out_gips || kind < 0 || kind > 19) BAD(ctx, "bad argument");
     int sms = 0;
     CUDA_TRY(ctx, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-    u32* sink = nullptr;
-    TRY(dev_alloc(ctx, 8, (void**)&sink));
+    DevBuf sink_buf;
+    TRY(sink_buf.alloc(ctx, 8));
+    u32* sink = (u32*)sink_buf.get();
     unsigned blocks = (unsigned)sms * 8;
-    cudaEvent_t e0, e1;
-    CUDA_TRY(ctx, cudaEventCreate(&e0));
-    CUDA_TRY(ctx, cudaEventCreate(&e1));
+    struct Events {
+        cudaEvent_t e0 = nullptr, e1 = nullptr;
+        ~Events() { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); }
+    } ev;
+    CUDA_TRY(ctx, cudaEventCreate(&ev.e0));
+    CUDA_TRY(ctx, cudaEventCreate(&ev.e1));
     auto launch = [&](u32 n) {
         switch (kind) {
             case 0: int_pipe_kernel<0><<<blocks, 256, 0, ctx->stream>>>(n, sink); break;
@@ -2234,14 +2146,12 @@ extern "C" int b200zkp_int_pipe_bench(b200zkp_ctx* ctx, int kind, uint32_t iters
         ctx->launches++;
     };
     launch(iters / 8 + 1);  // warm-up
-    CUDA_TRY(ctx, cudaEventRecord(e0, ctx->stream));
+    CUDA_TRY(ctx, cudaEventRecord(ev.e0, ctx->stream));
     launch(iters);
-    CUDA_TRY(ctx, cudaEventRecord(e1, ctx->stream));
-    CUDA_TRY(ctx, cudaEventSynchronize(e1));
+    CUDA_TRY(ctx, cudaEventRecord(ev.e1, ctx->stream));
+    CUDA_TRY(ctx, cudaEventSynchronize(ev.e1));
     float ms = 0;
-    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, e0, e1));
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
-    dev_release(ctx, sink, 8);
+    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ev.e0, ev.e1));
     double instr = (double)blocks * 256.0 * (double)iters * 64.0 * (kind == 7 ? 2.0 : 1.0);   // 8 rounds x 8 instructions (x2 for the carry pair)
     *out_gips = instr / (ms * 1e-3) / 1e9;
     return 0;
@@ -2305,29 +2215,25 @@ extern "C" int b200zkp_dev_quotient_values(b200zkp_ctx* ctx, const b200zkp_vanis
     for (int i = 0; i < 4; i++) p.pi_hash[i] = gl_host_canon(d->public_inputs_hash[i]);
     TwoLevel tw{};
     TRY(get_tw(ctx, 0, Q_log, &tw));
-    void* d_pack = nullptr;
-    TRY(dev_alloc(ctx, pack.size() * 8, &d_pack));
-    int rc = h2d(ctx, d_pack, pack.data(), pack.size() * 8);
-    if (!rc) {
-        // (the pageable source is staged by the runtime before cudaMemcpyAsync returns)
-        p.cs = (const u64*)cs; p.wires = (const u64*)wires; p.zpp = (const u64*)zpp;
-        p.cs_stride = cs_stride; p.wires_stride = wires_stride; p.zpp_stride = zpp_stride;
-        p.n_log = d->degree_bits; p.q_bits = d->quotient_degree_bits;
-        p.num_selectors = d->num_selectors; p.num_gate_consts = 2; p.num_routed = R; p.num_challenges = Cn;
-        p.num_prods = chunks - 1; p.degree = deg; p.n_gates = d->n_gates;
-        p.k_is = (const u64*)d_pack;
-        p.alpha_pows = p.k_is + R;
-        p.zh = p.alpha_pows + (size_t)Cn * p.n_terms;
-        p.zh_inv = p.zh + qn;
-        p.tw_lo = tw.lo; p.tw_hi = tw.hi; p.tw_lo_bits = tw.lo_bits;
-        p.n_inv = hostgl::inv(n % hostgl::P);
-        p.out = (u64*)out_dev; p.out_stride = out_stride;
-        vanish::quotient_values_kernel<<<(unsigned)((Q + 127) / 128), 128, 0, ctx->stream>>>(p);
-        ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) { ctx->err = "quotient_values_kernel launch failed"; rc = B200ZKP_ERR_CUDA; }
-    }
-    dev_release(ctx, d_pack, pack.size() * 8);     // (stream ordered: the next user of this buffer runs after the kernel)
-    return rc;
+    DevBuf d_pack;
+    TRY(d_pack.alloc(ctx, pack.size() * 8));
+    TRY(h2d(ctx, d_pack.get(), pack.data(), pack.size() * 8));    // (the pageable source is staged by the runtime before cudaMemcpyAsync returns)
+    p.cs = (const u64*)cs; p.wires = (const u64*)wires; p.zpp = (const u64*)zpp;
+    p.cs_stride = cs_stride; p.wires_stride = wires_stride; p.zpp_stride = zpp_stride;
+    p.n_log = d->degree_bits; p.q_bits = d->quotient_degree_bits;
+    p.num_selectors = d->num_selectors; p.num_gate_consts = 2; p.num_routed = R; p.num_challenges = Cn;
+    p.num_prods = chunks - 1; p.degree = deg; p.n_gates = d->n_gates;
+    p.k_is = d_pack.get();
+    p.alpha_pows = p.k_is + R;
+    p.zh = p.alpha_pows + (size_t)Cn * p.n_terms;
+    p.zh_inv = p.zh + qn;
+    p.tw_lo = tw.lo; p.tw_hi = tw.hi; p.tw_lo_bits = tw.lo_bits;
+    p.n_inv = hostgl::inv(n % hostgl::P);
+    p.out = (u64*)out_dev; p.out_stride = out_stride;
+    vanish::quotient_values_kernel<<<(unsigned)((Q + 127) / 128), 128, 0, ctx->stream>>>(p);
+    ctx->launches++;
+    if (cudaGetLastError() != cudaSuccess) { ctx->err = "quotient_values_kernel launch failed"; return B200ZKP_ERR_CUDA; }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------ multi-GPU (NCCL)

@@ -79,11 +79,6 @@ class Context:
 
     STAGES = ("intt", "lde", "leaf_hash", "tree")
 
-    def set_overlap(self, enabled: bool):
-        """LDE / leaf-hash overlap on two streams.  Off by default: measured on B200, co-resident transform and hash
-        kernels time-slice the issue slots instead of overlapping (DESIGN.md section 7)."""
-        self.check(self._lib.b200zkp_ctx_set_overlap(self._h, int(enabled)))
-
     def trim(self):
         """Synchronise and hand every cached device buffer back to the driver (b200zkp_ctx_trim)."""
         self.check(self._lib.b200zkp_ctx_trim(self._h))
