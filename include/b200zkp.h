@@ -275,8 +275,10 @@ int b200zkp_dev_partial_products_and_zs(b200zkp_ctx* ctx, const uint64_t* wires_
  * each gate's selector polynomial and selector group (gates/selectors.rs), num_constants = num_selectors + 2 gate constants,
  * standard_recursion_config's 135 wires / 80 routed wires.  Gate types evaluated: NoopGate, ConstantGate (2 constants),
  * PublicInputGate, ArithmeticGate (20 ops), PoseidonGate, PoseidonMdsGate, BaseSumGate<B>, ArithmeticExtensionGate,
- * MulExtensionGate, ReducingGate, ReducingExtensionGate, RandomAccessGate, ExponentiationGate; any other kind
- * (InterpolationGate, the u32 / comparison gates) is B200ZKP_ERR_UNSUPPORTED (not silently skipped). */
+ * MulExtensionGate, ReducingGate, ReducingExtensionGate, RandomAccessGate, ExponentiationGate,
+ * HighDegreeInterpolationGate, LowDegreeInterpolationGate; any other kind (the u32 / comparison gates, id 13) is
+ * B200ZKP_ERR_UNSUPPORTED (not silently skipped).  The wire layouts are restated from memory of plonky2 @ f99ed9c
+ * (parity unpinned, as for every gate here; DESIGN.md section 4d). */
 enum { B200ZKP_GATE_NOOP = 0, B200ZKP_GATE_CONSTANT = 1, B200ZKP_GATE_PUBLIC_INPUT = 2, B200ZKP_GATE_ARITHMETIC = 3,
        B200ZKP_GATE_POSEIDON = 4,
        /* gates with parameters take them from gate_params[i] = { p0, p1, p2 } (Gate::new_from_config values in brackets) */
@@ -287,7 +289,21 @@ enum { B200ZKP_GATE_NOOP = 0, B200ZKP_GATE_CONSTANT = 1, B200ZKP_GATE_PUBLIC_INP
        B200ZKP_GATE_REDUCING_EXTENSION = 9,   /* ReducingExtensionGate: { num_coeffs } [32] */
        B200ZKP_GATE_RANDOM_ACCESS = 10,       /* RandomAccessGate: { bits, num_copies, num_extra_constants } [e.g. 4, 4, 2] */
        B200ZKP_GATE_EXPONENTIATION = 11,      /* ExponentiationGate: { num_power_bits } [66] */
-       B200ZKP_GATE_POSEIDON_MDS = 12 };      /* PoseidonMdsGate */
+       B200ZKP_GATE_POSEIDON_MDS = 12,        /* PoseidonMdsGate */
+       /* 13 is not assigned.  The interpolation gates (gates/interpolation.rs, low_degree_interpolation.rs) take
+        * { subgroup_bits }: m = 2^subgroup_bits points of the coset shift * <g>, g = the primitive 2^subgroup_bits-th root of
+        * unity (the NTT's); D = 2, ext(j) = wires j, j + 1 as one element of F[X]/(X^2 - 7).  Shared layout: wire 0 the
+        * shift; value(i) = ext(1 + D i), i < m; evaluation point ext(1 + D m); evaluation value ext(3 + D m); coeff(i) =
+        * ext(5 + D m + D i), i < m; end_coeffs = 5 + 4m; the first 5 + 2m wires are routed. */
+       B200ZKP_GATE_INTERPOLATION_HIGH_DEGREE = 14, /* HighDegreeInterpolationGate { subgroup_bits 1..5 }: constraints
+        * value(i) - interpolant(shift g^i) for i < m, then eval_value - interpolant(eval_point), D components each:
+        * D (m + 1) constraints, 5 + 4m wires, degree m (a FRI arity <= 8) */
+       B200ZKP_GATE_INTERPOLATION_LOW_DEGREE = 15 };  /* LowDegreeInterpolationGate { subgroup_bits 1..4 }: also
+        * shift_pow(i) = wire end_coeffs + i - 2 and eval_pow(i) = ext(end_coeffs + m - 2 + D (i - 2)) for 2 <= i < m
+        * (shift_pow(1) = shift, eval_pow(1) = eval_point).  Constraints: shift_pow(i-1) shift - shift_pow(i), 2 <= i < m;
+        * value(i) - sum_j c_j shift_pow(j) g^(ij), i < m (shift_pow(0) = 1); eval_pow(i-1) eval_point - eval_pow(i),
+        * 2 <= i < m; eval_value - (c_0 + sum_(i>=1) c_i eval_pow(i)): 5m - 4 constraints, 7m - 1 wires, degree 2 (what
+        * standard_recursion_config's arity-16 FRI verifier instantiates, subgroup_bits 4) */
 #define B200ZKP_MAX_GATES 16
 typedef struct {
     uint32_t degree_bits;               /* n = 2^degree_bits rows */

@@ -2177,9 +2177,11 @@ extern "C" int b200zkp_dev_quotient_values(b200zkp_ctx* ctx, const b200zkp_vanis
     u32 max_constraints = 0;
     for (u32 i = 0; i < d->n_gates; i++) {
         const u32 kind = d->gate_kind[i];
-        if (kind >= vanish::N_GATE_KINDS) { ctx->err = "gate kind not supported by the device evaluator"; return B200ZKP_ERR_UNSUPPORTED; }
+        if (!vanish::gate_supported(kind)) { ctx->err = "gate kind not supported by the device evaluator"; return B200ZKP_ERR_UNSUPPORTED; }
         const u32 p0 = d->gate_params[i][0], p1 = d->gate_params[i][1], p2 = d->gate_params[i][2];
         if ((kind == vanish::GATE_BASE_SUM && (p0 < 2 || p0 > 64 || p1 == 0)) ||
+            (kind == vanish::GATE_INTERPOLATION_HIGH_DEGREE && (p0 == 0 || p0 > 5)) ||
+            (kind == vanish::GATE_INTERPOLATION_LOW_DEGREE && (p0 == 0 || p0 > 4)) ||
             ((kind == vanish::GATE_REDUCING || kind == vanish::GATE_REDUCING_EXTENSION || kind == vanish::GATE_EXPONENTIATION) && (p0 == 0 || p0 > 128)) ||
             (kind == vanish::GATE_RANDOM_ACCESS && (p0 == 0 || p0 > 6 || p1 == 0 || p1 > 64 || p2 > 2)) ||
             vanish::gate_num_wires(kind, R, p0, p1, p2) > 135)

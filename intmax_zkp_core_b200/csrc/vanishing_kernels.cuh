@@ -5,7 +5,7 @@
 // `evaluate_gate_constraints_base_batch`, plonk_common.rs `ZeroPolyOnCoset`, `eval_l_1`, `reduce_with_powers`,
 // gates/selectors.rs `compute_filter` and the eval_unfiltered of gates/{noop, constant, public_input, arithmetic_base,
 // poseidon, poseidon_mds, base_sum, arithmetic_extension, multiplication_extension, reducing, reducing_extension,
-// random_access, exponentiation}.rs.  Reached from the reference through every prove() (/root/reference/src/rollup/circuits/mod.rs:1247,
+// random_access, exponentiation, interpolation, low_degree_interpolation}.rs.  Reached from the reference through every prove() (/root/reference/src/rollup/circuits/mod.rs:1247,
 // src/transaction/circuits/mod.rs:453, src/zkdsa/circuits/mod.rs:326); PoseidonGate is what
 // /root/reference/src/poseidon/gadgets/mod.rs:7-22 instantiates.  Restated in oracle/vanishing_ref.py (parity unpinned: the
 // crate source is not on this machine; the verifier's identity pins the restatement, tests/test_oracle_vanishing.py).
@@ -35,7 +35,9 @@ enum GateKind : u32 {
     GATE_RANDOM_ACCESS = 10,         // params (bits, num_copies, num_extra_constants)
     GATE_EXPONENTIATION = 11,        // params (num_power_bits): base, power bits, output, intermediate values
     GATE_POSEIDON_MDS = 12,          // 12 extension inputs, 12 extension outputs
-    N_GATE_KINDS = 13
+    // (13 is not assigned)
+    GATE_INTERPOLATION_HIGH_DEGREE = 14,   // params (subgroup_bits): m = 2^subgroup_bits points, degree m
+    GATE_INTERPOLATION_LOW_DEGREE = 15     // params (subgroup_bits): the same with power wires, degree 2
 };
 static constexpr u32 D = 2;          // quadratic extension F[X] / (X^2 - 7)
 static constexpr u32 MAX_GATES = 16, MAX_CHALLENGES = 4;
@@ -43,7 +45,16 @@ static constexpr u32 UNUSED_SELECTOR = 0xFFFFFFFFu;
 // PoseidonGate wire layout (gates/poseidon.rs)
 static constexpr u32 W_IN = 0, W_OUT = 12, W_SWAP = 24, W_DELTA = 25, W_FULL0 = 29, W_PARTIAL = 65, W_FULL1 = 87;
 
+// InterpolationGate layout (gates/interpolation.rs, low_degree_interpolation.rs), m = 2^subgroup_bits, ext(j) = wires j, j + 1:
+// shift 0, value(i) ext(1 + D i), evaluation point ext(1 + D m), evaluation value ext(3 + D m), coeff(i) ext(5 + D m + D i), up
+// to end_coeffs = 5 + 4 m; LowDegree only: shift^i at end_coeffs + i - 2 and ext eval_point^i at end_coeffs + m - 2 + D (i - 2)
+// for 2 <= i < m
+
 struct GateDesc { u32 kind, selector_index, group_begin, group_end, p0, p1, p2; };
+
+GL_HD bool gate_supported(u32 kind) {
+    return kind <= GATE_POSEIDON_MDS || kind == GATE_INTERPOLATION_HIGH_DEGREE || kind == GATE_INTERPOLATION_LOW_DEGREE;
+}
 
 // Gate::num_constraints() of standard_recursion_config instances (host and device)
 GL_HD u32 gate_num_constraints(u32 kind, u32 num_routed, u32 num_gate_consts, u32 p0, u32 p1, u32 p2) {
@@ -59,6 +70,8 @@ GL_HD u32 gate_num_constraints(u32 kind, u32 num_routed, u32 num_gate_consts, u3
         case GATE_RANDOM_ACCESS: return p1 * (p0 + 2) + p2;
         case GATE_EXPONENTIATION: return p0 + 1;
         case GATE_POSEIDON_MDS: return 12 * D;
+        case GATE_INTERPOLATION_HIGH_DEGREE: return D * ((1u << p0) + 1);
+        case GATE_INTERPOLATION_LOW_DEGREE: return 5 * (1u << p0) - 4;
         default: return 0;
     }
 }
@@ -72,6 +85,8 @@ GL_HD u32 gate_num_wires(u32 kind, u32 num_routed, u32 p0, u32 p1, u32 p2) {
         case GATE_EXPONENTIATION: return 2 + 2 * p0;
         case GATE_POSEIDON_MDS: return 24 * D;
         case GATE_POSEIDON: return 135;
+        case GATE_INTERPOLATION_HIGH_DEGREE: return 5 + 4 * (1u << p0);
+        case GATE_INTERPOLATION_LOW_DEGREE: return 7 * (1u << p0) - 1;
         default: return num_routed;
     }
 }
@@ -133,6 +148,14 @@ GL_FN void mds_layer(u64 (&s)[12]) {
     }
 #pragma unroll
     for (int r = 0; r < 12; r++) s[r] = o[r];
+}
+
+// primitive 2^bits-th root of unity, the one the NTT uses: G^(2^(32 - bits)) for the generator G of the 2^32 subgroup
+GL_FN u64 root_of_unity(u32 bits) {
+    u64 g = 1753635133440165772ull;
+#pragma unroll 1
+    for (u32 k = bits; k < 32; k++) g = gl::mul(g, g);
+    return g;
 }
 
 // running sums of one gate's constraints, one per challenge
@@ -406,6 +429,58 @@ GL_FN void quotient_point(const Params& p, u64 t) {
                     f.add(gl::sub(wire(D * (12 + q)), s0[q]));
                     f.add(gl::sub(wire(D * (12 + q) + 1), s1[q]));
                 }
+                break;
+            }
+            case GATE_INTERPOLATION_HIGH_DEGREE:
+            case GATE_INTERPOLATION_LOW_DEGREE: {                     // gates/interpolation.rs, low_degree_interpolation.rs
+                // The coefficient wires are re-read from memory where they are used (not held: 2m words).  LowDegree uses its
+                // power wires exactly where plonky2 does: off the trace the wires do not satisfy the power relations, so
+                // recomputed powers would give different quotient values.
+                const u32 m = 1u << gd.p0, w_coeffs = 5 + D * m, end_coeffs = w_coeffs + D * m;
+                const bool low = gd.kind == GATE_INTERPOLATION_LOW_DEGREE;
+                const u64 shift = wire(0), g_sub = root_of_unity(gd.p0);
+                auto shift_pow = [&](u32 j) { return j == 0 ? (u64)1 : j == 1 ? shift : wire(end_coeffs + j - 2); };
+                auto eval_pow = [&](u32 j) { return j == 1 ? ext(1 + D * m) : ext(end_coeffs + (m - 2) + D * (j - 2)); };
+                if (low) {
+#pragma unroll 1
+                    for (u32 q = 2; q < m; q++) f.add(gl::sub(gl::mul(shift_pow(q - 1), shift), shift_pow(q)));
+                }
+                // value(i) - interpolant(shift g^i); LowDegree: with the coefficients c_j shift^j at the point g^i (Horner)
+                u64 g_i = 1;
+#pragma unroll 1
+                for (u32 q = 0; q < m; q++) {
+                    const u64 x_q = low ? g_i : gl::mul(shift, g_i);
+                    E2 v{0, 0};
+#pragma unroll 1
+                    for (u32 j = m; j-- > 0;) {
+                        const E2 c = low ? e2_scale(ext(w_coeffs + D * j), shift_pow(j)) : ext(w_coeffs + D * j);
+                        v = e2_add(e2_scale(v, x_q), c);
+                    }
+                    const E2 r = e2_sub(ext(1 + D * q), v);
+                    f.add(r.a); f.add(r.b);
+                    g_i = gl::mul(g_i, g_sub);
+                }
+                // evaluation value - interpolant(evaluation point); LowDegree: c_0 + sum_j c_j eval_point^j with the power wires
+                const E2 point = ext(1 + D * m);
+                E2 v;
+                if (low) {
+                    E2 prev = point;
+#pragma unroll 1
+                    for (u32 q = 2; q < m; q++) {
+                        const E2 cur = eval_pow(q), r = e2_sub(e2_mul(prev, point), cur);
+                        f.add(r.a); f.add(r.b);
+                        prev = cur;
+                    }
+                    v = ext(w_coeffs);
+#pragma unroll 1
+                    for (u32 j = 1; j < m; j++) v = e2_add(v, e2_mul(ext(w_coeffs + D * j), eval_pow(j)));
+                } else {
+                    v = E2{0, 0};
+#pragma unroll 1
+                    for (u32 j = m; j-- > 0;) v = e2_add(e2_mul(v, point), ext(w_coeffs + D * j));
+                }
+                const E2 r = e2_sub(ext(3 + D * m), v);
+                f.add(r.a); f.add(r.b);
                 break;
             }
             default: break;

@@ -163,6 +163,7 @@ def commit_quotient_device(ctx: Context, quotient_values, degree_bits: int, rate
 GATE_NOOP, GATE_CONSTANT, GATE_PUBLIC_INPUT, GATE_ARITHMETIC, GATE_POSEIDON = range(5)
 (GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_BASE_SUM, GATE_REDUCING, GATE_REDUCING_EXTENSION, GATE_RANDOM_ACCESS,
  GATE_EXPONENTIATION, GATE_POSEIDON_MDS) = range(5, 13)
+GATE_INTERPOLATION_HIGH_DEGREE, GATE_INTERPOLATION_LOW_DEGREE = 14, 15         # (13 is not assigned)
 MAX_GATES = 16
 
 
@@ -182,7 +183,9 @@ class CommonCircuitData:
     the selector polynomial and selector group of every gate (SelectorsInfo), quotient_degree_factor, k_is.
     gates: [(kind, selector_index, (group_begin, group_end)[, params]), ...]; params: the gate's own parameters
     (BaseSum (B, num_limbs), Reducing / ReducingExtension (num_coeffs,), RandomAccess (bits, num_copies, num_extra_constants),
-    Exponentiation (num_power_bits,))"""
+    Exponentiation (num_power_bits,), HighDegreeInterpolation (subgroup_bits,) with subgroup_bits 1..5,
+    LowDegreeInterpolation (subgroup_bits,) with subgroup_bits 1..4).  The u32 and comparison gates are refused
+    (B200ZkpError with code -4); the interpolation layouts are restated from memory as for the other gates (include/b200zkp.h)"""
 
     def __init__(self, degree_bits: int, gates, num_selectors: int, quotient_degree_factor: int = 8, num_routed_wires: int = 80,
                  k_is=None):

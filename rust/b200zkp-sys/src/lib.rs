@@ -26,6 +26,9 @@ pub const B200ZKP_GATE_REDUCING_EXTENSION: u32 = 9; // { num_coeffs }
 pub const B200ZKP_GATE_RANDOM_ACCESS: u32 = 10; // { bits, num_copies, num_extra_constants }
 pub const B200ZKP_GATE_EXPONENTIATION: u32 = 11; // { num_power_bits }
 pub const B200ZKP_GATE_POSEIDON_MDS: u32 = 12;
+// 13 is not assigned
+pub const B200ZKP_GATE_INTERPOLATION_HIGH_DEGREE: u32 = 14;
+pub const B200ZKP_GATE_INTERPOLATION_LOW_DEGREE: u32 = 15;
 
 /// include/b200zkp.h `b200zkp_vanishing_desc` (row N1b: what compute_quotient_polys reads of CommonCircuitData)
 #[repr(C)]
