@@ -14,6 +14,7 @@
 #include <mutex>
 #include <optional>
 #include <string>
+#include <tuple>
 #include <vector>
 
 #include "merkle_kernels.cuh"
@@ -45,17 +46,14 @@ struct b200zkp_ctx {
     u64 launches = 0;
     u64* wtab[2][ntt::MAX_PASS_BITS + 1] = {};          // [dir][B] w_{2^B}^(+-e)
     std::map<u32, TwoLevel> tw[2];                      // [dir][n_log] -> w_n^(+-e)
-    std::map<u64, std::vector<TwoLevel>> coset;         // (n_log<<8 | rate_bits) -> per leaf block (builder input)
-    std::map<u32, TwoLevel> shift7;                     // N_log -> 7^i (natural-order coset_lde helper, builder input)
     // direct tables read by the pass kernels
     struct Images { const u64* img[ntt::MAX_PASSES] = {}; };
-    std::map<u64, Images> twimg;                        // (n_log<<8 | dir<<1 | bitrev_out) -> twiddle image per pass
-    std::map<u64, u64*> coset_scale;                    // (n_log<<8 | rate_bits) -> [2^rate_bits][n] shift powers
-    std::map<u32, u64*> shift7_scale;                   // N_log -> 7^i, i < N
-    std::map<std::pair<u64, u32>, u64*> power_scale;    // (shift, bits) -> shift^i, i < 2^bits (FRI layer cosets)
+    std::map<std::tuple<u32, int, bool>, Images> twimg; // (n_log, dir, bitrev_out) -> twiddle image per pass
+    std::map<std::pair<u32, u32>, const u64*> coset_scale;   // (n_log, rate_bits) -> [2^rate_bits][n] shift powers
+    std::map<std::pair<u64, u32>, const u64*> power_scale;   // (shift, bits) -> shift^i, i < 2^bits (coset transforms)
     // second-generation passes (ntt_ct_kernels.cuh): block-twiddle tables Z, [n_blk][n] each
     struct ZTables { const u64* strided = nullptr; const u64* final_ = nullptr; };   // see ntc::ztab_entries / zfinal_words
-    std::map<u64, ZTables> ztab_lde;                    // (n_log<<8 | rate_bits) -> forward transform on every leaf block's coset
+    std::map<std::pair<u32, u32>, ZTables> ztab_lde;    // (n_log, rate_bits) -> forward transform on every leaf block's coset
     std::map<u32, ZTables> ztab_inv;                    // n_log -> inverse transform (s = 1), last level carries n^-1
     bool ntt_ct = true;                                 // B200ZKP_NTT_CT=0: every transform through ntt_kernels.cuh (A/B testing)
     bool ntt_tma = true;                                // B200ZKP_NTT_TMA=0: the new passes stage their tiles with plain loads
@@ -72,7 +70,7 @@ struct b200zkp_ctx {
     size_t pool_bytes = 0;
     size_t live_bytes = 0;                              // handed out by DevBuf::alloc and not yet returned (b200zkp_ctx_buffer_bytes)
     size_t pool_max_bytes = (size_t)16 << 30;         // reset to 1/8 of the device memory in ctx_create
-    std::vector<void*> table_allocs;
+    std::vector<void*> table_allocs;                    // the cached tables above and round_add, freed with the ctx
     // second, higher-priority stream: host uploads and copy-back beside the main stream (ensure_stream2)
     cudaStream_t stream2 = nullptr;
     std::vector<cudaEvent_t> sync_events;
@@ -118,11 +116,13 @@ struct StreamScope {
     ~StreamScope() { c->stream = saved; }
 };
 
+// (clears the thread's last error, so that a failure is reported by its own call only)
 #define CUDA_TRY(ctx, expr)                                                                   \
     do {                                                                                      \
         cudaError_t e__ = (expr);                                                             \
         if (e__ != cudaSuccess) {                                                             \
             (ctx)->err = std::string(#expr) + ": " + cudaGetErrorString(e__);                 \
+            (void)cudaGetLastError();                                                         \
             return e__ == cudaErrorMemoryAllocation ? B200ZKP_ERR_OOM : B200ZKP_ERR_CUDA;     \
         }                                                                                     \
     } while (0)
@@ -254,49 +254,81 @@ static bool log2_exact(u64 n, u32* lg) {
     return true;
 }
 
+// device memory kept for the life of the ctx
+static int table_alloc(b200zkp_ctx* ctx, u64 count, u64** out) {
+    CUDA_TRY(ctx, cudaMalloc((void**)out, count * sizeof(u64)));
+    ctx->table_allocs.push_back(*out);
+    return 0;
+}
+
 static int upload(b200zkp_ctx* ctx, const std::vector<u64>& h, u64** d) {
-    CUDA_TRY(ctx, cudaMalloc((void**)d, h.size() * sizeof(u64)));
-    ctx->table_allocs.push_back(*d);
-    CUDA_TRY(ctx, cudaMemcpyAsync(*d, h.data(), h.size() * sizeof(u64), cudaMemcpyHostToDevice, ctx->stream));
+    TRY(table_alloc(ctx, h.size(), d));
+    TRY(h2d(ctx, *d, h.data(), h.size() * sizeof(u64)));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 
-static int make_two_level(b200zkp_ctx* ctx, u64 base, u32 bits, TwoLevel* t) {
-    std::vector<u64> lo, hi;
-    t->lo_bits = hostgl::two_level_powers(base, bits, &lo, &hi);
-    TRY(upload(ctx, lo, &t->lo));
-    TRY(upload(ctx, hi, &t->hi));
-    return 0;
-}
-
-static int get_tw(b200zkp_ctx* ctx, int dir, u32 n_log, TwoLevel* out) {
-    auto it = ctx->tw[dir].find(n_log);
-    if (it == ctx->tw[dir].end()) {
-        u64 w = hostgl::root(n_log);
-        if (dir) w = hostgl::inv(w);
-        TwoLevel t;
-        TRY(make_two_level(ctx, w, n_log, &t));
-        it = ctx->tw[dir].emplace(n_log, t).first;
+// *out = the table cached under `key`, built by build(&table) on first use (a failed build caches nothing)
+template <typename Map, typename Build>
+static int get_or_build(Map& cache, const typename Map::key_type& key, typename Map::mapped_type* out, Build build) {
+    auto it = cache.find(key);
+    if (it == cache.end()) {
+        typename Map::mapped_type t{};
+        TRY(build(&t));
+        it = cache.emplace(key, t).first;
     }
     *out = it->second;
     return 0;
 }
 
-// per leaf block b of the LDE: powers of s_b = 7 * w_N^bitrev(b, rate_bits)
-static int get_coset(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, const std::vector<TwoLevel>** out) {
-    u64 key = ((u64)n_log << 8) | rate_bits;
-    auto it = ctx->coset.find(key);
-    if (it == ctx->coset.end()) {
-        std::vector<TwoLevel> v((size_t)1 << rate_bits);
-        for (u32 b = 0; b < (1u << rate_bits); b++) {
-            u64 s = hostgl::coset_shift_of_block(n_log, rate_bits, b);
-            TRY(make_two_level(ctx, s, n_log, &v[b]));
-        }
-        it = ctx->coset.emplace(key, std::move(v)).first;
-    }
-    *out = &it->second;
+static int get_tw(b200zkp_ctx* ctx, int dir, u32 n_log, TwoLevel* out) {
+    return get_or_build(ctx->tw[dir], n_log, out, [&](TwoLevel* t) -> int {
+        const u64 w = hostgl::root(n_log);
+        std::vector<u64> lo, hi;
+        t->lo_bits = hostgl::two_level_powers(dir ? hostgl::inv(w) : w, n_log, &lo, &hi);
+        TRY(upload(ctx, lo, &t->lo));
+        return upload(ctx, hi, &t->hi);
+    });
+}
+
+// dst[i] = base^i, i < 2^bits.  The two-level input lives only for the build: the stream is synchronised before it goes
+// back to the pool, so the build is safe on whichever stream ctx->stream is.
+static int fill_powers(b200zkp_ctx* ctx, u64 base, u32 bits, u64* dst) {
+    std::vector<u64> lo, hi;
+    const u32 lo_bits = hostgl::two_level_powers(base, bits, &lo, &hi);
+    DevBuf d_lo, d_hi;
+    TRY(d_lo.alloc(ctx, lo.size() * 8));
+    TRY(d_hi.alloc(ctx, hi.size() * 8));
+    TRY(h2d(ctx, d_lo.get(), lo.data(), d_lo.bytes()));
+    TRY(h2d(ctx, d_hi.get(), hi.data(), d_hi.bytes()));
+    const u64 n = (u64)1 << bits;
+    ntt::build_powers_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(dst, n, d_lo.get(), d_hi.get(), lo_bits);
+    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+
+// powers shift^i, i < 2^bits (scale table of a coset transform)
+static int get_power_scale(b200zkp_ctx* ctx, u64 shift, u32 bits, const u64** out) {
+    return get_or_build(ctx->power_scale, std::make_pair(shift, bits), out, [&](const u64** t) -> int {
+        u64* d = nullptr;
+        TRY(table_alloc(ctx, (u64)1 << bits, &d));
+        *t = d;
+        return fill_powers(ctx, shift, bits, d);
+    });
+}
+
+// [2^rate_bits][n]: row b holds the powers of the coset shift of leaf block b, s_b = 7 * w_N^bitrev(b, rate_bits)
+static int get_coset_scale(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, const u64** out) {
+    return get_or_build(ctx->coset_scale, std::make_pair(n_log, rate_bits), out, [&](const u64** t) -> int {
+        const u64 n = (u64)1 << n_log;
+        u64* d = nullptr;
+        TRY(table_alloc(ctx, n << rate_bits, &d));
+        for (u32 b = 0; b < (1u << rate_bits); b++)
+            TRY(fill_powers(ctx, hostgl::coset_shift_of_block(n_log, rate_bits, b), n_log, d + (u64)b * n));
+        *t = d;
+        return 0;
+    });
 }
 
 template <int B>
@@ -339,60 +371,28 @@ static int launch_canon_copy(b200zkp_ctx* ctx, const u64* src, u64* dst, u64 cou
     return 0;
 }
 
-static int table_alloc(b200zkp_ctx* ctx, u64 count, u64** out) {
-    CUDA_TRY(ctx, cudaMalloc((void**)out, count * sizeof(u64)));
-    ctx->table_allocs.push_back(*out);
-    return 0;
-}
-
 // twiddle images of every non-final pass of a 2^n_log transform (built on the device, cached per ctx);
 // the inverse direction carries n^-1 in the first image
 static int get_twiddle_images(b200zkp_ctx* ctx, u32 n_log, int dir, bool bitrev_out, b200zkp_ctx::Images* out) {
-    u64 key = ((u64)n_log << 8) | ((u64)dir << 1) | (bitrev_out ? 1 : 0);
-    auto it = ctx->twimg.find(key);
-    if (it == ctx->twimg.end()) {
-        b200zkp_ctx::Images im;
+    return get_or_build(ctx->twimg, std::make_tuple(n_log, dir, bitrev_out), out, [&](b200zkp_ctx::Images* im) -> int {
         ntt::TwiddleImageShape shapes[ntt::MAX_PASSES];
         u32 n_img = ntt::twiddle_images(n_log, shapes);
-        if (n_img) {
-            TwoLevel tw{};
-            TRY(get_tw(ctx, dir, n_log, &tw));
-            u64 n_inv = hostgl::inv(((u64)1 << n_log) % hostgl::P);
-            for (u32 pi = 0; pi < n_img; pi++) {
-                u64 count = (u64)1 << (shapes[pi].B + shapes[pi].C_log);
-                u64* d = nullptr;
-                TRY(table_alloc(ctx, count, &d));
-                u64 f = (dir == 1 && pi == 0) ? n_inv : 0;
-                ntt::build_twiddle_image_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(
-                    d, shapes[pi].B, shapes[pi].C_log, shapes[pi].shift, bitrev_out ? 1u : 0u, f, tw.lo, tw.hi, tw.lo_bits);
-                LAUNCH_CHECK(ctx);
-                im.img[pi] = d;
-            }
-        }
-        it = ctx->twimg.emplace(key, im).first;
-    }
-    *out = it->second;
-    return 0;
-}
-
-// [2^rate_bits][n] powers of the coset shift of every leaf block
-static int get_coset_scale(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, const u64** out) {
-    u64 key = ((u64)n_log << 8) | rate_bits;
-    auto it = ctx->coset_scale.find(key);
-    if (it == ctx->coset_scale.end()) {
-        const std::vector<TwoLevel>* cs;
-        TRY(get_coset(ctx, n_log, rate_bits, &cs));
-        u64 n = (u64)1 << n_log;
-        u64* d = nullptr;
-        TRY(table_alloc(ctx, n << rate_bits, &d));
-        for (u32 b = 0; b < (1u << rate_bits); b++) {
-            ntt::build_powers_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d + (u64)b * n, n, (*cs)[b].lo, (*cs)[b].hi, (*cs)[b].lo_bits);
+        if (!n_img) return 0;
+        TwoLevel tw{};
+        TRY(get_tw(ctx, dir, n_log, &tw));
+        u64 n_inv = hostgl::inv(((u64)1 << n_log) % hostgl::P);
+        for (u32 pi = 0; pi < n_img; pi++) {
+            u64 count = (u64)1 << (shapes[pi].B + shapes[pi].C_log);
+            u64* d = nullptr;
+            TRY(table_alloc(ctx, count, &d));
+            u64 f = (dir == 1 && pi == 0) ? n_inv : 0;
+            ntt::build_twiddle_image_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(
+                d, shapes[pi].B, shapes[pi].C_log, shapes[pi].shift, bitrev_out ? 1u : 0u, f, tw.lo, tw.hi, tw.lo_bits);
             LAUNCH_CHECK(ctx);
+            im->img[pi] = d;
         }
-        it = ctx->coset_scale.emplace(key, d).first;
-    }
-    *out = it->second;
-    return 0;
+        return 0;
+    });
 }
 
 // ---- second-generation passes: Z tables, tensor maps, launches
@@ -511,7 +511,8 @@ static int run_ct_plan(b200zkp_ctx* ctx, ntc::Plan& plan, cudaStream_t later_str
     return 0;
 }
 
-// Z tables of `n_blk` cosets s_b <w_n>: shifts[b] on the host; built on the device and kept for the life of the ctx
+// Z tables of `n_blk` cosets s_b <w_n>: shifts[b] on the host; built on the device and kept for the life of the ctx.
+// The squared shifts are a build input only: the stream is synchronised before they go back to the pool.
 static int build_ztab(b200zkp_ctx* ctx, u32 n_log, int dir, const std::vector<u64>& shifts, u64 last_scale, bool natural,
                       b200zkp_ctx::ZTables* out) {
     TwoLevel tw{};
@@ -521,46 +522,37 @@ static int build_ztab(b200zkp_ctx* ctx, u32 n_log, int dir, const std::vector<u6
         u64 x = shifts[b] % hostgl::P;
         for (u32 e = 0; e < n_log; e++) { spow[b * n_log + e] = x; x = hostgl::mul(x, x); }
     }
-    u64* d_spow = nullptr;
-    TRY(upload(ctx, spow, &d_spow));
+    DevBuf d_spow;
+    TRY(d_spow.alloc(ctx, spow.size() * 8));
+    TRY(h2d(ctx, d_spow.get(), spow.data(), d_spow.bytes()));
     const u64 count = ntc::ztab_entries(n_log), words = ntc::zfinal_words(n_log);
     u64 *d = nullptr, *f = nullptr;
     TRY(table_alloc(ctx, count * shifts.size(), &d));
     TRY(table_alloc(ctx, words * shifts.size(), &f));
     ntc::build_ztab_kernel<<<dim3((unsigned)((count + 255) / 256), (unsigned)shifts.size()), 256, 0, ctx->stream>>>(
-        d, count, n_log, d_spow, tw.lo, tw.hi, tw.lo_bits, last_scale);
+        d, count, n_log, d_spow.get(), tw.lo, tw.hi, tw.lo_bits, last_scale);
     LAUNCH_CHECK(ctx);
     ntc::build_zfinal_kernel<<<dim3((unsigned)((words + 255) / 256), (unsigned)shifts.size()), 256, 0, ctx->stream>>>(
-        f, words, n_log, ntc::last_pass_bits(n_log), natural ? 1u : 0u, d_spow, tw.lo, tw.hi, tw.lo_bits, last_scale);
+        f, words, n_log, ntc::last_pass_bits(n_log), natural ? 1u : 0u, d_spow.get(), tw.lo, tw.hi, tw.lo_bits, last_scale);
     LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     out->strided = d;
     out->final_ = f;
     return 0;
 }
 
 static int get_ztab_lde(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, b200zkp_ctx::ZTables* out) {
-    const u64 key = ((u64)n_log << 8) | rate_bits;
-    auto it = ctx->ztab_lde.find(key);
-    if (it == ctx->ztab_lde.end()) {
+    return get_or_build(ctx->ztab_lde, std::make_pair(n_log, rate_bits), out, [&](b200zkp_ctx::ZTables* t) {
         std::vector<u64> shifts;
         for (u32 b = 0; b < (1u << rate_bits); b++) shifts.push_back(hostgl::coset_shift_of_block(n_log, rate_bits, b));
-        b200zkp_ctx::ZTables t;
-        TRY(build_ztab(ctx, n_log, 0, shifts, 0, /*natural=*/false, &t));
-        it = ctx->ztab_lde.emplace(key, t).first;
-    }
-    *out = it->second;
-    return 0;
+        return build_ztab(ctx, n_log, 0, shifts, 0, /*natural=*/false, t);
+    });
 }
 
 static int get_ztab_inv(b200zkp_ctx* ctx, u32 n_log, b200zkp_ctx::ZTables* out) {
-    auto it = ctx->ztab_inv.find(n_log);
-    if (it == ctx->ztab_inv.end()) {
-        b200zkp_ctx::ZTables t;
-        TRY(build_ztab(ctx, n_log, 1, std::vector<u64>{1}, hostgl::inv(((u64)1 << n_log) % hostgl::P), /*natural=*/true, &t));
-        it = ctx->ztab_inv.emplace(n_log, t).first;
-    }
-    *out = it->second;
-    return 0;
+    return get_or_build(ctx->ztab_inv, n_log, out, [&](b200zkp_ctx::ZTables* t) {
+        return build_ztab(ctx, n_log, 1, std::vector<u64>{1}, hostgl::inv(((u64)1 << n_log) % hostgl::P), /*natural=*/true, t);
+    });
 }
 
 // One multi-pass transform over `ncols` columns, for `n_blk` blocks at once (blockIdx.y: the coset blocks of an
@@ -1040,27 +1032,24 @@ static int commit_host(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log
     // and extended on the main stream (columns are independent until the leaf hash), so the 8nk-byte H2D hides behind
     // the transforms when the caller's buffer is pinned.
     TRY(ensure_stream2(ctx));
-    cudaError_t e = cudaSuccess;
     const u32 n_chunks = (k >= 16 && d_in.bytes() >= ((size_t)64 << 20)) ? 8 : 1;
     const u32 per = (k + n_chunks - 1) / n_chunks;
     cudaEvent_t e_free;
     TRY(get_sync_event(ctx, 0, &e_free));
     // d_in / lde may be recycled buffers still in use by earlier work on the main stream
-    if (cudaEventRecord(e_free, ctx->stream) != cudaSuccess || cudaStreamWaitEvent(ctx->stream2, e_free, 0) != cudaSuccess) {
-        (void)cudaGetLastError(); ctx->err = "event error"; return B200ZKP_ERR_CUDA;
-    }
-    if (salt) e = cudaMemcpyAsync(d_salt.get(), salt, d_salt.bytes(), cudaMemcpyHostToDevice, ctx->stream2);
+    CUDA_TRY(ctx, cudaEventRecord(e_free, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, e_free, 0));
+    if (salt) CUDA_TRY(ctx, cudaMemcpyAsync(d_salt.get(), salt, d_salt.bytes(), cudaMemcpyHostToDevice, ctx->stream2));
     std::vector<cudaEvent_t> up(n_chunks);
-    for (u32 c = 0; c < n_chunks && e == cudaSuccess; c++) {
-        u32 c0 = std::min(k, c * per), c1 = std::min(k, (c + 1) * per);
-        TRY(get_sync_event(ctx, 1 + c, &up[c]));
-        if (c1 > c0) e = cudaMemcpyAsync(d_in.get() + (u64)c0 * n, in + (u64)c0 * n, (size_t)(c1 - c0) * n * 8, cudaMemcpyHostToDevice, ctx->stream2);
-        if (e == cudaSuccess) e = cudaEventRecord(up[c], ctx->stream2);
-    }
-    if (e != cudaSuccess) { ctx->err = std::string("H2D: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
     for (u32 c = 0; c < n_chunks; c++) {
         u32 c0 = std::min(k, c * per), c1 = std::min(k, (c + 1) * per);
-        if (cudaStreamWaitEvent(ctx->stream, up[c], 0) != cudaSuccess) { (void)cudaGetLastError(); ctx->err = "event error"; return B200ZKP_ERR_CUDA; }
+        TRY(get_sync_event(ctx, 1 + c, &up[c]));
+        if (c1 > c0) CUDA_TRY(ctx, cudaMemcpyAsync(d_in.get() + (u64)c0 * n, in + (u64)c0 * n, (size_t)(c1 - c0) * n * 8, cudaMemcpyHostToDevice, ctx->stream2));
+        CUDA_TRY(ctx, cudaEventRecord(up[c], ctx->stream2));
+    }
+    for (u32 c = 0; c < n_chunks; c++) {
+        u32 c0 = std::min(k, c * per), c1 = std::min(k, (c + 1) * per);
+        CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream, up[c], 0));
         if (c1 == c0) continue;
         const u64* src = d_in.get() + (u64)c0 * n;
         u64* cf = b->coeffs.get() + (u64)c0 * n;
@@ -1071,10 +1060,9 @@ static int commit_host(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log
             // copy-back: this chunk's coefficients go home while the later chunks are still being transformed
             cudaEvent_t e_cf;
             TRY(get_sync_event(ctx, 2 + n_chunks + c, &e_cf));
-            e = cudaEventRecord(e_cf, ctx->stream);
-            if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream2, e_cf, 0);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(cb->coeffs + (u64)c0 * n, cf, (size_t)(c1 - c0) * n * 8, cudaMemcpyDeviceToHost, ctx->stream2);
-            if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
+            CUDA_TRY(ctx, cudaEventRecord(e_cf, ctx->stream));
+            CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, e_cf, 0));
+            CUDA_TRY(ctx, cudaMemcpyAsync(cb->coeffs + (u64)c0 * n, cf, (size_t)(c1 - c0) * n * 8, cudaMemcpyDeviceToHost, ctx->stream2));
         }
         TRY(dev_lde_locked(ctx, cf, n, ld, N, n_log, c1 - c0, rate_bits, 0, 1u << rate_bits));
     }
@@ -1084,26 +1072,25 @@ static int commit_host(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log
     if (cb && (cb->coeffs || cb->leaves)) {
         cudaEvent_t e_lde;
         TRY(get_sync_event(ctx, 1 + n_chunks, &e_lde));
-        e = cudaEventRecord(e_lde, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream2, e_lde, 0);
-        if (e == cudaSuccess && cb->leaves) {
+        CUDA_TRY(ctx, cudaEventRecord(e_lde, ctx->stream));
+        CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->stream2, e_lde, 0));
+        if (cb->leaves) {
             u64 chunk_rows = std::min<u64>(N, std::max<u64>(1, ((u64)256 << 20) / ((u64)row * 8)));
             TRY(stage.alloc(ctx, (size_t)chunk_rows * row * 8));
             StreamScope on_copy(ctx, ctx->stream2);     // transposes are issued on the copy stream (same order as their D2H)
-            for (u64 r0 = 0; r0 < N && e == cudaSuccess; r0 += chunk_rows) {
+            for (u64 r0 = 0; r0 < N; r0 += chunk_rows) {
                 u64 nr = std::min(chunk_rows, N - r0);
                 TRY(dev_transpose_rows_locked(ctx, b->lde.get(), N, row, r0, nr, stage.get()));
-                e = cudaMemcpyAsync(cb->leaves + r0 * row, stage.get(), (size_t)nr * row * 8, cudaMemcpyDeviceToHost, ctx->stream2);
+                CUDA_TRY(ctx, cudaMemcpyAsync(cb->leaves + r0 * row, stage.get(), (size_t)nr * row * 8, cudaMemcpyDeviceToHost, ctx->stream2));
             }
         }
-        if (e != cudaSuccess) { ctx->err = std::string("copy-back: ") + cudaGetErrorString(e); (void)cudaGetLastError(); return B200ZKP_ERR_CUDA; }
     }
     TRY(dev_merkle_locked(ctx, b->lde.get(), /*row_stride=*/1, /*col_stride=*/N, row, N, cap_height, b->digests.get(), b->cap.get()));
-    if (cb && cb->digests && b->digests.bytes()) e = cudaMemcpyAsync(cb->digests, b->digests.get(), b->digests.bytes(), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && cb && cb->cap) e = cudaMemcpyAsync(cb->cap, b->cap.get(), b->cap.bytes(), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream2);
-    if (e != cudaSuccess) { ctx->err = std::string("commit: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    if (cb && cb->digests && b->digests.bytes())
+        CUDA_TRY(ctx, cudaMemcpyAsync(cb->digests, b->digests.get(), b->digests.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    if (cb && cb->cap) CUDA_TRY(ctx, cudaMemcpyAsync(cb->cap, b->cap.get(), b->cap.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream2));
     if (out) *out = b.release();
     return 0;
 }
@@ -1181,30 +1168,40 @@ extern "C" int b200zkp_batch_leaves(b200zkp_batch* b, uint64_t* out) {
     return 0;
 }
 
-static int gather_locked(b200zkp_ctx* ctx, const u64* lde, u64 N, u32 row, const u64* digests, u32 sub_log,
+// MerkleTree::get + prove on the device, asynchronous: idx, rows [n_idx][row_len] and siblings [n_idx][depth][4] are
+// device buffers (rows or siblings may be null); element (row, c) of a leaf is lde[c * col_stride + row].  Each index is
+// reduced modulo n_leaves (a power of two), so no index reads out of range.
+static int dev_gather_locked(b200zkp_ctx* ctx, const u64* lde, u64 col_stride, u32 row_len, const u64* digests, u64 n_leaves,
+                             u32 depth, const u64* idx, u64 n_idx, u64* rows, u64* siblings) {
+    const u64 n_rows = rows ? n_idx * row_len : 0, n_sib = siblings ? n_idx * depth : 0;
+    if (n_rows) {
+        merkle::gather_rows_kernel<<<(unsigned)((n_rows + 255) / 256), 256, 0, ctx->stream>>>(lde, col_stride, row_len, idx, n_idx, rows,
+                                                                                            n_leaves - 1);
+        LAUNCH_CHECK(ctx);
+    }
+    if (n_sib) {
+        merkle::TreeShape shape; shape.sub_log = depth; shape.sub_digests = 2 * (((u64)1 << depth) - 1);
+        merkle::gather_siblings_kernel<<<(unsigned)((n_sib + 255) / 256), 256, 0, ctx->stream>>>(digests, shape, idx, n_idx, siblings,
+                                                                                               n_leaves - 1);
+        LAUNCH_CHECK(ctx);
+    }
+    return 0;
+}
+
+// the same for host indices and host outputs, synchronous; an index >= N is an error
+static int gather_locked(b200zkp_ctx* ctx, const u64* lde, u64 N, u32 row, const u64* digests, u32 depth,
                          const u64* idx, u64 n_idx, u64* rows, u64* siblings) {
     if (!n_idx) return 0;
     for (u64 i = 0; i < n_idx; i++) if (idx[i] >= N) BAD(ctx, "leaf index out of range");
     DevBuf d_idx, d_rows, d_sib;
     TRY(d_idx.alloc(ctx, n_idx * 8));
     TRY(d_rows.alloc(ctx, rows ? n_idx * row * 8 : 0));
-    TRY(d_sib.alloc(ctx, siblings ? n_idx * sub_log * 32 : 0));
+    TRY(d_sib.alloc(ctx, siblings ? n_idx * depth * 32 : 0));
     TRY(h2d(ctx, d_idx.get(), idx, d_idx.bytes()));
-    if (d_rows.bytes()) {
-        u64 cnt = n_idx * row;
-        merkle::gather_rows_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(lde, N, row, d_idx.get(), n_idx, d_rows.get(), N - 1);
-        ctx->launches++;
-        TRY(d2h(ctx, rows, d_rows.get(), d_rows.bytes()));
-    }
-    if (d_sib.bytes()) {
-        merkle::TreeShape shape; shape.sub_log = sub_log; shape.sub_digests = 2 * (((u64)1 << sub_log) - 1);
-        u64 cnt = n_idx * sub_log;
-        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(digests, shape, d_idx.get(), n_idx, d_sib.get(), N - 1);
-        ctx->launches++;
-        TRY(d2h(ctx, siblings, d_sib.get(), d_sib.bytes()));
-    }
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    TRY(dev_gather_locked(ctx, lde, N, row, digests, N, depth, d_idx.get(), n_idx, d_rows.get(), d_sib.get()));
+    if (d_rows.bytes()) CUDA_TRY(ctx, cudaMemcpyAsync(rows, d_rows.get(), d_rows.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_sib.bytes()) CUDA_TRY(ctx, cudaMemcpyAsync(siblings, d_sib.get(), d_sib.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 
@@ -1251,23 +1248,11 @@ extern "C" int b200zkp_dev_gather(b200zkp_ctx* ctx, const uint64_t* lde, uint64_
     u32 lg = 0;
     if (!log2_exact(n_leaves, &lg)) BAD(ctx, "number of leaves must be a power of two");
     if (cap_height > lg) BAD(ctx, "cap_height exceeds log2(number of leaves)");
-    if (rows_dev) {
-        if (!lde) BAD(ctx, "null leaf buffer");
-        u64 cnt = n_idx * row_len;
-        if (cnt) {
-            merkle::gather_rows_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>((const u64*)lde, col_stride, row_len, (const u64*)idx_dev, n_idx, (u64*)rows_dev, n_leaves - 1);
-            LAUNCH_CHECK(ctx);
-        }
-    }
-    u32 depth = lg - cap_height;
-    if (siblings_dev && depth) {
-        if (!digests) BAD(ctx, "null digests buffer");
-        merkle::TreeShape shape; shape.sub_log = depth; shape.sub_digests = 2 * (((u64)1 << depth) - 1);
-        u64 cnt = n_idx * depth;
-        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>((const u64*)digests, shape, (const u64*)idx_dev, n_idx, (u64*)siblings_dev, n_leaves - 1);
-        LAUNCH_CHECK(ctx);
-    }
-    return 0;
+    const u32 depth = lg - cap_height;
+    if (rows_dev && !lde) BAD(ctx, "null leaf buffer");
+    if (siblings_dev && depth && !digests) BAD(ctx, "null digests buffer");
+    return dev_gather_locked(ctx, (const u64*)lde, col_stride, row_len, (const u64*)digests, n_leaves, depth, (const u64*)idx_dev, n_idx,
+                             (u64*)rows_dev, (u64*)siblings_dev);
 }
 
 // ------------------------------------------------------------------------------------------------ openings (N3)
@@ -1286,11 +1271,9 @@ static int dev_eval_ext2_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 col_str
     TRY(d_part.alloc(ctx, (size_t)k * n_seg * sizeof(evalk::Ext2)));
     dim3 grid((unsigned)n_seg, k);
     evalk::eval_segments_kernel<<<grid, evalk::EVAL_THREADS, 0, ctx->stream>>>(coeffs, col_stride, n, seg_len, z, (evalk::Ext2*)d_part.get());
-    ctx->launches++;
+    LAUNCH_CHECK(ctx);
     evalk::eval_combine_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>((const evalk::Ext2*)d_part.get(), (u32)n_seg, seg_len, k, z, (evalk::Ext2*)d_out);
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ctx->err = std::string("eval: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
     return 0;
 }
 
@@ -1358,27 +1341,8 @@ static int fri_alloc_state(b200zkp_ctx* ctx, u32 n_log, u32 rate_bits, std::uniq
     f->coef_stride[0] = f->N; f->coef_stride[1] = std::max<u64>(f->N / 2, 1);
     for (int i = 0; i < 2; i++) TRY(f->coef[i].alloc(ctx, (size_t)2 * f->coef_stride[i] * 8));
     TRY(f->values.alloc(ctx, (size_t)2 * f->N * 8));
-    cudaError_t e = cudaMemsetAsync(f->coef[0].get(), 0, f->coef[0].bytes(), ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("fri: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    CUDA_TRY(ctx, cudaMemsetAsync(f->coef[0].get(), 0, f->coef[0].bytes(), ctx->stream));
     *out = std::move(f);
-    return 0;
-}
-
-// powers shift^i, i < 2^bits (scale table of a coset transform), cached per ctx
-static int get_power_scale(b200zkp_ctx* ctx, u64 shift, u32 bits, const u64** out) {
-    auto key = std::make_pair(shift, bits);
-    auto it = ctx->power_scale.find(key);
-    if (it == ctx->power_scale.end()) {
-        TwoLevel t;
-        TRY(make_two_level(ctx, shift, bits, &t));
-        u64 n = (u64)1 << bits;
-        u64* d = nullptr;
-        TRY(table_alloc(ctx, n, &d));
-        ntt::build_powers_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(d, n, t.lo, t.hi, t.lo_bits);
-        LAUNCH_CHECK(ctx);
-        it = ctx->power_scale.emplace(key, d).first;
-    }
-    *out = it->second;
     return 0;
 }
 
@@ -1442,22 +1406,20 @@ extern "C" int b200zkp_fri_begin(b200zkp_ctx* ctx, b200zkp_batch* const* oracles
         off += k;
         TRY(h2d(ctx, d_ptrs.get(), ptrs.data(), (size_t)k * 8));
         frik::ext_powers_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>(to_dev(alpha), k, pw);
-        ctx->launches++;
+        LAUNCH_CHECK(ctx);
         frik::reduce_polys_base_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(
             (const u64* const*)d_ptrs.get(), k, n, pw, comp_a, comp_im);
-        ctx->launches++;
+        LAUNCH_CHECK(ctx);
         HostExt z{gl_host_canon(points[2 * b]), gl_host_canon(points[2 * b + 1])};
         frik::scan_totals_kernel<<<n_seg, frik::SCAN_THREADS, 0, ctx->stream>>>(comp_a, comp_im, n, to_dev(z), tot);
-        ctx->launches++;
+        LAUNCH_CHECK(ctx);
         frik::scan_carries_kernel<<<1, frik::SCAN_THREADS, 0, ctx->stream>>>(tot, n_seg, to_dev(z), carry);
-        ctx->launches++;
+        LAUNCH_CHECK(ctx);
         // alpha.shift_poly(&mut final_poly): final_poly *= alpha^count, count = polynomials of this batch
         frik::divide_by_linear_kernel<<<n_seg, frik::SCAN_THREADS, 0, ctx->stream>>>(
             comp_a, comp_im, n, to_dev(z), carry, to_dev(host_ext_pow(alpha, k)),
             (flags & B200ZKP_FRI_MUL_BY_X) ? 1u : 0u, fin_a, fin_b);
-        ctx->launches++;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) { ctx->err = std::string("fri_begin: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+        LAUNCH_CHECK(ctx);
         // the pointer table is reused by the next batch: the copy above is stream-ordered after these kernels
     }
     TRY(fri_compute_values(f.get()));
@@ -1478,8 +1440,7 @@ extern "C" int b200zkp_fri_begin_from_coeffs(b200zkp_ctx* ctx, const uint64_t* c
     // stage the interleaved input in the (still unused) values buffer
     TRY(h2d(ctx, f->values.get(), coeffs, (size_t)n * 16));
     frik::deinterleave_kernel<<<(unsigned)((2 * n + 255) / 256), 256, 0, ctx->stream>>>(f->values.get(), n, f->coef[0].get(), f->coef[0].get() + f->coef_stride[0]);
-    ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: deinterleave launch failed"; return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
     TRY(fri_compute_values(f.get()));
     *out = f.release();
     return 0;
@@ -1505,8 +1466,7 @@ static int fri_copy_coeffs(b200zkp_fri* f, u64 len, u64* out) {
     TRY(d.alloc(ctx, (size_t)len * 16));
     const u64* pa = f->coef[f->cur].get();
     frik::interleave_kernel<<<(unsigned)((2 * len + 255) / 256), 256, 0, ctx->stream>>>(pa, pa + f->coef_stride[f->cur], len, d.get());
-    ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: interleave launch failed"; return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
     return d2h(ctx, out, d.get(), d.bytes());
 }
 
@@ -1538,8 +1498,7 @@ extern "C" int b200zkp_fri_commit_layer(b200zkp_fri* f, uint32_t arity_bits, uin
     TRY(L.digests.alloc(ctx, (size_t)2 * (L.n_leaves - ((u64)1 << cap_height)) * 32));
     TRY(L.cap.alloc(ctx, ((size_t)32) << cap_height));
     frik::interleave_kernel<<<(unsigned)((2 * M + 255) / 256), 256, 0, ctx->stream>>>(f->values.get(), f->values.get() + M, M, L.rows.get());
-    ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess) { ctx->err = "fri: interleave launch failed"; return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
     u32 leaf_len = 2u << arity_bits;
     TRY(dev_merkle_locked(ctx, L.rows.get(), leaf_len, 1, leaf_len, L.n_leaves, cap_height, L.digests.get(), L.cap.get()));
     TRY(d2h(ctx, cap_out, L.cap.get(), L.cap.bytes()));
@@ -1586,23 +1545,18 @@ extern "C" int b200zkp_fri_query(b200zkp_fri* f, uint32_t layer, const uint64_t*
     DevBuf d_idx, d_rows, d_sib;
     TRY(d_idx.alloc(ctx, n_idx * 8));
     TRY(d_rows.alloc(ctx, evals ? n_idx * row_len * 8 : 0));
-    TRY(d_sib.alloc(ctx, (siblings && depth) ? n_idx * depth * 32 : 0));
+    TRY(d_sib.alloc(ctx, siblings ? n_idx * depth * 32 : 0));
     TRY(h2d(ctx, d_idx.get(), idx, d_idx.bytes()));
     if (d_rows.bytes()) {
         u64 cnt = n_idx * row_len;
         frik::gather_rows_rm_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.rows.get(), row_len, d_idx.get(), n_idx, d_rows.get());
-        ctx->launches++;
-        TRY(d2h(ctx, evals, d_rows.get(), d_rows.bytes()));
+        LAUNCH_CHECK(ctx);
     }
-    if (d_sib.bytes()) {
-        merkle::TreeShape shape; shape.sub_log = depth; shape.sub_digests = 2 * (((u64)1 << depth) - 1);
-        u64 cnt = n_idx * depth;
-        merkle::gather_siblings_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, ctx->stream>>>(L.digests.get(), shape, d_idx.get(), n_idx, d_sib.get(), ~0ull);
-        ctx->launches++;
-        TRY(d2h(ctx, siblings, d_sib.get(), d_sib.bytes()));
-    }
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    // the layer's leaves are row-major: only the siblings come from the shared gather
+    TRY(dev_gather_locked(ctx, nullptr, 0, 0, L.digests.get(), L.n_leaves, depth, d_idx.get(), n_idx, nullptr, d_sib.get()));
+    if (d_rows.bytes()) CUDA_TRY(ctx, cudaMemcpyAsync(evals, d_rows.get(), d_rows.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_sib.bytes()) CUDA_TRY(ctx, cudaMemcpyAsync(siblings, d_sib.get(), d_sib.bytes(), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 
@@ -1624,8 +1578,7 @@ extern "C" int b200zkp_pow_grind(b200zkp_ctx* ctx, const uint64_t state[12], uin
         u64 count = std::min(window, max_candidates - start);
         frik::pow_grind_kernel<<<(unsigned)((count + 255) / 256), 256, 0, ctx->stream>>>(
             d.get(), witness_pos, response_pos, min_leading_zeros, start, count, (unsigned long long*)d.get() + 12);
-        ctx->launches++;
-        if (cudaGetLastError() != cudaSuccess) { ctx->err = "pow_grind launch failed"; return B200ZKP_ERR_CUDA; }
+        LAUNCH_CHECK(ctx);
         TRY(d2h(ctx, &best, d.get() + 12, 8));
         if (best != ~(u64)0) break;
         start += count;
@@ -1656,8 +1609,7 @@ extern "C" int b200zkp_merkle_new(b200zkp_ctx* ctx, const uint64_t* leaves, uint
     TRY(d_leaves.alloc(ctx, std::max<size_t>((size_t)n_leaves * leaf_len * 8, 8)));
     TRY(h2d(ctx, d_leaves.get(), leaves, (size_t)n_leaves * leaf_len * 8));
     TRY(dev_merkle_locked(ctx, d_leaves.get(), leaf_len, 1, leaf_len, n_leaves, cap_height, t->digests.get(), t->cap.get()));
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("merkle_new: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     *out = t.release();
     return 0;
 }
@@ -1683,13 +1635,9 @@ extern "C" int b200zkp_tree_prove(b200zkp_tree* t, const uint64_t* idx, uint64_t
     Guard g(t->ctx);
     u32 lg = 0;
     log2_exact(t->n_leaves, &lg);
-    if (lg == t->cap_height) {
-        for (u64 i = 0; i < n_idx; i++) if (idx[i] >= t->n_leaves) BAD(t->ctx, "leaf index out of range");
-        return 0;  // empty proofs
-    }
-    if (!siblings && n_idx) BAD(t->ctx, "null out");
-    return gather_locked(t->ctx, nullptr, t->n_leaves, 0, t->digests.get(), lg - t->cap_height, (const u64*)idx, n_idx,
-                         nullptr, (u64*)siblings);
+    const u32 depth = lg - t->cap_height;     // 0: empty proofs, only the indices are checked
+    if (!siblings && n_idx && depth) BAD(t->ctx, "null out");
+    return gather_locked(t->ctx, nullptr, t->n_leaves, 0, t->digests.get(), depth, (const u64*)idx, n_idx, nullptr, (u64*)siblings);
 }
 
 // ------------------------------------------------------------------------------------------------ permutation argument (N1a)
@@ -1713,25 +1661,20 @@ static int dev_partial_products_locked(b200zkp_ctx* ctx, const u64* wires, u64 w
     TRY(d_run.alloc(ctx, (size_t)C * chunks * n * 8));
     TRY(d_tot.alloc(ctx, (size_t)C * n_blocks * 8));
     TRY(h2d(ctx, d_small.get(), small.data(), d_small.bytes()));
-    {   // `small` is a pageable host vector
-        cudaError_t e0 = cudaStreamSynchronize(ctx->stream);
-        if (e0 != cudaSuccess) { ctx->err = cudaGetErrorString(e0); return B200ZKP_ERR_CUDA; }
-    }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));    // `small` is a pageable host vector
     perm::Params p;
     p.wires = wires; p.wires_stride = wires_stride; p.sigmas = sigmas; p.sigmas_stride = sigmas_stride;
     p.k_is = d_small.get(); p.betas = d_small.get() + R; p.gammas = d_small.get() + R + C;
     p.omega = hostgl::root(n_log); p.n = n; p.R = R; p.degree = degree; p.chunks = chunks; p.C = C;
     perm::chunk_products_kernel<<<dim3((unsigned)((n + 127) / 128), C), 128, 0, ctx->stream>>>(p, d_run.get());
-    ctx->launches++;
+    LAUNCH_CHECK(ctx);
     perm::block_totals_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>(d_run.get(), n, chunks, per, d_tot.get());
-    ctx->launches++;
+    LAUNCH_CHECK(ctx);
     perm::scan_totals_kernel<<<C, perm::SCAN_THREADS, 0, ctx->stream>>>(d_tot.get(), n_blocks);
-    ctx->launches++;
+    LAUNCH_CHECK(ctx);
     perm::finish_kernel<<<dim3(n_blocks, C), perm::SCAN_THREADS, 0, ctx->stream>>>(d_run.get(), d_tot.get(), n, chunks, per, C, out, out_stride);
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { ctx->err = cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return 0;
 }
 
@@ -1963,25 +1906,16 @@ extern "C" int b200zkp_coset_lde(b200zkp_ctx* ctx, const uint64_t* coeffs, uint3
     u32 N_log = n_log + rate_bits;
     if (N_log > 32 || rate_bits > 8) BAD(ctx, "n_log + rate_bits exceeds two-adicity");
     u64 n = (u64)1 << n_log, N = (u64)1 << N_log;
-    auto it = ctx->shift7_scale.find(N_log);
-    if (it == ctx->shift7_scale.end()) {
-        TwoLevel t;
-        TRY(make_two_level(ctx, 7, N_log, &t));
-        u64* d = nullptr;
-        TRY(table_alloc(ctx, N, &d));
-        ntt::build_powers_kernel<<<(unsigned)((N + 255) / 256), 256, 0, ctx->stream>>>(d, N, t.lo, t.hi, t.lo_bits);
-        LAUNCH_CHECK(ctx);
-        it = ctx->shift7_scale.emplace(N_log, d).first;
-    }
+    const u64* scale = nullptr;
+    TRY(get_power_scale(ctx, 7, N_log, &scale));
     size_t big = (size_t)k * N * 8;
     DevBuf d_pad, d_scr, d_out;
     TRY(d_pad.alloc(ctx, big));
     TRY(d_scr.alloc(ctx, big));
     TRY(d_out.alloc(ctx, big));
-    cudaError_t e = cudaMemsetAsync(d_pad.get(), 0, big, ctx->stream);
-    if (e == cudaSuccess) e = cudaMemcpy2DAsync(d_pad.get(), N * 8, coeffs, n * 8, n * 8, k, cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) { ctx->err = std::string("coset_lde H2D: ") + cudaGetErrorString(e); return B200ZKP_ERR_CUDA; }
-    TRY(run_transform(ctx, d_pad.get(), N, d_out.get(), N, d_scr.get(), N_log, k, 0, false, it->second, 0, false, true));
+    CUDA_TRY(ctx, cudaMemsetAsync(d_pad.get(), 0, big, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpy2DAsync(d_pad.get(), N * 8, coeffs, n * 8, n * 8, k, cudaMemcpyHostToDevice, ctx->stream));
+    TRY(run_transform(ctx, d_pad.get(), N, d_out.get(), N, d_scr.get(), N_log, k, 0, false, scale, 0, false, true));
     return d2h(ctx, out, d_out.get(), big);
 }
 
@@ -2233,8 +2167,7 @@ extern "C" int b200zkp_dev_quotient_values(b200zkp_ctx* ctx, const b200zkp_vanis
     p.n_inv = hostgl::inv(n % hostgl::P);
     p.out = (u64*)out_dev; p.out_stride = out_stride;
     vanish::quotient_values_kernel<<<(unsigned)((Q + 127) / 128), 128, 0, ctx->stream>>>(p);
-    ctx->launches++;
-    if (cudaGetLastError() != cudaSuccess) { ctx->err = "quotient_values_kernel launch failed"; return B200ZKP_ERR_CUDA; }
+    LAUNCH_CHECK(ctx);
     return 0;
 }
 

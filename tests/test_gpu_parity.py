@@ -281,6 +281,30 @@ def test_rows_proofs_and_lde_values(z, ctx, oracle):
     assert (b.merkle_tree.prove(5).siblings == oracle.merkle_prove(ref["digests"], N, h, 5)).all()
 
 
+def test_dev_gather_matches_batch_rows(z, ctx, oracle):
+    """b200zkp_dev_gather on a batch's own device buffers: device indices in, device rows and proofs out, the same
+    words as PolynomialBatch.rows; an index past the last leaf is reduced modulo the number of leaves."""
+    import ctypes as C
+    import torch
+    n_log, k, r, h = 7, 11, 3, 4
+    N, depth = 1 << (n_log + r), n_log + r - h
+    b = z.PolynomialBatch.from_values(oracle.synthetic_values(k, 1 << n_log, seed=9), r, False, h, ctx=ctx)
+    idx = np.array([0, 1, N // 2, N - 1, 37, 38, 1000], np.uint64)
+    rows, sib = b.rows(idx)
+    _, lde, digests, _ = b.device_ptrs()
+    d_idx = torch.from_numpy(np.array([*idx, N + 37], np.uint64).view(np.int64)).cuda()
+    d_rows = torch.zeros((idx.size + 1, k), dtype=torch.int64, device="cuda")
+    d_sib = torch.zeros((idx.size + 1, depth, 4), dtype=torch.int64, device="cuda")
+    torch.cuda.synchronize()
+    p = lambda t: C.c_void_p(t.data_ptr())
+    ctx.check(ctx._lib.b200zkp_dev_gather(ctx._h, C.c_void_p(lde), N, k, C.c_void_p(digests), N, h, p(d_idx), idx.size + 1,
+                                          p(d_rows), p(d_sib)))
+    ctx.synchronize()
+    got_rows, got_sib = d_rows.cpu().numpy().view(np.uint64), d_sib.cpu().numpy().view(np.uint64)
+    assert (got_rows[:-1] == rows).all() and (got_sib[:-1] == sib).all()
+    assert (got_rows[-1] == rows[4]).all() and (got_sib[-1] == sib[4]).all()
+
+
 @pytest.mark.parametrize("N,L,h", [(1, 5, 0), (2, 3, 1), (16, 4, 2), (16, 5, 0), (64, 32, 4), (256, 135, 4),
                                    (1024, 9, 10), (4096, 2, 3), (8, 0, 1)])
 def test_merkle_tree_new(z, ctx, oracle, N, L, h):
