@@ -144,6 +144,21 @@ class PolynomialBatch {
                                        bool blinding, size_t cap_height, const std::vector<std::vector<F>>& salt = {}) {
         return commit(c, polynomials, true, rate_bits, blinding, cap_height, salt);
     }
+    // from_values / from_coeffs of a k x n column-major matrix already in device memory (b200zkp_batch_from_device); the
+    // commit is enqueued on the ctx stream, `in_dev` must stay valid until it has run (the cap read below waits for it)
+    static PolynomialBatch from_device(const Context& c, const uint64_t* in_dev, bool is_coeffs, size_t n_log, size_t k,
+                                       size_t rate_bits, size_t cap_height) {
+        PolynomialBatch b;
+        b.ctx_ = &c;
+        b.degree_log = n_log; b.rate_bits = rate_bits; b.cap_height = cap_height; b.num_polys = k;
+        b200zkp_batch* h = nullptr;
+        c.check(b200zkp_batch_from_device(c.raw(), in_dev, is_coeffs ? 1 : 0, (uint32_t)n_log, (uint32_t)k, (uint32_t)rate_bits,
+                                          (uint32_t)cap_height, nullptr, &h));
+        b.h_.reset(h, b200zkp_batch_free);
+        b.cap.resize(size_t(1) << cap_height);
+        c.check(b200zkp_batch_cap(h, b.cap[0].elements.data()));
+        return b;
+    }
     // &leaves[reverse_bits(index * step, degree_log + rate_bits)][..len - salt]
     std::vector<F> get_lde_values(uint64_t index, uint64_t step = 1) const {
         std::vector<F> out(num_polys);
@@ -265,5 +280,29 @@ class ShardedPolynomialBatch {
     std::shared_ptr<b200zkp_comm> comm_;      // (declared before h_: the buffers are released first)
     std::shared_ptr<b200zkp_sharded> h_;
 };
+
+// OpeningSet::new in its FRI form (b200zkp_batch_openings): for each point, the values of its (oracle, index) polynomials
+inline std::vector<std::vector<std::array<F, 2>>> batch_openings(
+        const Context& c, const std::vector<const PolynomialBatch*>& oracles, const std::vector<std::array<F, 2>>& points,
+        const std::vector<std::vector<std::pair<uint32_t, uint32_t>>>& polys) {
+    if (points.size() != polys.size()) throw std::invalid_argument("one polynomial list per point");
+    std::vector<b200zkp_batch*> handles;
+    for (auto* o : oracles) handles.push_back(o->raw());
+    std::vector<uint32_t> counts, po, pi;
+    for (auto& ps : polys) {
+        counts.push_back((uint32_t)ps.size());
+        for (auto& p : ps) { po.push_back(p.first); pi.push_back(p.second); }
+    }
+    std::vector<std::array<F, 2>> flat(std::max<size_t>(po.size(), 1));
+    c.check(b200zkp_batch_openings(c.raw(), handles.data(), (uint32_t)handles.size(), (uint32_t)points.size(), points[0].data(),
+                                   counts.data(), po.data(), pi.data(), flat[0].data()));
+    std::vector<std::vector<std::array<F, 2>>> out;
+    size_t off = 0;
+    for (auto& ps : polys) {
+        out.emplace_back(flat.begin() + off, flat.begin() + off + ps.size());
+        off += ps.size();
+    }
+    return out;
+}
 
 }  // namespace plonky2

@@ -100,6 +100,13 @@ int b200zkp_commit_from_coeffs(b200zkp_ctx* ctx, const uint64_t* coeffs, uint32_
 int b200zkp_commit_copy_back(b200zkp_ctx* ctx, const uint64_t* in, int is_coeffs, uint32_t n_log, uint32_t k,
                              uint32_t rate_bits, uint32_t cap_height, const uint64_t* salt, uint64_t* coeffs_out,
                              uint64_t* leaves_out, uint64_t* digests_out, uint64_t* cap_out, b200zkp_batch** out);
+/* the same commitment of a k x n matrix already in HBM (in_dev, column-major as for b200zkp_dev_commit; salt_dev NULL or
+ * 4*N device words as for b200zkp_commit_from_values): an owned handle like the one b200zkp_commit_from_values returns,
+ * which every b200zkp_batch_* call and b200zkp_fri_begin accept.  Asynchronous on the ctx stream; the inputs are only read
+ * and must stay valid until the stream has run the commit.  Argument errors as for b200zkp_dev_commit; on any error *out
+ * stays NULL. */
+int b200zkp_batch_from_device(b200zkp_ctx* ctx, const uint64_t* in_dev, int is_coeffs, uint32_t n_log, uint32_t k,
+                              uint32_t rate_bits, uint32_t cap_height, const uint64_t* salt_dev, b200zkp_batch** out);
 void b200zkp_batch_free(b200zkp_batch* b);
 /* shape: n_log, k, rate_bits, cap_height, salt_size */
 int b200zkp_batch_shape(const b200zkp_batch* b, uint32_t shape[5]);
@@ -125,6 +132,15 @@ int b200zkp_batch_eval_ext2(b200zkp_batch* b, const uint64_t zeta[2], uint64_t* 
 /* same on caller-owned device buffers (coeffs [k][col_stride], out_dev k*2 on the device; async on the ctx stream) */
 int b200zkp_dev_eval_ext2(b200zkp_ctx* ctx, const uint64_t* coeffs, uint64_t col_stride, uint32_t n_log, uint32_t k,
                           const uint64_t zeta[2], uint64_t* out_dev);
+
+/* OpeningSet::new in its FRI form (to_fri_openings): every polynomial of an opening instance evaluated at its point, the
+ * instance described as for b200zkp_fri_begin (oracles, points, polynomials per point as (oracle, index) pairs).
+ * out: 2 words per listed polynomial, batch after batch — the order the challenger observes them.  One launch pair for the
+ * whole instance, one copy back.  Errors (before anything is launched): bad arg for null or empty arguments, an oracle of
+ * another ctx, oracles of differing n_log or rate_bits, an oracle or polynomial index out of range. */
+int b200zkp_batch_openings(b200zkp_ctx* ctx, b200zkp_batch* const* oracles, uint32_t n_oracles, uint32_t n_points,
+                           const uint64_t* points, const uint32_t* point_n_polys, const uint32_t* poly_oracle,
+                           const uint32_t* poly_index, uint64_t* out);
 
 /* ---- opening proof (rows N2 + N3): PolynomialBatch::prove_openings / fri_proof ---------------- */
 /* Replaces the data-parallel steps of plonky2 @ f99ed9c  fri/oracle.rs `prove_openings`, fri/prover.rs

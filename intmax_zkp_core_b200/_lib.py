@@ -93,6 +93,8 @@ _SIGS = {
     "b200zkp_commit_from_values": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.POINTER(C.c_void_p)]),
     "b200zkp_commit_from_coeffs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.POINTER(C.c_void_p)]),
     "b200zkp_commit_copy_back": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "b200zkp_batch_from_device": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p,
+                                            C.POINTER(C.c_void_p)]),
     "b200zkp_batch_free": (None, [C.c_void_p]),
     "b200zkp_batch_shape": (C.c_int, [C.c_void_p, u32p]),
     "b200zkp_batch_cap": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -106,6 +108,8 @@ _SIGS = {
     "b200zkp_dev_eval_ext2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
     "b200zkp_dev_gather": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p,
                                      C.c_uint64, C.c_void_p, C.c_void_p]),
+    "b200zkp_batch_openings": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p]),
     "b200zkp_fri_begin": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)]),
     "b200zkp_fri_begin_from_coeffs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)]),

@@ -953,11 +953,17 @@ extern "C" int b200zkp_dev_lde_merkle(b200zkp_ctx* ctx, const uint64_t* coeffs, 
                                  block_end, k, cap_height, (u64*)digests, (u64*)cap);
 }
 
-static int dev_commit_locked(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log, u32 k, u32 rate_bits,
-                             u32 cap_height, const u64* salt, u64* coeffs, u64* lde, u64* digests, u64* cap) {
+// plonky2's asserts on the shape of a PolynomialBatch
+static int check_commit_shape(b200zkp_ctx* ctx, u32 n_log, u32 k, u32 rate_bits, u32 cap_height) {
     if (k == 0) BAD(ctx, "empty polynomial batch");
     if (n_log + rate_bits > 32 || rate_bits > 8) BAD(ctx, "n_log + rate_bits exceeds two-adicity");
     if (cap_height > n_log + rate_bits) BAD(ctx, "cap_height exceeds log2(LDE size)");
+    return 0;
+}
+
+static int dev_commit_locked(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log, u32 k, u32 rate_bits,
+                             u32 cap_height, const u64* salt, u64* coeffs, u64* lde, u64* digests, u64* cap) {
+    TRY(check_commit_shape(ctx, n_log, k, rate_bits, cap_height));
     if (!in || !coeffs || !lde || !cap) BAD(ctx, "null buffer");
     u64 n = (u64)1 << n_log, N = n << rate_bits;
     u32 row = k + (salt ? B200ZKP_SALT_SIZE : 0);
@@ -1006,9 +1012,7 @@ static int commit_host(b200zkp_ctx* ctx, const u64* in, int is_coeffs, u32 n_log
                        u32 cap_height, const u64* salt, b200zkp_batch** out, const CopyBack* cb = nullptr) {
     if (!out && !cb) BAD(ctx, "null out");
     if (out) *out = nullptr;
-    if (k == 0) BAD(ctx, "empty polynomial batch");
-    if (n_log + rate_bits > 32 || rate_bits > 8) BAD(ctx, "n_log + rate_bits exceeds two-adicity");
-    if (cap_height > n_log + rate_bits) BAD(ctx, "cap_height exceeds log2(LDE size)");
+    TRY(check_commit_shape(ctx, n_log, k, rate_bits, cap_height));
     if (!in) BAD(ctx, "null input");
     u64 n = (u64)1 << n_log, N = n << rate_bits;
     u32 row = k + (salt ? B200ZKP_SALT_SIZE : 0);
@@ -1118,6 +1122,37 @@ extern "C" int b200zkp_commit_from_coeffs(b200zkp_ctx* ctx, const uint64_t* coef
     if (!ctx) return B200ZKP_ERR_BAD_ARG;
     Guard g(ctx);
     return commit_host(ctx, (const u64*)coeffs, 1, n_log, k, rate_bits, cap_height, (const u64*)salt, out);
+}
+
+// PolynomialBatch::from_values / from_coeffs on a matrix already in HBM: dev_commit_locked writing into the handle's buffers
+extern "C" int b200zkp_batch_from_device(b200zkp_ctx* ctx, const uint64_t* in_dev, int is_coeffs, uint32_t n_log, uint32_t k,
+                                         uint32_t rate_bits, uint32_t cap_height, const uint64_t* salt_dev, b200zkp_batch** out) {
+    if (!ctx) return B200ZKP_ERR_BAD_ARG;
+    Guard g(ctx);
+    if (!out) BAD(ctx, "null out");
+    *out = nullptr;
+    TRY(check_commit_shape(ctx, n_log, k, rate_bits, cap_height));
+    if (!in_dev) BAD(ctx, "null buffer");
+    u64 N = (u64)1 << (n_log + rate_bits);
+    std::unique_ptr<b200zkp_batch> b(new (std::nothrow) b200zkp_batch());
+    if (!b) return B200ZKP_ERR_OOM;
+    b->ctx = ctx; b->n_log = n_log; b->k = k; b->rate_bits = rate_bits; b->cap_height = cap_height;
+    b->salt = salt_dev ? B200ZKP_SALT_SIZE : 0;
+    TRY(b->coeffs.alloc(ctx, ((size_t)k * 8) << n_log));
+    TRY(b->lde.alloc(ctx, (size_t)(k + b->salt) * N * 8));
+    TRY(b->digests.alloc(ctx, (size_t)2 * (N - ((u64)1 << cap_height)) * 32));
+    TRY(b->cap.alloc(ctx, ((size_t)32) << cap_height));
+    int rc = dev_commit_locked(ctx, (const u64*)in_dev, is_coeffs, n_log, k, rate_bits, cap_height, (const u64*)salt_dev,
+                               b->coeffs.get(), b->lde.get(), b->digests.get(), b->cap.get());
+    if (rc) {
+        // the buffers go back to the pool: nothing may still be writing them
+        cudaStreamSynchronize(ctx->stream);
+        if (ctx->stream2) cudaStreamSynchronize(ctx->stream2);
+        (void)cudaGetLastError();
+        return rc;
+    }
+    *out = b.release();
+    return 0;
 }
 
 extern "C" void b200zkp_batch_free(b200zkp_batch* b) {
@@ -1256,25 +1291,33 @@ extern "C" int b200zkp_dev_gather(b200zkp_ctx* ctx, const uint64_t* lde, uint64_
 }
 
 // ------------------------------------------------------------------------------------------------ openings (N3)
-static int dev_eval_ext2_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 col_stride, u32 n_log, u32 k, const u64 zeta[2],
-                                u64* d_out /* k*2 */) {
-    if (!k) return 0;
-    if (n_log > 32) BAD(ctx, "n_log out of range");
+// the two launches of every opening evaluation: m entries of L, each a column of n = 2^n_log coefficients -> d_out[m]
+static int eval_list_locked(b200zkp_ctx* ctx, const evalk::EvalList& L, u32 m, u32 n_log, evalk::Ext2* d_out) {
+    if (!m) return 0;
     u64 n = (u64)1 << n_log;
-    evalk::Ext2 z; z.a = gl_host_canon(zeta[0]); z.b = gl_host_canon(zeta[1]);
     // segments: enough CTAs to fill the GPU (~4 per SM), at least 1024 coefficients each
-    u64 want = (4 * 148 + k - 1) / k;
+    u64 want = (4 * 148 + m - 1) / m;
     u64 n_seg = 1;
     while (n_seg < want && (n / (n_seg * 2)) >= 1024) n_seg *= 2;
     u64 seg_len = n / n_seg;
     DevBuf d_part;
-    TRY(d_part.alloc(ctx, (size_t)k * n_seg * sizeof(evalk::Ext2)));
-    dim3 grid((unsigned)n_seg, k);
-    evalk::eval_segments_kernel<<<grid, evalk::EVAL_THREADS, 0, ctx->stream>>>(coeffs, col_stride, n, seg_len, z, (evalk::Ext2*)d_part.get());
+    TRY(d_part.alloc(ctx, (size_t)m * n_seg * sizeof(evalk::Ext2)));
+    dim3 grid((unsigned)n_seg, m);
+    evalk::eval_segments_kernel<<<grid, evalk::EVAL_THREADS, 0, ctx->stream>>>(L, n, seg_len, (evalk::Ext2*)d_part.get());
     LAUNCH_CHECK(ctx);
-    evalk::eval_combine_kernel<<<(k + 127) / 128, 128, 0, ctx->stream>>>((const evalk::Ext2*)d_part.get(), (u32)n_seg, seg_len, k, z, (evalk::Ext2*)d_out);
+    evalk::eval_combine_kernel<<<(m + 127) / 128, 128, 0, ctx->stream>>>(L, (const evalk::Ext2*)d_part.get(), (u32)n_seg, seg_len, m, d_out);
     LAUNCH_CHECK(ctx);
     return 0;
+}
+
+static int dev_eval_ext2_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 col_stride, u32 n_log, u32 k, const u64 zeta[2],
+                                u64* d_out /* k*2 */) {
+    if (!k) return 0;
+    if (n_log > 32) BAD(ctx, "n_log out of range");
+    evalk::EvalList L{};
+    L.base = coeffs; L.col_stride = col_stride;
+    L.z0.a = gl_host_canon(zeta[0]); L.z0.b = gl_host_canon(zeta[1]);
+    return eval_list_locked(ctx, L, k, n_log, (evalk::Ext2*)d_out);
 }
 
 extern "C" int b200zkp_dev_eval_ext2(b200zkp_ctx* ctx, const uint64_t* coeffs, uint64_t col_stride, uint32_t n_log, uint32_t k,
@@ -1292,6 +1335,63 @@ extern "C" int b200zkp_batch_eval_ext2(b200zkp_batch* b, const uint64_t zeta[2],
     DevBuf d_out;
     TRY(d_out.alloc(ctx, (size_t)b->k * 16));
     TRY(dev_eval_ext2_locked(ctx, b->coeffs.get(), (u64)1 << b->n_log, b->n_log, b->k, (const u64*)zeta, d_out.get()));
+    return d2h(ctx, out, d_out.get(), d_out.bytes());
+}
+
+// an opening instance as b200zkp_fri_begin and b200zkp_batch_openings take it: every check before anything is launched
+static int check_instance(b200zkp_ctx* ctx, b200zkp_batch* const* oracles, uint32_t n_oracles, uint32_t n_points, const uint64_t* points,
+                          const uint32_t* point_n_polys, const uint32_t* poly_oracle, const uint32_t* poly_index, u32* total_out,
+                          u32* max_k_out) {
+    if (!oracles || !n_oracles || !n_points || !points || !point_n_polys || !poly_oracle || !poly_index)
+        BAD(ctx, "null or empty argument");
+    u32 n_log = oracles[0] ? oracles[0]->n_log : 0, rate_bits = oracles[0] ? oracles[0]->rate_bits : 0;
+    for (u32 i = 0; i < n_oracles; i++) {
+        if (!oracles[i] || oracles[i]->ctx != ctx) BAD(ctx, "oracle belongs to another context");
+        if (oracles[i]->n_log != n_log || oracles[i]->rate_bits != rate_bits) BAD(ctx, "oracles differ in degree or rate");
+    }
+    u64 total = 0;
+    u32 max_k = 0;
+    for (u32 b = 0; b < n_points; b++) { total += point_n_polys[b]; max_k = std::max(max_k, point_n_polys[b]); }
+    if (total > UINT32_MAX) BAD(ctx, "too many polynomials");
+    for (u64 i = 0; i < total; i++) {
+        if (poly_oracle[i] >= n_oracles) BAD(ctx, "oracle index out of range");
+        if (poly_index[i] >= oracles[poly_oracle[i]]->k) BAD(ctx, "polynomial index out of range");
+    }
+    if (!max_k) BAD(ctx, "no polynomial to open");
+    *total_out = (u32)total;
+    *max_k_out = max_k;
+    return 0;
+}
+
+extern "C" int b200zkp_batch_openings(b200zkp_ctx* ctx, b200zkp_batch* const* oracles, uint32_t n_oracles, uint32_t n_points,
+                                      const uint64_t* points, const uint32_t* point_n_polys, const uint32_t* poly_oracle,
+                                      const uint32_t* poly_index, uint64_t* out) {
+    if (!ctx) return B200ZKP_ERR_BAD_ARG;
+    Guard g(ctx);
+    if (!out) BAD(ctx, "null out");
+    u32 m = 0, max_k = 0;
+    TRY(check_instance(ctx, oracles, n_oracles, n_points, points, point_n_polys, poly_oracle, poly_index, &m, &max_k));
+    const u32 n_log = oracles[0]->n_log;
+    const u64 n = (u64)1 << n_log;
+    // one table: the m entries, then the points
+    std::vector<evalk::EvalEntry> tab(m + n_points);
+    u32 e = 0;
+    for (u32 b = 0; b < n_points; b++)
+        for (u32 j = 0; j < point_n_polys[b]; j++, e++) {
+            tab[e].col = oracles[poly_oracle[e]]->coeffs.get() + (u64)poly_index[e] * n;
+            tab[e].point = b;
+        }
+    evalk::Ext2* pts = (evalk::Ext2*)(tab.data() + m);
+    for (u32 b = 0; b < n_points; b++) { pts[b].a = gl_host_canon(points[2 * b]); pts[b].b = gl_host_canon(points[2 * b + 1]); }
+    static_assert(sizeof(evalk::EvalEntry) == sizeof(evalk::Ext2), "points share the entry table");
+    DevBuf d_tab, d_out;
+    TRY(d_tab.alloc(ctx, tab.size() * sizeof(evalk::EvalEntry)));
+    TRY(d_out.alloc(ctx, (size_t)m * sizeof(evalk::Ext2)));
+    TRY(h2d(ctx, d_tab.get(), tab.data(), d_tab.bytes()));
+    evalk::EvalList L{};
+    L.entries = (const evalk::EvalEntry*)d_tab.get();
+    L.points = (const evalk::Ext2*)(L.entries + m);
+    TRY(eval_list_locked(ctx, L, m, n_log, (evalk::Ext2*)d_out.get()));
     return d2h(ctx, out, d_out.get(), d_out.bytes());
 }
 
@@ -1365,21 +1465,11 @@ extern "C" int b200zkp_fri_begin(b200zkp_ctx* ctx, b200zkp_batch* const* oracles
     Guard g(ctx);
     if (!out) BAD(ctx, "null out");
     *out = nullptr;
-    if (!oracles || !n_oracles || !n_points || !points || !point_n_polys || !poly_oracle || !poly_index || !alpha_in)
-        BAD(ctx, "null or empty argument");
-    u32 n_log = oracles[0] ? oracles[0]->n_log : 0, rate_bits = oracles[0] ? oracles[0]->rate_bits : 0;
-    for (u32 i = 0; i < n_oracles; i++) {
-        if (!oracles[i] || oracles[i]->ctx != ctx) BAD(ctx, "oracle belongs to another context");
-        if (oracles[i]->n_log != n_log || oracles[i]->rate_bits != rate_bits) BAD(ctx, "oracles differ in degree or rate");
-    }
-    u64 n = (u64)1 << n_log;
+    if (!alpha_in) BAD(ctx, "null or empty argument");
     u32 total = 0, max_k = 0;
-    for (u32 b = 0; b < n_points; b++) { total += point_n_polys[b]; max_k = std::max(max_k, point_n_polys[b]); }
-    for (u32 i = 0; i < total; i++) {
-        if (poly_oracle[i] >= n_oracles) BAD(ctx, "oracle index out of range");
-        if (poly_index[i] >= oracles[poly_oracle[i]]->k) BAD(ctx, "polynomial index out of range");
-    }
-    if (!max_k) BAD(ctx, "no polynomial to open");
+    TRY(check_instance(ctx, oracles, n_oracles, n_points, points, point_n_polys, poly_oracle, poly_index, &total, &max_k));
+    const u32 n_log = oracles[0]->n_log, rate_bits = oracles[0]->rate_bits;
+    u64 n = (u64)1 << n_log;
     std::unique_ptr<b200zkp_fri> f;
     TRY(fri_alloc_state(ctx, n_log, rate_bits, &f));
     HostExt alpha{gl_host_canon(alpha_in[0]), gl_host_canon(alpha_in[1])};

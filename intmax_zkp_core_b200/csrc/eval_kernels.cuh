@@ -10,6 +10,10 @@
 // p(z) = sum_t z^t * Q_t(z^256),  Q_t(y) = sum_j c[256 j + t] y^j : thread t of a CTA runs Horner in y over its strided
 // (coalesced) coefficients; columns are cut into segments so the grid fills the GPU; a second tiny kernel adds the
 // segment partials  sum_s z^(s * seg_len) * P_s.
+//
+// One launch pair evaluates a list of entries e = (column, point): the whole of OpeningSet::new (every polynomial of four
+// batches at zeta, the Zs at g zeta) is one list.  Without a table (entries == nullptr) entry e is the column
+// base + e * col_stride at the point z0, which is what the one-batch, one-point callers pass by value.
 #pragma once
 #include "goldilocks.cuh"
 
@@ -37,16 +41,33 @@ GL_FN Ext2 ext_pow(Ext2 x, u64 e) {
 
 static constexpr int EVAL_THREADS = 256;
 
+struct EvalEntry { const u64* col; u64 point; };   // a column of n coefficients and the index of its point
+
 #ifndef B200ZKP_HOST_EMU
-// grid (segments, columns); partial[col][seg] = sum_{i in segment} c[i] z^(i - seg_start)
+struct EvalList {
+    const EvalEntry* entries;   // nullptr: column base + e * col_stride at z0
+    const Ext2* points;
+    const u64* base;
+    u64 col_stride;
+    Ext2 z0;
+};
+
+GL_FN void eval_entry(const EvalList& L, u64 e, const u64** col, Ext2* z) {
+    if (L.entries) { const EvalEntry en = L.entries[e]; *col = en.col; *z = L.points[en.point]; }
+    else { *col = L.base + e * L.col_stride; *z = L.z0; }
+}
+
+// grid (segments, entries); partial[e][seg] = sum_{i in segment} c[i] z^(i - seg_start)
 __global__ void __launch_bounds__(EVAL_THREADS)
-eval_segments_kernel(const u64* __restrict__ coeffs, u64 col_stride, u64 n, u64 seg_len, Ext2 z, Ext2* __restrict__ partial) {
+eval_segments_kernel(EvalList L, u64 n, u64 seg_len, Ext2* __restrict__ partial) {
     __shared__ Ext2 red[EVAL_THREADS];
     const u32 t = threadIdx.x;
-    const u64 seg = blockIdx.x, col = blockIdx.y;
+    const u64 seg = blockIdx.x, e = blockIdx.y;
     const u64 i0 = seg * seg_len;
     const u64 i1 = (i0 + seg_len < n) ? i0 + seg_len : n;
-    const u64* c = coeffs + col * col_stride;
+    const u64* c;
+    Ext2 z;
+    eval_entry(L, e, &c, &z);
     const Ext2 y = ext_pow(z, EVAL_THREADS);
     // this thread's coefficients: i0 + t, i0 + t + 256, ...; Horner from the top
     Ext2 acc; acc.a = 0; acc.b = 0;
@@ -64,17 +85,20 @@ eval_segments_kernel(const u64* __restrict__ coeffs, u64 col_stride, u64 n, u64 
         if (t < s) red[t] = ext_add(red[t], red[t + s]);
         __syncthreads();
     }
-    if (t == 0) partial[col * gridDim.x + seg] = red[0];
+    if (t == 0) partial[e * gridDim.x + seg] = red[0];
 }
 
-// out[col] = sum_s z^(s * seg_len) * partial[col][s]
-__global__ void eval_combine_kernel(const Ext2* __restrict__ partial, u32 n_seg, u64 seg_len, u32 k, Ext2 z, Ext2* __restrict__ out) {
-    u32 col = blockIdx.x * blockDim.x + threadIdx.x;
-    if (col >= k) return;
+// out[e] = sum_s z_e^(s * seg_len) * partial[e][s]
+__global__ void eval_combine_kernel(EvalList L, const Ext2* __restrict__ partial, u32 n_seg, u64 seg_len, u32 m, Ext2* __restrict__ out) {
+    u32 e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= m) return;
+    const u64* c;
+    Ext2 z;
+    eval_entry(L, e, &c, &z);
     Ext2 step = ext_pow(z, seg_len);
     Ext2 acc; acc.a = 0; acc.b = 0;
-    for (u32 s = n_seg; s-- > 0;) acc = ext_add(ext_mul(acc, step), partial[(u64)col * n_seg + s]);
-    out[col] = acc;
+    for (u32 s = n_seg; s-- > 0;) acc = ext_add(ext_mul(acc, step), partial[(u64)e * n_seg + s]);
+    out[e] = acc;
 }
 #endif
 

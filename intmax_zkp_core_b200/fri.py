@@ -220,6 +220,35 @@ class FriProof:
     pow_witness: int
 
 
+def _instance_args(instance: FriInstanceInfo, oracles: Sequence[PolynomialBatch]):
+    """oracles, n_oracles, n_points, points, point_n_polys, poly_oracle, poly_index as b200zkp_fri_begin and
+    b200zkp_batch_openings take them (each pointer keeps its array alive)"""
+    handles = (C.c_void_p * len(oracles))(*[o._h for o in oracles])
+    points = _u64([list(b.point) for b in instance.batches]).reshape(-1)
+    counts = np.array([len(b.polynomials) for b in instance.batches], dtype=np.uint32)
+    po = np.array([p.oracle_index for b in instance.batches for p in b.polynomials], dtype=np.uint32)
+    pi = np.array([p.polynomial_index for b in instance.batches for p in b.polynomials], dtype=np.uint32)
+    return (handles, len(oracles), len(instance.batches), _p(points), counts.ctypes.data_as(C.c_void_p),
+            po.ctypes.data_as(C.c_void_p), pi.ctypes.data_as(C.c_void_p))
+
+
+def batch_openings(instance: FriInstanceInfo, oracles: Sequence[PolynomialBatch], ctx: Optional[Context] = None) -> List[List[Ext]]:
+    """OpeningSet::new in its FRI form (to_fri_openings): the value of every polynomial of `instance` at its batch's point,
+    batch after batch, in the order the challenger observes them.  One device call for the whole instance
+    (b200zkp_batch_openings) on the resident coefficients."""
+    ctx = ctx or oracles[0]._ctx
+    m = sum(len(b.polynomials) for b in instance.batches)
+    out = np.empty((max(m, 1), 2), dtype=np.uint64)
+    args = _instance_args(instance, oracles)
+    ctx.check(ctx._lib.b200zkp_batch_openings(ctx._h, *args, _p(out)))
+    vals = [(int(a), int(b)) for a, b in out[:m]]
+    res, off = [], 0
+    for b in instance.batches:
+        res.append(vals[off:off + len(b.polynomials)])
+        off += len(b.polynomials)
+    return res
+
+
 class FriCommitPhase:
     """Device state of one opening proof: current coefficients / values and the committed layer trees."""
 
@@ -231,16 +260,10 @@ class FriCommitPhase:
                      ctx: Optional[Context] = None) -> "FriCommitPhase":
         """prove_openings up to (and including) `lde_final_values`."""
         ctx = ctx or oracles[0]._ctx
-        handles = (C.c_void_p * len(oracles))(*[o._h for o in oracles])
-        points = _u64([list(b.point) for b in instance.batches]).reshape(-1)
-        counts = np.array([len(b.polynomials) for b in instance.batches], dtype=np.uint32)
-        po = np.array([p.oracle_index for b in instance.batches for p in b.polynomials], dtype=np.uint32)
-        pi = np.array([p.polynomial_index for b in instance.batches for p in b.polynomials], dtype=np.uint32)
         a = _u64(list(alpha))
         h = C.c_void_p()
-        ctx.check(ctx._lib.b200zkp_fri_begin(ctx._h, handles, len(oracles), len(instance.batches), _p(points),
-                                             counts.ctypes.data_as(C.c_void_p), po.ctypes.data_as(C.c_void_p),
-                                             pi.ctypes.data_as(C.c_void_p), _p(a), FRI_MUL_BY_X if mul_by_x else 0, C.byref(h)))
+        ctx.check(ctx._lib.b200zkp_fri_begin(ctx._h, *_instance_args(instance, oracles), _p(a), FRI_MUL_BY_X if mul_by_x else 0,
+                                             C.byref(h)))
         return cls(ctx, h)
 
     @classmethod

@@ -410,9 +410,12 @@ class _BatchMerkleTree:
 
     def __init__(self, batch: "PolynomialBatch"):
         self._b = batch
-        self.cap = batch._cap
         self._digests = None
         self._leaves = None
+
+    @property
+    def cap(self) -> MerkleCap:
+        return self._b._cap
 
     @property
     def leaves(self) -> np.ndarray:
@@ -514,6 +517,56 @@ class PolynomialBatch:
     def from_coeffs(cls, polynomials, rate_bits: int, blinding: bool, cap_height: int, timing=None,
                     fft_root_table=None, salt=None, ctx: Optional[Context] = None, copy_back: bool = False) -> "PolynomialBatch":
         return cls._commit(polynomials, True, rate_bits, blinding, cap_height, salt, ctx, copy_back)
+
+    @classmethod
+    def from_device(cls, tensor, rate_bits: int, blinding: bool, cap_height: int, is_coeffs: bool = False,
+                    ctx: Optional[Context] = None, salt=None) -> "PolynomialBatch":
+        """from_values (from_coeffs with is_coeffs) of a (k, n) CUDA tensor of 64-bit words already in HBM
+        (b200zkp_batch_from_device): asynchronous on the ctx stream, nothing crosses PCIe.  The batch keeps `tensor` (and
+        `salt`, (4, N) on the device when blinding) alive for its own lifetime, so the commit never reads freed memory.
+        `coeffs` and `lde` are torch views of the handle's coefficients and leaf-order LDE."""
+        from .device import _dev_view
+        ctx = ctx or default_context()
+        if tensor.dim() != 2 or not tensor.is_cuda or not tensor.is_contiguous() or tensor.element_size() != 8 or tensor.shape[0] == 0:
+            raise ValueError("expected a non-empty contiguous (k, n) CUDA tensor of 64-bit words")
+        k, n = tensor.shape
+        n_log = log2_strict(n)
+        if cap_height > n_log + rate_bits:
+            raise ValueError(f"cap_height={cap_height} should be at most log2(leaves.len())={n_log + rate_bits}")
+        if blinding:
+            if salt is None or tuple(salt.shape) != (SALT_SIZE, n << rate_bits) or not salt.is_cuda or not salt.is_contiguous():
+                raise ValueError(f"blinding needs a contiguous ({SALT_SIZE}, {n << rate_bits}) CUDA salt tensor")
+        else:
+            salt = None
+        h = C.c_void_p()
+        ctx.check(ctx._lib.b200zkp_batch_from_device(ctx._h, C.c_void_p(tensor.data_ptr()), int(is_coeffs), n_log, k, rate_bits,
+                                                     cap_height, C.c_void_p(salt.data_ptr()) if salt is not None else None,
+                                                     C.byref(h)))
+        self = object.__new__(cls)
+        self._ctx, self._h, self._keep = ctx, h, (tensor, salt)
+        self.degree_log, self.rate_bits, self.blinding, self.cap_height = n_log, rate_bits, bool(blinding), cap_height
+        self.num_polys, self.salt_size = k, SALT_SIZE if blinding else 0
+        self._polys = None
+        coeffs, lde, _, cap = self.device_ptrs()
+        self.coeffs = _dev_view(coeffs, (k, n), ctx.device)
+        self.lde = _dev_view(lde, (k + self.salt_size, n << rate_bits), ctx.device)
+        self._cap_dev = _dev_view(cap, (1 << cap_height, 4), ctx.device)
+        self._cap_host = None
+        self.merkle_tree = _BatchMerkleTree(self)
+        return self
+
+    @property
+    def _cap(self) -> MerkleCap:
+        """the Merkle cap, read back on first use (for a device commit that synchronises the ctx stream)"""
+        if self._cap_host is None:
+            cap = np.empty((1 << self.cap_height, 4), dtype=np.uint64)
+            self._ctx.check(self._ctx._lib.b200zkp_batch_cap(self._h, _p(cap)))
+            self._cap_host = MerkleCap(cap)
+        return self._cap_host
+
+    @_cap.setter
+    def _cap(self, cap: MerkleCap):
+        self._cap_host = cap
 
     @property
     def polynomials(self) -> np.ndarray:

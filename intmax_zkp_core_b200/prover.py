@@ -12,11 +12,13 @@ the commitment without leaving HBM.  Same names and argument meaning as plonky2;
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence
+from dataclasses import dataclass
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from .plonky2 import Context, P, PolynomialBatch, _p, _u64, coset_ifft_batch, default_context, log2_strict
+from .fri import batch_openings
+from .plonky2 import Context, MerkleCap, P, PolynomialBatch, _p, _u64, coset_ifft_batch, default_context, log2_strict
 
 MULTIPLICATIVE_GROUP_GENERATOR = 7
 
@@ -135,12 +137,11 @@ def commit_quotient(quotient_values, degree_bits: int, rate_bits: int, blinding:
                                        blinding, cap_height, salt=salt, ctx=ctx)
 
 
-def commit_quotient_device(ctx: Context, quotient_values, degree_bits: int, rate_bits: int, cap_height: int,
-                           quotient_degree_factor: Optional[int] = None):
-    """device-resident form: (C, n << q) CUDA tensor of quotient values -> DeviceCommitment of the C * quotient_degree_factor
-    chunks (default 2^q); the coefficients never leave HBM (the divisibility check reads one flag back)"""
+def quotient_chunks_device(ctx: Context, quotient_values, degree_bits: int, quotient_degree_factor: Optional[int] = None):
+    """device-resident form of quotient_poly_chunks: (C, n << q) CUDA tensor of quotient values -> the (C * quotient_degree_factor,
+    n) coefficient chunks (default 2^q per challenge) in HBM; only the divisibility check (quotient_degree_factor < 2^q) reads
+    one flag back"""
     import torch
-    from .device import commit_device
     Cn, total = quotient_values.shape
     n = 1 << degree_bits
     assert quotient_values.is_cuda and quotient_values.is_contiguous() and total % n == 0
@@ -156,7 +157,17 @@ def commit_quotient_device(ctx: Context, quotient_values, degree_bits: int, rate
         if bool(coeffs[:, qdf * n:].any()):
             raise QuotientError("Quotient has failed: coefficients beyond quotient_degree_factor * n are not zero")
         coeffs = coeffs[:, :qdf * n].contiguous()
-    return commit_device(ctx, coeffs.view(Cn * qdf, n), rate_bits, cap_height, is_coeffs=True)
+        torch.cuda.current_stream(coeffs.device).synchronize()
+    return coeffs.view(Cn * qdf, n)
+
+
+def commit_quotient_device(ctx: Context, quotient_values, degree_bits: int, rate_bits: int, cap_height: int,
+                           quotient_degree_factor: Optional[int] = None):
+    """device-resident form: (C, n << q) CUDA tensor of quotient values -> DeviceCommitment of the C * quotient_degree_factor
+    chunks (default 2^q); the coefficients never leave HBM (the divisibility check reads one flag back)"""
+    from .device import commit_device
+    chunks = quotient_chunks_device(ctx, quotient_values, degree_bits, quotient_degree_factor)
+    return commit_device(ctx, chunks, rate_bits, cap_height, is_coeffs=True)
 
 
 # ------------------------------------------------------------------------------------------------ row N1b: compute_quotient_polys
@@ -237,3 +248,159 @@ def compute_quotient_values_device(ctx: Context, common: CommonCircuitData, cons
                                                    C.c_void_p(zs_partial_products_lde.data_ptr()), zs_partial_products_lde.stride(0),
                                                    C.c_void_p(out.data_ptr()), out.stride(0)))
     return out
+
+
+# ------------------------------------------------------------------------------------------------ the whole proof
+class CircuitData:
+    """What prove() needs of plonky2's CircuitData (prover_only + common): the CommonCircuitData above, the constants + sigmas
+    PolynomialBatch (committed from HBM), the sigma values on H as a CUDA tensor, circuit_digest, FriParams, num_challenges."""
+
+    def __init__(self, common: CommonCircuitData, constants_sigmas_commitment: PolynomialBatch, sigmas, circuit_digest,
+                 fri_params, num_challenges: int):
+        self.common, self.constants_sigmas_commitment, self.sigmas = common, constants_sigmas_commitment, sigmas
+        self.circuit_digest, self.fri_params, self.num_challenges = circuit_digest, fri_params, num_challenges
+
+    @property
+    def num_constants(self) -> int:
+        return self.common.num_selectors + 2
+
+
+def circuit_data(ctx: Context, common: CommonCircuitData, constants_sigmas_values, fri_config, num_challenges: int = 2) -> CircuitData:
+    """The commitment CircuitBuilder::build makes: constants_sigmas_values is the (num_constants + num_routed_wires, n) CUDA tensor
+    of selector + gate-constant columns followed by the sigma columns, values on H.  circuit_digest =
+    hash_no_pad(constants_sigmas_cap.flatten()) (restated from memory of plonky2 @ f99ed9c, unpinned like the rest)."""
+    from .plonky2 import PoseidonHash
+    if constants_sigmas_values.shape != (common.num_selectors + 2 + common.num_routed_wires, 1 << common.degree_bits):
+        raise ValueError("constants_sigmas_values must hold num_selectors + 2 + num_routed_wires columns of 2^degree_bits values")
+    cfg = fri_config
+    batch = PolynomialBatch.from_device(constants_sigmas_values, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
+    digest = PoseidonHash.hash_no_pad(batch._cap.flatten(), ctx)
+    return CircuitData(common, batch, constants_sigmas_values[common.num_selectors + 2:], digest,
+                       cfg.fri_params(common.degree_bits), num_challenges)
+
+
+@dataclass
+class OpeningSet:
+    """plonk/proof.rs OpeningSet: extension values (re, im) at zeta, plonk_zs_next at g zeta"""
+    constants: List[Tuple[int, int]]
+    plonk_sigmas: List[Tuple[int, int]]
+    wires: List[Tuple[int, int]]
+    plonk_zs: List[Tuple[int, int]]
+    plonk_zs_next: List[Tuple[int, int]]
+    partial_products: List[Tuple[int, int]]
+    quotient_polys: List[Tuple[int, int]]
+
+    def to_fri_openings(self) -> List[List[Tuple[int, int]]]:
+        """the values batch by batch, in the order the challenger observes them"""
+        return [self.constants + self.plonk_sigmas + self.wires + self.plonk_zs + self.partial_products + self.quotient_polys,
+                self.plonk_zs_next]
+
+
+@dataclass
+class Proof:
+    wires_cap: MerkleCap
+    plonk_zs_partial_products_cap: MerkleCap
+    quotient_polys_cap: MerkleCap
+    openings: OpeningSet
+    opening_proof: "FriProof"
+
+
+@dataclass
+class ProofWithPublicInputs:
+    proof: Proof
+    public_inputs: List[int]
+
+
+def fri_instance(data: CircuitData, zeta, oracles) -> "FriInstanceInfo":
+    """CommonCircuitData::get_fri_instance: every polynomial of the four oracles at zeta, the Zs at g zeta"""
+    from .fri import FriBatchInfo, FriInstanceInfo, FriPolynomialInfo
+    g = _root(data.common.degree_bits)
+    zeta_next = (zeta[0] * g % P, zeta[1] * g % P)
+    all_polys = [FriPolynomialInfo(o, i) for o, b in enumerate(oracles) for i in range(b.num_polys)]
+    zs = FriPolynomialInfo.from_range(2, range(data.num_challenges))
+    return FriInstanceInfo([FriBatchInfo(tuple(zeta), all_polys), FriBatchInfo(zeta_next, zs)])
+
+
+def _root(n_log: int) -> int:
+    return pow(1753635133440165772, 1 << (32 - n_log), P)
+
+
+def _ext_pow(x, e: int):
+    r, x = (1, 0), tuple(x)
+    while e:
+        if e & 1:
+            r = ((r[0] * x[0] + 7 * r[1] * x[1]) % P, (r[0] * x[1] + r[1] * x[0]) % P)
+        x = ((x[0] * x[0] + 7 * x[1] * x[1]) % P, 2 * x[0] * x[1] % P)
+        e >>= 1
+    return r
+
+
+PROVE_STAGES = ("wires_commit", "z", "z_commit", "quotient_values", "quotient_commit", "openings", "fri")
+
+
+def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool, on_stage=None) -> ProofWithPublicInputs:
+    """plonk/prover.rs prove() on the device, in plonky2's transcript order.  wires: the (135, n) CUDA tensor of witness values
+    (num_wires columns); it is only read.  Every polynomial stays in HBM: only challenges, caps, openings and query answers
+    cross PCIe.  Raises QuotientError for a witness whose vanishing polynomial is not divisible by Z_H (only checked when
+    quotient_degree_factor < 2^quotient_degree_bits).  mul_by_x has no default, for the reason fri.prove_openings gives.
+    on_stage(name), when given, is called as each stage is about to be enqueued (PROVE_STAGES) and with "end" after the last
+    one, e.g. to record CUDA events on the ctx stream."""
+    import torch
+    from .fri import Challenger, prove_openings
+    from .plonky2 import PoseidonHash
+    common, cfg = data.common, data.fri_params.config
+    n = 1 << common.degree_bits
+    if wires.dim() != 2 or wires.shape[1] != n or wires.shape[0] < 135 or not wires.is_cuda:
+        raise ValueError("wires must be a (num_wires, 2^degree_bits) CUDA tensor")
+    wires = wires.contiguous()
+    torch.cuda.current_stream(wires.device).synchronize()        # inputs written on torch's stream are complete
+    Cn = data.num_challenges
+    challenger = Challenger(ctx)
+    public_inputs_hash = PoseidonHash.hash_no_pad(_u64(list(public_inputs)), ctx)
+    challenger.observe_hash(data.circuit_digest)
+    challenger.observe_hash(public_inputs_hash)
+    stage = on_stage or (lambda name: None)
+
+    stage("wires_commit")
+    wires_commitment = PolynomialBatch.from_device(wires, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
+    challenger.observe_cap(wires_commitment._cap)
+    betas = challenger.get_n_challenges(Cn)
+    gammas = challenger.get_n_challenges(Cn)
+
+    stage("z")
+    zpp = zs_partial_products_device(ctx, wires[:common.num_routed_wires], data.sigmas, common.k_is, betas, gammas,
+                                     common.quotient_degree_factor)
+    stage("z_commit")
+    zpp_commitment = PolynomialBatch.from_device(zpp, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
+    challenger.observe_cap(zpp_commitment._cap)
+    alphas = challenger.get_n_challenges(Cn)
+
+    cs = data.constants_sigmas_commitment
+    stage("quotient_values")
+    q = compute_quotient_values_device(ctx, common, cs.lde, wires_commitment.lde, zpp_commitment.lde, betas, gammas, alphas,
+                                       public_inputs_hash.elements)
+    stage("quotient_commit")
+    chunks = quotient_chunks_device(ctx, q, common.degree_bits, common.quotient_degree_factor)
+    quotient_commitment = PolynomialBatch.from_device(chunks, cfg.rate_bits, False, cfg.cap_height, is_coeffs=True, ctx=ctx)
+    challenger.observe_cap(quotient_commitment._cap)
+
+    zeta = challenger.get_extension_challenge()
+    if _ext_pow(zeta, n) == (1, 0):
+        raise ValueError("Opening point is in the subgroup.")
+    oracles = [cs, wires_commitment, zpp_commitment, quotient_commitment]
+    instance = fri_instance(data, zeta, oracles)
+    stage("openings")
+    at_zeta, at_next = batch_openings(instance, oracles)
+    for values in (at_zeta, at_next):
+        challenger.observe_extension_elements(values)
+    nc = data.num_constants
+    k_cs, k_w = cs.num_polys, wires_commitment.num_polys
+    ow, oz = k_cs + k_w, k_cs + k_w + zpp_commitment.num_polys
+    openings = OpeningSet(constants=at_zeta[:nc], plonk_sigmas=at_zeta[nc:k_cs], wires=at_zeta[k_cs:ow],
+                          plonk_zs=at_zeta[ow:ow + Cn], plonk_zs_next=at_next, partial_products=at_zeta[ow + Cn:oz],
+                          quotient_polys=at_zeta[oz:])
+    stage("fri")
+    opening_proof = prove_openings(instance, oracles, challenger, data.fri_params, mul_by_x)
+    stage("end")
+    proof = Proof(wires_commitment._cap, zpp_commitment._cap, quotient_commitment._cap, openings, opening_proof)
+    return ProofWithPublicInputs(proof, [int(v) % P for v in public_inputs])

@@ -63,6 +63,7 @@ extern "C" {
         cap_height: u32, salt: *const u64, out: *mut *mut b200zkp_batch) -> c_int;
     pub fn b200zkp_batch_free(b: *mut b200zkp_batch);
     pub fn b200zkp_batch_cap(b: *mut b200zkp_batch, out: *mut u64) -> c_int;
+    pub fn b200zkp_batch_shape(b: *const b200zkp_batch, shape: *mut u32) -> c_int;
     pub fn b200zkp_batch_coeffs(b: *mut b200zkp_batch, out: *mut u64) -> c_int;
     pub fn b200zkp_batch_leaves(b: *mut b200zkp_batch, out: *mut u64) -> c_int;
     pub fn b200zkp_batch_digests(b: *mut b200zkp_batch, out: *mut u64) -> c_int;
@@ -80,6 +81,11 @@ extern "C" {
     pub fn b200zkp_two_to_one(ctx: *mut b200zkp_ctx, left: *const u64, right: *const u64, count: u64, out: *mut u64) -> c_int;
     // opening proof (prove_openings / fri_proof): see include/b200zkp.h and INTEGRATION.md
     pub fn b200zkp_batch_eval_ext2(b: *mut b200zkp_batch, zeta: *const u64, out: *mut u64) -> c_int;
+    // the whole prove() on the device: commitments of matrices already in HBM, OpeningSet::new in one call
+    pub fn b200zkp_batch_from_device(ctx: *mut b200zkp_ctx, in_dev: *const u64, is_coeffs: c_int, n_log: u32, k: u32,
+        rate_bits: u32, cap_height: u32, salt_dev: *const u64, out: *mut *mut b200zkp_batch) -> c_int;
+    pub fn b200zkp_batch_openings(ctx: *mut b200zkp_ctx, oracles: *const *mut b200zkp_batch, n_oracles: u32, n_points: u32,
+        points: *const u64, point_n_polys: *const u32, poly_oracle: *const u32, poly_index: *const u32, out: *mut u64) -> c_int;
     pub fn b200zkp_fri_begin(ctx: *mut b200zkp_ctx, oracles: *const *mut b200zkp_batch, n_oracles: u32, n_points: u32,
         points: *const u64, point_n_polys: *const u32, poly_oracle: *const u32, poly_index: *const u32, alpha: *const u64,
         flags: u32, out: *mut *mut b200zkp_fri) -> c_int;

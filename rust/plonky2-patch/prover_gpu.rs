@@ -54,3 +54,66 @@ fn quotient_poly_chunks<F: RichField>(quotient_values: Vec<Vec<F>>, degree: usiz
     assert_eq!(rc, 0, "b200zkp_coset_intt failed");
     flat.chunks(degree).map(|c| PolynomialCoeffs::new(c.iter().map(|&x| F::from_canonical_u64(x)).collect())).collect()
 }
+
+/// The whole prove() (zero_knowledge = false) with every polynomial resident in HBM, in plonky2's transcript order
+/// (the sequence intmax_zkp_core_b200/prover.py::prove runs and tests/test_gpu_prove.py checks word for word).
+/// `wires_dev`: the 135 x n column-major witness matrix already on the device; `cs`: the constants + sigmas handle that
+/// CircuitBuilder::build committed with b200zkp_batch_from_device, `sigmas_dev` its sigma columns.  Sketch only: the
+/// device allocations, the vanishing descriptor and the FRI query loop are those of prover.py / fri.py.
+#[allow(dead_code)]
+fn prove_gpu<F: RichField + Extendable<D>, C: GenericConfig<D, F = F>, const D: usize>(
+    ctx: *mut sys::b200zkp_ctx,
+    cs: *mut sys::b200zkp_batch,
+    sigmas_dev: *const u64,
+    wires_dev: *const u64,
+    public_inputs: &[F],
+    circuit_digest: &[F; 4],
+    common_data: &CommonCircuitData<F, C, D>,
+    challenger: &mut crate::iop::challenger::Challenger<F, C::Hasher>,
+) {
+    let n_log = common_data.degree_bits() as u32;
+    let n = 1u64 << n_log;
+    let cfg = &common_data.config.fri_config;
+    let nc = common_data.config.num_challenges;
+    let commit = |input: *const u64, k: usize, is_coeffs: bool| {
+        let mut b = std::ptr::null_mut();
+        assert_eq!(unsafe { sys::b200zkp_batch_from_device(ctx, input, is_coeffs as i32, n_log, k as u32, cfg.rate_bits as u32,
+                                                            cfg.cap_height as u32, std::ptr::null(), &mut b) }, 0);
+        b
+    };
+    // 1. circuit digest, public inputs hash
+    challenger.observe_elements(circuit_digest);
+    challenger.observe_hash::<C::InnerHasher>(C::InnerHasher::hash_no_pad(public_inputs));
+    // 2. wires
+    let wires = commit(wires_dev, common_data.config.num_wires, false);
+    // observe_cap(b200zkp_batch_cap(wires)); betas = get_n_challenges(nc); gammas = get_n_challenges(nc)
+    // 3. Z + partial products: b200zkp_dev_partial_products_and_zs(ctx, wires_dev, n, sigmas_dev, n, ...) into zpp_dev
+    let zpp_dev: *const u64 = std::ptr::null(); // (device buffer of nc * (1 + num_partial_products) columns)
+    let zpp = commit(zpp_dev, nc * (1 + common_data.num_partial_products), false);
+    // observe_cap(zpp); alphas = get_n_challenges(nc)
+    // 4. quotient: b200zkp_dev_quotient_values on the LDE pointers of cs / wires / zpp (b200zkp_batch_device_ptrs),
+    //    b200zkp_dev_coset_intt(shift 7) into chunks_dev, then
+    let chunks_dev: *const u64 = std::ptr::null();
+    let quotient = commit(chunks_dev, nc * common_data.quotient_degree_factor, true);
+    // observe_cap(quotient)
+    // 5. zeta = get_extension_challenge(); ensure!(zeta.exp_power_of_2(degree_bits) != ONE)
+    // 6. OpeningSet::new + to_fri_openings in one call: every polynomial of the four oracles at zeta, the Zs at g zeta
+    let oracles = [cs, wires, zpp, quotient];
+    let mut counts = [0u32; 2];
+    let (mut po, mut pi) = (Vec::new(), Vec::new());
+    for (o, &b) in oracles.iter().enumerate() {
+        let mut shape = [0u32; 5];
+        unsafe { sys::b200zkp_batch_shape(b, shape.as_mut_ptr()) };
+        for i in 0..shape[1] { po.push(o as u32); pi.push(i); }
+        counts[0] += shape[1];
+    }
+    for i in 0..nc as u32 { po.push(2); pi.push(i); }
+    counts[1] = nc as u32;
+    let points = [0u64; 4]; // (zeta, g * zeta) as (re, im) pairs
+    let mut openings = vec![0u64; 2 * po.len()];
+    assert_eq!(unsafe { sys::b200zkp_batch_openings(ctx, oracles.as_ptr(), 4, 2, points.as_ptr(), counts.as_ptr(), po.as_ptr(),
+                                                    pi.as_ptr(), openings.as_mut_ptr()) }, 0);
+    // challenger.observe_extension_elements per batch, then
+    // 7. PolynomialBatch::prove_openings(get_fri_instance(zeta), [cs, wires, zpp, quotient]) through b200zkp_fri_begin (oracle_gpu.rs)
+    let _ = (n, wires, zpp, quotient);
+}
