@@ -235,6 +235,16 @@ int b200zkp_dev_lde(b200zkp_ctx* ctx, const uint64_t* coeffs, uint64_t coeff_str
 /* salt [4][N] natural order -> rows of lde columns in leaf order for blocks [block_begin, block_end) */
 int b200zkp_dev_salt(b200zkp_ctx* ctx, const uint64_t* salt, uint64_t* lde_salt_cols, uint64_t lde_stride,
                      uint32_t n_log, uint32_t rate_bits, uint32_t block_begin, uint32_t block_end);
+/* F::rand_vec on the device: out_dev[e] = element (first + e) of the stream (key, nonce), e < count; async on the ctx stream.
+ * The stream: ChaCha20 of RFC 8439 (20 rounds, key and nonce read as little-endian words, 32-bit block counter from 0).
+ * Element j is keystream bytes [16 j, 16 j + 16) read as little-endian u64 lo, hi: (lo + 2^64 hi) mod p, canonical (within
+ * 2^-64 of uniform; plonky2's own draw is exactly uniform).  key and nonce are host pointers, read before the call returns.
+ * The salts of a blinded commitment: 4N elements, element c*N + i = salt column c at natural LDE row i, the salt_dev layout
+ * of b200zkp_batch_from_device.  The key must be secret and fresh for every proof (drawn from the OS); a nonce per oracle.
+ * count == 0 launches nothing.  B200ZKP_ERR_BAD_ARG: a null key, nonce or out_dev with count > 0, or a range that needs a
+ * block counter of 2^32 or more (first + count > 2^34). */
+int b200zkp_dev_random_field(b200zkp_ctx* ctx, const uint8_t key[32], const uint8_t nonce[12], uint64_t first,
+                             uint64_t count, uint64_t* out_dev);
 /* Merkle forest over n_leaves leaves, element (row, c) at leaves[row*row_stride + c*col_stride]:
  * digests 4*2*(n_leaves - 2^cap_height), cap 4*2^cap_height (both device). */
 int b200zkp_dev_merkle(b200zkp_ctx* ctx, const uint64_t* leaves, uint64_t row_stride, uint64_t col_stride,

@@ -139,6 +139,7 @@ _SIGS = {
     "b200zkp_dev_intt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_uint32]),
     "b200zkp_dev_lde": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
     "b200zkp_dev_salt": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32]),
+    "b200zkp_dev_random_field": (C.c_int, [C.c_void_p, C.c_char_p, C.c_char_p, C.c_uint64, C.c_uint64, C.c_void_p]),
     "b200zkp_dev_merkle": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p]),
     "b200zkp_dev_lde_merkle": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p]),
     "b200zkp_dev_commit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -23,6 +23,7 @@
 #include "fri_kernels.cuh"
 #include "perm_kernels.cuh"
 #include "vanishing_kernels.cuh"
+#include "random_kernels.cuh"
 #include "host_plan.hpp"
 
 using gl::u32;
@@ -832,6 +833,25 @@ extern "C" int b200zkp_dev_salt(b200zkp_ctx* ctx, const uint64_t* salt, uint64_t
     Guard g(ctx);
     if (!salt || !lde_salt_cols) BAD(ctx, "null buffer");
     return dev_salt_locked(ctx, (const u64*)salt, (u64*)lde_salt_cols, lde_stride, n_log, rate_bits, block_begin, block_end);
+}
+
+// F::rand_vec: elements [first, first + count) of the ChaCha20 stream (key, nonce), one thread per block (random_kernels.cuh)
+extern "C" int b200zkp_dev_random_field(b200zkp_ctx* ctx, const uint8_t key[32], const uint8_t nonce[12], uint64_t first,
+                                        uint64_t count, uint64_t* out_dev) {
+    if (!ctx) return B200ZKP_ERR_BAD_ARG;
+    Guard g(ctx);
+    if (!count) return 0;
+    if (!key || !nonce || !out_dev) BAD(ctx, "null key, nonce or output");
+    if (!rnd::range_ok(first, count)) BAD(ctx, "the range needs a ChaCha20 block counter of 2^32 or more (first + count > 2^34)");
+    rnd::ChaChaKey k;
+    for (int i = 0; i < 8; i++)
+        k.key[i] = (u32)key[4 * i] | (u32)key[4 * i + 1] << 8 | (u32)key[4 * i + 2] << 16 | (u32)key[4 * i + 3] << 24;
+    for (int i = 0; i < 3; i++)
+        k.nonce[i] = (u32)nonce[4 * i] | (u32)nonce[4 * i + 1] << 8 | (u32)nonce[4 * i + 2] << 16 | (u32)nonce[4 * i + 3] << 24;
+    const u64 n_blocks = rnd::blocks_of_range(first, count);
+    rnd::random_field_kernel<<<(unsigned)((n_blocks + 255) / 256), 256, 0, ctx->stream>>>(k, first, count, n_blocks, (u64*)out_dev);
+    LAUNCH_CHECK(ctx);
+    return 0;
 }
 
 static int merkle_shape(b200zkp_ctx* ctx, u64 n_leaves, u32 cap_height, const void* leaves, const void* digests, const void* cap,

@@ -12,13 +12,14 @@ the commitment without leaving HBM.  Same names and argument meaning as plonky2;
 from __future__ import annotations
 
 import ctypes as C
+import secrets
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
 from .fri import batch_openings
-from .plonky2 import Context, MerkleCap, P, PolynomialBatch, _p, _u64, coset_ifft_batch, default_context, log2_strict
+from .plonky2 import SALT_SIZE, Context, MerkleCap, P, PolynomialBatch, _p, _u64, coset_ifft_batch, default_context, log2_strict
 
 MULTIPLICATIVE_GROUP_GENERATOR = 7
 
@@ -250,25 +251,63 @@ def compute_quotient_values_device(ctx: Context, common: CommonCircuitData, cons
     return out
 
 
+# ------------------------------------------------------------------------------------------------ salts
+def random_field_device(ctx: Context, key: bytes, nonce: bytes, count: int, first: int = 0, out=None):
+    """F::rand_vec on the device (b200zkp_dev_random_field): elements [first, first + count) of the ChaCha20 stream (key, nonce)
+    as a (count,) int64 CUDA tensor of canonical field elements, written asynchronously on the ctx stream.  key: 32 bytes, secret;
+    nonce: 12 bytes.  out: a contiguous int64 CUDA tensor of `count` elements to fill instead of a new one."""
+    import torch
+    key, nonce = bytes(key), bytes(nonce)
+    if len(key) != 32 or len(nonce) != 12:
+        raise ValueError("the key must be 32 bytes and the nonce 12 bytes")
+    if out is None:
+        out = torch.empty(int(count), dtype=torch.int64, device=f"cuda:{ctx.device}")
+    elif not out.is_cuda or out.dtype != torch.int64 or not out.is_contiguous() or out.numel() != count:
+        raise ValueError("out must be a contiguous int64 CUDA tensor of `count` elements")
+    ctx.check(ctx._lib.b200zkp_dev_random_field(ctx._h, key, nonce, int(first), int(count),
+                                                C.c_void_p(out.data_ptr()) if count else None))
+    return out
+
+
+# PlonkOracle indices: the salt of oracle i is drawn with the nonce le32(i) || 0^8
+PLONK_ORACLE_WIRES, PLONK_ORACLE_ZS_PARTIAL_PRODUCTS, PLONK_ORACLE_QUOTIENT = 1, 2, 3
+
+
+def oracle_nonce(oracle_index: int) -> bytes:
+    return int(oracle_index).to_bytes(4, "little") + bytes(8)
+
+
+def salt_device(ctx: Context, key: bytes, oracle_index: int, lde_size: int):
+    """the (SALT_SIZE, N) salt of one blinded commitment: elements [0, SALT_SIZE * N) of the stream (key, oracle_nonce(oracle_index)),
+    element c*N + i = salt column c at natural LDE row i (the layout PolynomialBatch.from_device takes)"""
+    return random_field_device(ctx, key, oracle_nonce(oracle_index), SALT_SIZE * lde_size).view(SALT_SIZE, lde_size)
+
+
 # ------------------------------------------------------------------------------------------------ the whole proof
 class CircuitData:
     """What prove() needs of plonky2's CircuitData (prover_only + common): the CommonCircuitData above, the constants + sigmas
-    PolynomialBatch (committed from HBM), the sigma values on H as a CUDA tensor, circuit_digest, FriParams, num_challenges."""
+    PolynomialBatch (committed from HBM), the sigma values on H as a CUDA tensor, circuit_digest, FriParams, num_challenges,
+    and CircuitConfig::zero_knowledge (fri_params.hiding follows it)."""
 
     def __init__(self, common: CommonCircuitData, constants_sigmas_commitment: PolynomialBatch, sigmas, circuit_digest,
-                 fri_params, num_challenges: int):
+                 fri_params, num_challenges: int, zero_knowledge: bool = False):
         self.common, self.constants_sigmas_commitment, self.sigmas = common, constants_sigmas_commitment, sigmas
         self.circuit_digest, self.fri_params, self.num_challenges = circuit_digest, fri_params, num_challenges
+        self.zero_knowledge = bool(zero_knowledge)
 
     @property
     def num_constants(self) -> int:
         return self.common.num_selectors + 2
 
 
-def circuit_data(ctx: Context, common: CommonCircuitData, constants_sigmas_values, fri_config, num_challenges: int = 2) -> CircuitData:
+def circuit_data(ctx: Context, common: CommonCircuitData, constants_sigmas_values, fri_config, num_challenges: int = 2,
+                 zero_knowledge: bool = False) -> CircuitData:
     """The commitment CircuitBuilder::build makes: constants_sigmas_values is the (num_constants + num_routed_wires, n) CUDA tensor
     of selector + gate-constant columns followed by the sigma columns, values on H.  circuit_digest =
-    hash_no_pad(constants_sigmas_cap.flatten()) (restated from memory of plonky2 @ f99ed9c, unpinned like the rest)."""
+    hash_no_pad(constants_sigmas_cap.flatten()) (restated from memory of plonky2 @ f99ed9c, unpinned like the rest).
+    zero_knowledge: prove() salts the wires, Z + partial products and quotient commitments and FriParams.hiding is set; the
+    blinding rows are part of the circuit the caller describes (CircuitBuilder::blind_and_pad).  Constants + sigmas are never
+    salted."""
     from .plonky2 import PoseidonHash
     if constants_sigmas_values.shape != (common.num_selectors + 2 + common.num_routed_wires, 1 << common.degree_bits):
         raise ValueError("constants_sigmas_values must hold num_selectors + 2 + num_routed_wires columns of 2^degree_bits values")
@@ -276,7 +315,7 @@ def circuit_data(ctx: Context, common: CommonCircuitData, constants_sigmas_value
     batch = PolynomialBatch.from_device(constants_sigmas_values, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
     digest = PoseidonHash.hash_no_pad(batch._cap.flatten(), ctx)
     return CircuitData(common, batch, constants_sigmas_values[common.num_selectors + 2:], digest,
-                       cfg.fri_params(common.degree_bits), num_challenges)
+                       cfg.fri_params(common.degree_bits, hiding=bool(zero_knowledge)), num_challenges, zero_knowledge)
 
 
 @dataclass
@@ -318,7 +357,8 @@ def fri_instance(data: CircuitData, zeta, oracles) -> "FriInstanceInfo":
     zeta_next = (zeta[0] * g % P, zeta[1] * g % P)
     all_polys = [FriPolynomialInfo(o, i) for o, b in enumerate(oracles) for i in range(b.num_polys)]
     zs = FriPolynomialInfo.from_range(2, range(data.num_challenges))
-    return FriInstanceInfo([FriBatchInfo(tuple(zeta), all_polys), FriBatchInfo(zeta_next, zs)])
+    zk = data.zero_knowledge
+    return FriInstanceInfo([FriBatchInfo(tuple(zeta), all_polys), FriBatchInfo(zeta_next, zs)], oracles_blinding=[False, zk, zk, zk])
 
 
 def _root(n_log: int) -> int:
@@ -338,13 +378,17 @@ def _ext_pow(x, e: int):
 PROVE_STAGES = ("wires_commit", "z", "z_commit", "quotient_values", "quotient_commit", "openings", "fri")
 
 
-def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool, on_stage=None) -> ProofWithPublicInputs:
+def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool, on_stage=None, salt_key=None) -> ProofWithPublicInputs:
     """plonk/prover.rs prove() on the device, in plonky2's transcript order.  wires: the (135, n) CUDA tensor of witness values
     (num_wires columns); it is only read.  Every polynomial stays in HBM: only challenges, caps, openings and query answers
     cross PCIe.  Raises QuotientError for a witness whose vanishing polynomial is not divisible by Z_H (only checked when
     quotient_degree_factor < 2^quotient_degree_bits).  mul_by_x has no default, for the reason fri.prove_openings gives.
     on_stage(name), when given, is called as each stage is about to be enqueued (PROVE_STAGES) and with "end" after the last
-    one, e.g. to record CUDA events on the ctx stream."""
+    one, e.g. to record CUDA events on the ctx stream.
+    With data.zero_knowledge, the wires, Z + partial products and quotient commitments are salted (plonky2's blinding = true):
+    each salt is generated on the device inside its commit stage from the ChaCha20 stream of salt_key (random_field_device,
+    nonce = the PlonkOracle index).  salt_key defaults to 32 fresh bytes from the OS for every proof; pass one only to
+    reproduce a proof.  A salt_key for a circuit without zero_knowledge, or one that is not 32 bytes, is a ValueError."""
     import torch
     from .fri import Challenger, prove_openings
     from .plonky2 import PoseidonHash
@@ -352,6 +396,15 @@ def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool,
     n = 1 << common.degree_bits
     if wires.dim() != 2 or wires.shape[1] != n or wires.shape[0] < 135 or not wires.is_cuda:
         raise ValueError("wires must be a (num_wires, 2^degree_bits) CUDA tensor")
+    zk = data.zero_knowledge
+    if salt_key is not None and not zk:
+        raise ValueError("salt_key is only used when the circuit has zero_knowledge")
+    if zk:
+        salt_key = secrets.token_bytes(32) if salt_key is None else bytes(salt_key)
+        if len(salt_key) != 32:
+            raise ValueError("salt_key must be 32 bytes")
+    N = n << cfg.rate_bits
+    salt = (lambda oracle: salt_device(ctx, salt_key, oracle, N)) if zk else (lambda oracle: None)
     wires = wires.contiguous()
     torch.cuda.current_stream(wires.device).synchronize()        # inputs written on torch's stream are complete
     Cn = data.num_challenges
@@ -362,7 +415,7 @@ def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool,
     stage = on_stage or (lambda name: None)
 
     stage("wires_commit")
-    wires_commitment = PolynomialBatch.from_device(wires, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
+    wires_commitment = PolynomialBatch.from_device(wires, cfg.rate_bits, zk, cfg.cap_height, ctx=ctx, salt=salt(PLONK_ORACLE_WIRES))
     challenger.observe_cap(wires_commitment._cap)
     betas = challenger.get_n_challenges(Cn)
     gammas = challenger.get_n_challenges(Cn)
@@ -371,17 +424,21 @@ def prove(ctx: Context, data: CircuitData, wires, public_inputs, mul_by_x: bool,
     zpp = zs_partial_products_device(ctx, wires[:common.num_routed_wires], data.sigmas, common.k_is, betas, gammas,
                                      common.quotient_degree_factor)
     stage("z_commit")
-    zpp_commitment = PolynomialBatch.from_device(zpp, cfg.rate_bits, False, cfg.cap_height, ctx=ctx)
+    zpp_commitment = PolynomialBatch.from_device(zpp, cfg.rate_bits, zk, cfg.cap_height, ctx=ctx,
+                                                 salt=salt(PLONK_ORACLE_ZS_PARTIAL_PRODUCTS))
     challenger.observe_cap(zpp_commitment._cap)
     alphas = challenger.get_n_challenges(Cn)
 
     cs = data.constants_sigmas_commitment
     stage("quotient_values")
-    q = compute_quotient_values_device(ctx, common, cs.lde, wires_commitment.lde, zpp_commitment.lde, betas, gammas, alphas,
+    # (the salt columns come last in a blinded LDE: the quotient reads the polynomial columns only, as get_lde_values does)
+    q = compute_quotient_values_device(ctx, common, cs.lde, wires_commitment.lde[:wires_commitment.num_polys],
+                                       zpp_commitment.lde[:zpp_commitment.num_polys], betas, gammas, alphas,
                                        public_inputs_hash.elements)
     stage("quotient_commit")
     chunks = quotient_chunks_device(ctx, q, common.degree_bits, common.quotient_degree_factor)
-    quotient_commitment = PolynomialBatch.from_device(chunks, cfg.rate_bits, False, cfg.cap_height, is_coeffs=True, ctx=ctx)
+    quotient_commitment = PolynomialBatch.from_device(chunks, cfg.rate_bits, zk, cfg.cap_height, is_coeffs=True, ctx=ctx,
+                                                      salt=salt(PLONK_ORACLE_QUOTIENT))
     challenger.observe_cap(quotient_commitment._cap)
 
     zeta = challenger.get_extension_challenge()

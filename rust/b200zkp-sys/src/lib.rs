@@ -11,6 +11,7 @@ use std::os::raw::{c_char, c_int, c_void};
 #[repr(C)] pub struct b200zkp_sharded { _p: [u8; 0] }
 
 pub const B200ZKP_COMM_ID_BYTES: usize = 128;
+pub const B200ZKP_SALT_SIZE: u32 = 4; // plonky2 fri/oracle.rs SALT_SIZE
 pub const B200ZKP_MAX_GATES: usize = 16;
 /// gate kinds of `b200zkp_vanishing_desc::gate_kind` (include/b200zkp.h B200ZKP_GATE_*); parameters in `gate_params`
 pub const B200ZKP_GATE_NOOP: u32 = 0;
@@ -84,6 +85,9 @@ extern "C" {
     // the whole prove() on the device: commitments of matrices already in HBM, OpeningSet::new in one call
     pub fn b200zkp_batch_from_device(ctx: *mut b200zkp_ctx, in_dev: *const u64, is_coeffs: c_int, n_log: u32, k: u32,
         rate_bits: u32, cap_height: u32, salt_dev: *const u64, out: *mut *mut b200zkp_batch) -> c_int;
+    // zero_knowledge: F::rand_vec on the device, out_dev[e] = element (first + e) of the ChaCha20 stream (key, nonce)
+    pub fn b200zkp_dev_random_field(ctx: *mut b200zkp_ctx, key: *const u8, nonce: *const u8, first: u64, count: u64,
+        out_dev: *mut u64) -> c_int;
     pub fn b200zkp_batch_openings(ctx: *mut b200zkp_ctx, oracles: *const *mut b200zkp_batch, n_oracles: u32, n_points: u32,
         points: *const u64, point_n_polys: *const u32, poly_oracle: *const u32, poly_index: *const u32, out: *mut u64) -> c_int;
     pub fn b200zkp_fri_begin(ctx: *mut b200zkp_ctx, oracles: *const *mut b200zkp_batch, n_oracles: u32, n_points: u32,
