@@ -367,7 +367,7 @@ int b200zkp_dev_quotient_values(b200zkp_ctx* ctx, const b200zkp_vanishing_desc* 
  *     the owners' windows over NVLink and files them in the local coefficient matrix on the way (one fused kernel, no NCCL
  *     call, no staging); ordering by epoch-stamped flags in peer memory (CUDA events inside one process).  Host inputs form a
  *     pipeline of column chunks: upload / inverse transform / gather + coset transforms / sponge absorption.
- *   NCCL exchange (fallback, or b200zkp_comm_set_peer_exchange(comm, 0) / B200ZKP_PEER_EXCHANGE=0): point-to-point groups into
+ *   NCCL exchange (fallback, or b200zkp_comm_set_peer_exchange(comm, 0)): point-to-point groups into
  *     a local gather buffer after the inverse transforms; the same kernels then read the shards from there.
  *
  * Two ways to form the communicator, matching how the caller is deployed:

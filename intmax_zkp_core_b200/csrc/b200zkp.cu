@@ -56,12 +56,8 @@ struct b200zkp_ctx {
     struct ZTables { const u64* strided = nullptr; const u64* final_ = nullptr; };   // see ntc::ztab_entries / zfinal_words
     std::map<std::pair<u32, u32>, ZTables> ztab_lde;    // (n_log, rate_bits) -> forward transform on every leaf block's coset
     std::map<u32, ZTables> ztab_inv;                    // n_log -> inverse transform (s = 1), last level carries n^-1
-    bool ntt_ct = true;                                 // B200ZKP_NTT_CT=0: every transform through ntt_kernels.cuh (A/B testing)
-    bool ntt_tma = true;                                // B200ZKP_NTT_TMA=0: the new passes stage their tiles with plain loads
     u32 ct_smem_set = 0;                                // kernels whose dynamic shared memory limit has been raised on this device
     u32 sm_count = 0;                                   // (queried on first use)
-    u64 coop_leaf_rows = 2048;                          // leaf sponges: the same switch (B200ZKP_COOP_LEAF_ROWS)
-    u64 coop_level_nodes = 2048;                        // tree levels of at most this many parents use the latency form (B200ZKP_COOP_LEVEL_NODES)
     // mailbox: 64 KB of mapped pinned host memory the small host-buffer calls (single hashes, the Fiat-Shamir transcript)
     // read and write directly from the kernel: no cudaMemcpy on those paths, one launch + one stream synchronise per call
     void* mailbox = nullptr;
@@ -489,7 +485,7 @@ static int run_ct_plan(b200zkp_ctx* ctx, ntc::Plan& plan, cudaStream_t later_str
         if (p.use_tma) {
             // the staged side of a coset loop has a single block; every other side walks the blocks of its buffer
             const bool loop = kind == ntc::KIND_STRIDED_LOOP || pull;
-            bool ok = ctx->ntt_tma && encode_tile_map(&tm_out, p.out, B, p.S, p.C_log, p.n_blk, p.out_blk_stride, map_cols, p.out_col_stride);
+            bool ok = encode_tile_map(&tm_out, p.out, B, p.S, p.C_log, p.n_blk, p.out_blk_stride, map_cols, p.out_col_stride);
             if (ok && pull) {
                 ok = encode_tile_map(&tm_copy, p.copy_out, B, p.S, p.C_log, 1, 0, map_cols, p.copy_col_stride);
                 // a source's matrix holds col_run local columns per group of col_period columns of the commitment
@@ -624,10 +620,6 @@ extern "C" int b200zkp_ctx_create(int device, void* stream, b200zkp_ctx** out) {
         }
         ctx->own_stream = true;
     }
-    if (const char* e = getenv("B200ZKP_NTT_CT")) ctx->ntt_ct = atoi(e) != 0;
-    if (const char* e = getenv("B200ZKP_NTT_TMA")) ctx->ntt_tma = atoi(e) != 0;
-    if (const char* e = getenv("B200ZKP_COOP_LEAF_ROWS")) { const long v = atol(e); if (v >= 0 && v <= (1 << 24)) ctx->coop_leaf_rows = (u64)v; }
-    if (const char* e = getenv("B200ZKP_COOP_LEVEL_NODES")) { const long v = atol(e); if (v >= 0 && v <= (1 << 20)) ctx->coop_level_nodes = (u64)v; }
     size_t mem_free = 0, mem_total = 0;
     if (cudaMemGetInfo(&mem_free, &mem_total) == cudaSuccess && mem_total) ctx->pool_max_bytes = mem_total / 8;
     else (void)cudaGetLastError();
@@ -728,17 +720,15 @@ extern "C" void b200zkp_host_free(void* p) { if (p) cudaFreeHost(p); }
 
 static int dev_intt_locked(b200zkp_ctx* ctx, const u64* values, u64 in_stride, u64* coeffs, u64 out_stride,
                            u64* scratch, u32 n_log, u32 k) {
-    if (ctx->ntt_ct && scratch && k) {
+    if (scratch && k && ntc::covers(n_log)) {
         // 2^11 points and more: block-twiddle passes (ntt_ct_kernels.cuh), natural order out through the scratch buffer
         b200zkp_ctx::ZTables z;
+        TRY(get_ztab_inv(ctx, n_log, &z));
         ntc::Plan plan;
-        if (ntc::covers(n_log)) {
-            TRY(get_ztab_inv(ctx, n_log, &z));
-            if (ntc::make_plan(&plan, values, in_stride, coeffs, out_stride, scratch, n_log, k, 1, 0, /*natural_out=*/true, z.strided,
-                               z.final_, hostgl::inv(((u64)1 << n_log) % hostgl::P), ctx->ntt_tma)) {
-                StageTimer tm(ctx, B200ZKP_STAGE_INTT);
-                return run_ct_plan(ctx, plan);
-            }
+        if (ntc::make_plan(&plan, values, in_stride, coeffs, out_stride, scratch, n_log, k, 1, 0, /*natural_out=*/true, z.strided,
+                           z.final_, hostgl::inv(((u64)1 << n_log) % hostgl::P), /*use_tma=*/true)) {
+            StageTimer tm(ctx, B200ZKP_STAGE_INTT);
+            return run_ct_plan(ctx, plan);
         }
     }
     StageTimer tm(ctx, B200ZKP_STAGE_INTT);
@@ -759,13 +749,13 @@ static int dev_lde_locked(b200zkp_ctx* ctx, const u64* coeffs, u64 coeff_stride,
     if (rate_bits > 8 || n_log + rate_bits > 32) BAD(ctx, "rate_bits / n_log out of range");
     if (b0 > b1 || b1 > (1u << rate_bits)) BAD(ctx, "bad coset block range");
     u64 n = (u64)1 << n_log;
-    if (ctx->ntt_ct && k && b1 > b0 && ntc::covers(n_log)) {
+    if (k && b1 > b0 && ntc::covers(n_log)) {
         // block-twiddle passes: the coset shift lives in the twiddles, the first pass stages a coefficient tile once for all blocks
         b200zkp_ctx::ZTables z;
         TRY(get_ztab_lde(ctx, n_log, rate_bits, &z));
         ntc::Plan plan;
         if (ntc::make_plan(&plan, coeffs, coeff_stride, lde, lde_stride, nullptr, n_log, k, b1 - b0, n, /*natural_out=*/false,
-                           z.strided + (u64)b0 * ntc::ztab_entries(n_log), z.final_ + (u64)b0 * ntc::zfinal_words(n_log), 0, ctx->ntt_tma)) {
+                           z.strided + (u64)b0 * ntc::ztab_entries(n_log), z.final_ + (u64)b0 * ntc::zfinal_words(n_log), 0, /*use_tma=*/true)) {
             StageTimer tm(ctx, B200ZKP_STAGE_LDE);
             return run_ct_plan(ctx, plan);
         }
@@ -788,12 +778,12 @@ static int dev_lde_cols_locked(b200zkp_ctx* ctx, const ntc::ColumnSet& cols, con
     if (rate_bits > 8 || n_log + rate_bits > 32) BAD(ctx, "rate_bits / n_log out of range");
     if (b0 >= b1 || b1 > (1u << rate_bits)) BAD(ctx, "bad coset block range");
     const u64 n = (u64)1 << n_log;
-    if (!ctx->ntt_ct || !ntc::covers(n_log)) return B200ZKP_ERR_UNSUPPORTED;
+    if (!ntc::covers(n_log)) return B200ZKP_ERR_UNSUPPORTED;
     b200zkp_ctx::ZTables z;
     TRY(get_ztab_lde(ctx, n_log, rate_bits, &z));
     ntc::Plan plan;
     if (!ntc::make_plan(&plan, coeffs, coeff_stride, lde, lde_stride, nullptr, n_log, 0, b1 - b0, n, /*natural_out=*/false,
-                        z.strided + (u64)b0 * ntc::ztab_entries(n_log), z.final_ + (u64)b0 * ntc::zfinal_words(n_log), 0, ctx->ntt_tma, &cols))
+                        z.strided + (u64)b0 * ntc::ztab_entries(n_log), z.final_ + (u64)b0 * ntc::zfinal_words(n_log), 0, /*use_tma=*/true, &cols))
         return B200ZKP_ERR_UNSUPPORTED;
     if (later_stream) return run_ct_plan(ctx, plan, later_stream, first_done, pull_ctas_per_sm);   // (the caller times the whole pipeline)
     StageTimer tm(ctx, B200ZKP_STAGE_LDE);
@@ -874,13 +864,15 @@ static unsigned hash_block_threads(u64 n_items) {
     return t;
 }
 
-static constexpr u64 COOP_MAX_NODES = 2048;   // below this the latency form of the permutation wins (merkle_kernels.cuh)
+// Leaf batches, tree levels and hash batches of at most this many items use the latency form of the permutation
+// (merkle_kernels.cuh), which wins while the work cannot fill the GPU; sweeps of both thresholds: profiles/r2z_*_sweep.log.
+static constexpr u64 COOP_MAX_NODES = 2048;
 
 static int launch_leaf_hash(b200zkp_ctx* ctx, const u64* leaves, u64 row_stride, u64 col_stride, u32 leaf_len, u64 row0,
                             u64 n_rows, const merkle::TreeShape& shape, u64* digests, u64* cap) {
     if (!n_rows) return 0;
     StageTimer tm(ctx, B200ZKP_STAGE_LEAF_HASH);
-    if (n_rows <= ctx->coop_leaf_rows) {
+    if (n_rows <= COOP_MAX_NODES) {
         merkle::leaf_hash_coop_kernel<<<(unsigned)((n_rows * 16 + 127) / 128), 128, 0, ctx->stream>>>(
             leaves, row_stride, col_stride, leaf_len, row0, n_rows, shape, digests, cap, 1u, ctx->round_add);
         LAUNCH_CHECK(ctx);
@@ -909,7 +901,7 @@ static int launch_tree_levels(b200zkp_ctx* ctx, u64 n_leaves, const merkle::Tree
             break;
         }
         u64 n_parents = n_leaves >> (layer + 1);
-        if (n_parents <= ctx->coop_level_nodes) {
+        if (n_parents <= COOP_MAX_NODES) {
             // too few nodes to fill the GPU: one node per 16 lanes, ~4x less latency per level
             merkle::merkle_level_coop_kernel<<<(unsigned)((n_parents * 16 + 127) / 128), 128, 0, ctx->stream>>>(
                 digests, cap, shape, layer, n_parents, ctx->round_add);

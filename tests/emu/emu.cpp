@@ -167,6 +167,20 @@ int emu_ct_lde_cols(const u64* const* src, u32 G, u32 w, u32 k, u32 col0, u32 co
     for (u32 pi = 0; pi < plan.n_passes; pi++) run_ct_pass(plan.pass[pi], plan.bits[pi], plan.kind[pi], plan.grid[pi]);
     return 1;
 }
+// the plan the library makes (use_tma asked for) for an inverse transform (natural_out) or an LDE of n_blk coset blocks with
+// columns out_stride apart, over 16-byte aligned buffers it never touches: -1 when make_plan refuses it, else bit pi set when
+// pass pi keeps TMA staging
+int emu_ct_plan_tma(u32 n_log, u32 k, u64 out_stride, u32 n_blk, int natural_out) {
+    alignas(16) static u64 in[2], out[2], scratch[2], ztab[2], zfinal[2];
+    const u64 n = (u64)1 << n_log;
+    ntc::Plan plan;
+    if (!ntc::make_plan(&plan, in, n, out, out_stride, natural_out ? scratch : nullptr, n_log, k, n_blk, natural_out ? 0 : n,
+                        natural_out != 0, ztab, zfinal, 0, true))
+        return -1;
+    int mask = 0;
+    for (u32 pi = 0; pi < plan.n_passes; pi++) if (plan.pass[pi].use_tma) mask |= 1 << pi;
+    return mask;
+}
 // row N1b: vanish::quotient_point stepped over every leaf of the quotient coset; LDEs [columns][Q] in leaf order,
 // gates: n_gates x (kind, selector_index, group_begin, group_end, p0, p1, p2); out [C][Q] natural order
 void emu_quotient_values(const u64* cs, const u64* wires, const u64* zpp, u32 n_log, u32 q_bits, u32 num_selectors, u32 C, u32 degree,

@@ -31,6 +31,7 @@ def emu():
     lib.emu_node_slot.restype = C.c_uint64
     lib.emu_node_slot.argtypes = [C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint64]
     lib.emu_sponge.argtypes = [u64p, C.c_uint64, C.c_uint32, C.c_uint32, u64p]
+    lib.emu_ct_plan_tma.argtypes = [C.c_uint32, C.c_uint32, C.c_uint64, C.c_uint32, C.c_int]
     return lib
 
 
@@ -135,6 +136,21 @@ def test_ct_pass_bodies(emu, oracle, n_log):
         perm = bitrev_perm(n_log + r)
         for c in range(k):
             assert (lde[c] == oracle.coset_lde(v[c], r)[perm][b0 * n:b1 * n]).all(), (r, b0, b1)
+
+
+@pytest.mark.parametrize("n_log", [11, 12, 13, 14, 15, 16, 17, 19, 20])
+def test_ct_plan_other_paths(emu, n_log):
+    """The plans test_gpu_parity.py::test_second_generation_passes counts on to reach the other transform paths on one
+    context: make_plan refuses an odd output column stride (the last pass moves pairs of elements), so b200zkp_dev_intt and
+    b200zkp_dev_lde fall back to the four-step kernels (ntt_kernels.cuh); and with 16 coset blocks the first pass reads the
+    one input block for every block (block stride 0), so it stages with plain loads while the other strided passes keep TMA."""
+    n, k = 1 << n_log, 2
+    strided = (1 << ((n_log + 7) // 8 - 1)) - 1          # every pass but the last (which never uses TMA)
+    assert emu.emu_ct_plan_tma(n_log, k, n, 1, 1) == strided
+    assert emu.emu_ct_plan_tma(n_log, k, n + 1, 1, 1) == -1
+    for nb in (1, 2, 8, 16):
+        assert emu.emu_ct_plan_tma(n_log, k, nb * n, nb, 0) == (strided & ~1 if nb == 16 else strided), nb
+        assert emu.emu_ct_plan_tma(n_log, k, nb * n + 1, nb, 0) == -1, nb
 
 
 def owned_columns(k, G, g):

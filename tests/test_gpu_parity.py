@@ -132,50 +132,54 @@ def test_transforms_three_and_four_passes(z, ctx, oracle, n_log):
 
 
 @pytest.mark.parametrize("n_log,k", [(11, 5), (12, 3), (13, 4), (14, 2), (15, 2), (16, 3), (17, 2), (19, 1), (20, 2)])
-def test_second_generation_passes(z, oracle, n_log, k, monkeypatch):
-    """ntt_ct_kernels.cuh (block-twiddle passes, TMA-staged tiles) against the oracle and against the first-generation
-    passes: inverse transform in natural order; coset LDE blocks in leaf order with the coset loop (2^r <= 8 blocks), without
-    it (16 blocks), with plain-load staging instead of TMA, and for a sub-range of the blocks (a multi-GPU rank's share)."""
+def test_second_generation_passes(z, ctx, oracle, n_log, k):
+    """ntt_ct_kernels.cuh (block-twiddle passes) against the oracle and against the four-step passes (ntt_kernels.cuh):
+    inverse transform in natural order; coset LDE blocks in leaf order with the coset loop (2^r <= 8 blocks), without it
+    (16 blocks: the first pass reads the one input block for every block, so make_plan stages it with plain loads instead of
+    TMA), and for a sub-range of the blocks (a multi-GPU rank's share).  The same calls into outputs with an odd column stride,
+    which the block-twiddle plans refuse (test_emu_kernels.py::test_ct_plan_other_paths), run the four-step kernels and must
+    give the same words.  Last, a whole commitment against the CPU references."""
     import ctypes as C
+    import os
     import torch
     rng = np.random.default_rng(500 + n_log)
     n = 1 << n_log
     v = rng.integers(0, 2**64, size=(k, n), dtype=np.uint64)
     v[0, :4] = [2**64 - 1, P, P - 1, 0]
-    ctxs = {}
-    for name, env in (("tma", {}), ("plain", {"B200ZKP_NTT_TMA": "0"}), ("gen1", {"B200ZKP_NTT_CT": "0"})):
-        for key in ("B200ZKP_NTT_TMA", "B200ZKP_NTT_CT"):
-            monkeypatch.delenv(key, raising=False)
-        for key, val in env.items():
-            monkeypatch.setenv(key, val)
-        ctxs[name] = z.Context(0)
-    want_c = np.stack([oracle.ifft(c) for c in v]) if n_log <= 17 else None
-    got = {name: z.ifft_batch(v, c) for name, c in ctxs.items()}
-    assert (got["tma"] == got["gen1"]).all() and (got["plain"] == got["gen1"]).all()
-    if want_c is not None:
-        assert (got["tma"] == want_c).all()
     vt = torch.from_numpy(v.view(np.int64)).cuda()
-    perm = None
+    scratch = torch.empty((k, n), dtype=torch.int64, device="cuda")
+    lib, p = ctx._lib, lambda t: C.c_void_p(t.data_ptr())
+
+    def run(call, width, stride):
+        out = torch.zeros((k, stride), dtype=torch.int64, device="cuda")
+        ctx.check(call(p(out), stride))
+        ctx.synchronize()
+        return out[:, :width].cpu().numpy().view(np.uint64)
+
+    intt = lambda out, stride: lib.b200zkp_dev_intt(ctx._h, p(vt), n, out, stride, p(scratch), n_log, k)
+    got = run(intt, n, n)
+    assert (got == np.stack([oracle.ifft(c) for c in v])).all()
+    assert (run(intt, n, n + 1) == got).all()
+    want = {}
     for r, b0, b1 in ((3, 0, 8), (3, 2, 4), (1, 0, 2), (4, 0, 16), (0, 0, 1)):
         if n_log >= 19 and r == 4:
             continue
-        outs = {}
-        for name, c in ctxs.items():
-            lde = torch.zeros((k, (b1 - b0) * n), dtype=torch.int64, device="cuda")
-            c.check(c._lib.b200zkp_dev_lde(c._h, C.c_void_p(vt.data_ptr()), n, C.c_void_p(lde.data_ptr()), (b1 - b0) * n, n_log, k, r, b0, b1))
-            c.synchronize()
-            outs[name] = lde.cpu().numpy().view(np.uint64)
-        assert (outs["tma"] == outs["gen1"]).all(), (r, b0, b1)
-        assert (outs["plain"] == outs["gen1"]).all(), (r, b0, b1)
-        if n_log <= 14:
+        if r not in want:
             perm = bitrev_perm(n_log + r)
-            for c in range(k):
-                assert (outs["tma"][c] == oracle.coset_lde(v[c], r)[perm][b0 * n:b1 * n]).all(), (r, b0, b1)
-    # a whole commitment through each generation
-    caps = {name: z.PolynomialBatch.from_values(v, 3, False, min(4, n_log), ctx=c).merkle_tree.cap.elements for name, c in ctxs.items()}
-    assert (caps["tma"] == caps["gen1"]).all() and (caps["plain"] == caps["gen1"]).all()
-    for c in ctxs.values():
-        c.close()
+            want[r] = np.stack([oracle.coset_lde(c, r)[perm] for c in v])
+        m = (b1 - b0) * n
+        lde = lambda out, stride: lib.b200zkp_dev_lde(ctx._h, p(vt), n, out, stride, n_log, k, r, b0, b1)
+        got = run(lde, m, m)
+        assert (got == want[r][:, b0 * n:b1 * n]).all(), (r, b0, b1)
+        assert (run(lde, m, m + 1) == got).all(), (r, b0, b1)
+    # a whole commitment: the single-threaded oracle up to 2^14 rows, the multithreaded CPU port above
+    cap = z.PolynomialBatch.from_values(v, 3, False, 4, ctx=ctx).merkle_tree.cap.elements
+    if n_log <= 14:
+        ref = oracle.commit(v, 3, 4)
+    else:
+        oracle.baseline_set_threads(len(os.sched_getaffinity(0)))
+        ref, _ = oracle.baseline_commit(v, 3, 4)
+    assert (cap == ref["cap"]).all()
 
 
 def test_transform_roundtrip_large(z, ctx):

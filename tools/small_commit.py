@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
-"""Device-resident commit latency of one small shape, median of 20 (tuning helper for the latency-form switches):
-    [B200ZKP_COOP_LEAF_ROWS=..] [B200ZKP_COOP_LEVEL_NODES=..] python tools/small_commit.py n_log k"""
+"""Device-resident commit latency of one small shape, median of 20:
+    python tools/small_commit.py n_log k"""
 import os
 import statistics
 import sys
@@ -21,5 +21,5 @@ for it in range(25):
     torch.cuda.synchronize()
     if it >= 5:
         ts.append(e0.elapsed_time(e1))
-print(f"2^{n_log} x {k}: {statistics.median(ts):.4f} ms (COOP_LEAF_ROWS={os.environ.get('B200ZKP_COOP_LEAF_ROWS', 'default')})")
+print(f"2^{n_log} x {k}: {statistics.median(ts):.4f} ms")
 ctx.close()
