@@ -302,9 +302,11 @@ int b200zkp_dev_partial_products_and_zs(b200zkp_ctx* ctx, const uint64_t* wires_
  * standard_recursion_config's 135 wires / 80 routed wires.  Gate types evaluated: NoopGate, ConstantGate (2 constants),
  * PublicInputGate, ArithmeticGate (20 ops), PoseidonGate, PoseidonMdsGate, BaseSumGate<B>, ArithmeticExtensionGate,
  * MulExtensionGate, ReducingGate, ReducingExtensionGate, RandomAccessGate, ExponentiationGate,
- * HighDegreeInterpolationGate, LowDegreeInterpolationGate; any other kind (the u32 / comparison gates, id 13) is
- * B200ZKP_ERR_UNSUPPORTED (not silently skipped).  The wire layouts are restated from memory of plonky2 @ f99ed9c
- * (parity unpinned, as for every gate here; DESIGN.md section 4d). */
+ * HighDegreeInterpolationGate, LowDegreeInterpolationGate, and plonky2_u32's U32ArithmeticGate, U32AddManyGate,
+ * U32SubtractionGate, U32RangeCheckGate and ComparisonGate (what circuits built with the reference's `ecdsa` feature add);
+ * any other kind (id 13, or a later plonky2_u32 gate) is B200ZKP_ERR_UNSUPPORTED (not silently skipped).  The wire layouts
+ * are restated from memory of plonky2 @ f99ed9c and the plonky2_u32 of that date (parity unpinned, as for every gate here;
+ * DESIGN.md section 4d). */
 enum { B200ZKP_GATE_NOOP = 0, B200ZKP_GATE_CONSTANT = 1, B200ZKP_GATE_PUBLIC_INPUT = 2, B200ZKP_GATE_ARITHMETIC = 3,
        B200ZKP_GATE_POSEIDON = 4,
        /* gates with parameters take them from gate_params[i] = { p0, p1, p2 } (Gate::new_from_config values in brackets) */
@@ -324,13 +326,41 @@ enum { B200ZKP_GATE_NOOP = 0, B200ZKP_GATE_CONSTANT = 1, B200ZKP_GATE_PUBLIC_INP
        B200ZKP_GATE_INTERPOLATION_HIGH_DEGREE = 14, /* HighDegreeInterpolationGate { subgroup_bits 1..5 }: constraints
         * value(i) - interpolant(shift g^i) for i < m, then eval_value - interpolant(eval_point), D components each:
         * D (m + 1) constraints, 5 + 4m wires, degree m (a FRI arity <= 8) */
-       B200ZKP_GATE_INTERPOLATION_LOW_DEGREE = 15 };  /* LowDegreeInterpolationGate { subgroup_bits 1..4 }: also
+       B200ZKP_GATE_INTERPOLATION_LOW_DEGREE = 15,   /* LowDegreeInterpolationGate { subgroup_bits 1..4 }: also
         * shift_pow(i) = wire end_coeffs + i - 2 and eval_pow(i) = ext(end_coeffs + m - 2 + D (i - 2)) for 2 <= i < m
         * (shift_pow(1) = shift, eval_pow(1) = eval_point).  Constraints: shift_pow(i-1) shift - shift_pow(i), 2 <= i < m;
         * value(i) - sum_j c_j shift_pow(j) g^(ij), i < m (shift_pow(0) = 1); eval_pow(i-1) eval_point - eval_pow(i),
         * 2 <= i < m; eval_value - (c_0 + sum_(i>=1) c_i eval_pow(i)): 5m - 4 constraints, 7m - 1 wires, degree 2 (what
         * standard_recursion_config's arity-16 FRI verifier instantiates, subgroup_bits 4) */
-#define B200ZKP_MAX_GATES 16
+       /* The plonky2_u32 gates.  "Limb range" is prod_{v < 4} (limb - v): limbs are 2 bits, combined little endian in base 4
+        * ("combined"); every count parameter is >= 1 and every gate reads at most 135 wires. */
+       B200ZKP_GATE_U32_ARITHMETIC = 16,  /* U32ArithmeticGate { num_ops } [3]: op i has m0 6i, m1 6i+1, addend 6i+2, lo 6i+3,
+        * hi 6i+4, inverse 6i+5, limb j < 32 at 6 num_ops + 32i + j.  Constraints per op: (inverse (2^32 - 1 - hi) - 1) lo
+        * (canonicity); hi 2^32 + lo - (m0 m1 + addend); the limb range of limb j for j = 31 down to 0; limbs j < 16 combined
+        * minus lo; limbs j >= 16 combined minus hi.  36 num_ops constraints, 38 num_ops wires, degree 4 */
+       B200ZKP_GATE_U32_ADD_MANY = 17,    /* U32AddManyGate { num_addends 1..16, num_ops } [e.g. 16, 3]: op i (a = num_addends)
+        * has addend j at (a+3)i + j, carry_in (a+3)i + a, result (a+3)i + a + 1, carry_out (a+3)i + a + 2, limb j < 18 at
+        * (a+3) num_ops + 18i + j (16 result limbs, then 2 carry limbs).  Constraints per op: carry_out 2^32 + result -
+        * (sum addends + carry_in); the limb range of limb j for j = 17 down to 0; result limbs combined minus result; carry
+        * limbs combined minus carry_out.  21 num_ops constraints, (a + 21) num_ops wires, degree 4 */
+       B200ZKP_GATE_U32_SUBTRACTION = 18, /* U32SubtractionGate { num_ops } [6]: op i has x 5i, y 5i+1, borrow_in 5i+2,
+        * result 5i+3, borrow_out 5i+4, limb j < 16 at 5 num_ops + 16i + j.  Constraints per op: result - (x - y - borrow_in
+        * + 2^32 borrow_out); the limb range of limb j for j = 15 down to 0; limbs combined minus result;
+        * borrow_out (1 - borrow_out).  19 num_ops constraints, 21 num_ops wires, degree 4 */
+       B200ZKP_GATE_U32_RANGE_CHECK = 19, /* U32RangeCheckGate { num_input_limbs }: input i at wire i, its limb j < 16 at
+        * num_input_limbs + 16i + j.  Constraints per input: its limbs combined minus the input, then the limb range of limb
+        * j for j = 0 up to 15.  17 num_input_limbs constraints and wires, degree 4 */
+       B200ZKP_GATE_COMPARISON = 20 };    /* ComparisonGate { num_bits 1..63, num_chunks 1..num_bits } [32, 16]: nc =
+        * num_chunks chunks of cb = ceil(num_bits / nc) <= 3 bits.  Wires: first input 0, second input 1, result 2, most
+        * significant diff (msd) 3, first chunk c at 4 + c, second chunk 4 + nc + c, equality dummy 4 + 2nc + c, chunks_equal
+        * 4 + 3nc + c, intermediate value 4 + 4nc + c, bit b <= cb of 2^cb + msd at 4 + 5nc + b.  Constraints: first chunks
+        * combined in base 2^cb minus first input; the same for the second; per chunk c (diff = second - first chunk):
+        * prod_{v < 2^cb} (first - v), the same for second, diff dummy - (1 - eq), eq diff, inter - eq so_far, after which
+        * so_far = inter + (1 - eq) diff (so_far starts at 0); msd - so_far; b (1 - b) for each bit, b = 0 up to cb;
+        * (2^cb + msd) - sum_b bit_b 2^b; result - bit_cb.  6 + 5nc + cb constraints, 5 + 5nc + cb wires, degree 2^cb */
+/* B200ZKP_MAX_GATES was 16 before the plonky2_u32 gates: an ecdsa circuit that also verifies a proof holds 20 kinds.  The
+ * layout of b200zkp_vanishing_desc changed with it; a caller compiled against the old header must be rebuilt. */
+#define B200ZKP_MAX_GATES 32
 typedef struct {
     uint32_t degree_bits;               /* n = 2^degree_bits rows */
     uint32_t quotient_degree_bits;      /* the quotient is evaluated on n << quotient_degree_bits points (<= rate_bits of the LDEs) */

@@ -2220,6 +2220,10 @@ extern "C" int b200zkp_dev_quotient_values(b200zkp_ctx* ctx, const b200zkp_vanis
             (kind == vanish::GATE_INTERPOLATION_LOW_DEGREE && (p0 == 0 || p0 > 4)) ||
             ((kind == vanish::GATE_REDUCING || kind == vanish::GATE_REDUCING_EXTENSION || kind == vanish::GATE_EXPONENTIATION) && (p0 == 0 || p0 > 128)) ||
             (kind == vanish::GATE_RANDOM_ACCESS && (p0 == 0 || p0 > 6 || p1 == 0 || p1 > 64 || p2 > 2)) ||
+            ((kind == vanish::GATE_U32_ARITHMETIC || kind == vanish::GATE_U32_SUBTRACTION || kind == vanish::GATE_U32_RANGE_CHECK) &&
+             (p0 == 0 || p0 > 135)) ||
+            (kind == vanish::GATE_U32_ADD_MANY && (p0 == 0 || p0 > 16 || p1 == 0 || p1 > 135)) ||
+            (kind == vanish::GATE_COMPARISON && (p0 == 0 || p0 > 63 || p1 == 0 || p1 > p0 || vanish::comparison_chunk_bits(p0, p1) > 3)) ||
             vanish::gate_num_wires(kind, R, p0, p1, p2) > 135)
             BAD(ctx, "gate parameters out of range for 135 wires");
         if (d->gate_selector_index[i] >= d->num_selectors || d->gate_group_begin[i] > i || d->gate_group_end[i] <= i ||

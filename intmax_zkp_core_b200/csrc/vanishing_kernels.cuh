@@ -37,10 +37,15 @@ enum GateKind : u32 {
     GATE_POSEIDON_MDS = 12,          // 12 extension inputs, 12 extension outputs
     // (13 is not assigned)
     GATE_INTERPOLATION_HIGH_DEGREE = 14,   // params (subgroup_bits): m = 2^subgroup_bits points, degree m
-    GATE_INTERPOLATION_LOW_DEGREE = 15     // params (subgroup_bits): the same with power wires, degree 2
+    GATE_INTERPOLATION_LOW_DEGREE = 15,    // params (subgroup_bits): the same with power wires, degree 2
+    GATE_U32_ARITHMETIC = 16,        // params (num_ops): lo + 2^32 hi = m0 m1 + addend, 32 two-bit limbs per op
+    GATE_U32_ADD_MANY = 17,          // params (num_addends, num_ops): result + 2^32 carry_out = sum + carry_in, 18 limbs per op
+    GATE_U32_SUBTRACTION = 18,       // params (num_ops): result = x - y - borrow_in + 2^32 borrow_out, 16 limbs per op
+    GATE_U32_RANGE_CHECK = 19,       // params (num_input_limbs): 16 two-bit limbs per input
+    GATE_COMPARISON = 20             // params (num_bits, num_chunks): result = first <= second, degree 2^chunk_bits
 };
 static constexpr u32 D = 2;          // quadratic extension F[X] / (X^2 - 7)
-static constexpr u32 MAX_GATES = 16, MAX_CHALLENGES = 4;
+static constexpr u32 MAX_GATES = 32, MAX_CHALLENGES = 4;
 static constexpr u32 UNUSED_SELECTOR = 0xFFFFFFFFu;
 // PoseidonGate wire layout (gates/poseidon.rs)
 static constexpr u32 W_IN = 0, W_OUT = 12, W_SWAP = 24, W_DELTA = 25, W_FULL0 = 29, W_PARTIAL = 65, W_FULL1 = 87;
@@ -50,10 +55,21 @@ static constexpr u32 W_IN = 0, W_OUT = 12, W_SWAP = 24, W_DELTA = 25, W_FULL0 = 
 // to end_coeffs = 5 + 4 m; LowDegree only: shift^i at end_coeffs + i - 2 and ext eval_point^i at end_coeffs + m - 2 + D (i - 2)
 // for 2 <= i < m
 
+// plonky2_u32 layouts (gates/*_u32.rs, comparison.rs; include/b200zkp.h states them with their constraint order).  Limbs are 2
+// bits, combined little endian in base 4.  U32Arithmetic op i: m0 6i, m1 6i+1, addend 6i+2, lo 6i+3, hi 6i+4, inverse 6i+5,
+// limb j at 6 num_ops + 32i + j.  U32AddMany (a addends) op i: addend j (a+3)i + j, carry_in (a+3)i + a, result +1, carry_out
+// +2, limb j at (a+3) num_ops + 18i + j (16 result limbs, 2 carry limbs).  U32Subtraction op i: x 5i, y 5i+1, borrow_in 5i+2,
+// result 5i+3, borrow_out 5i+4, limb j at 5 num_ops + 16i + j.  U32RangeCheck: input i at i, its limb j at num_input_limbs +
+// 16i + j.  Comparison (nc chunks of cb = ceil(num_bits / nc) bits): first 0, second 1, result 2, most-significant diff 3,
+// first chunk c 4 + c, second chunk 4 + nc + c, equality dummy 4 + 2nc + c, chunks_equal 4 + 3nc + c, intermediate 4 + 4nc + c,
+// bit b <= cb of 2^cb + msd at 4 + 5nc + b
+static constexpr u32 U32_LIMBS_PER_WORD = 16;
+GL_HD u32 comparison_chunk_bits(u32 num_bits, u32 num_chunks) { return num_chunks ? (num_bits + num_chunks - 1) / num_chunks : 0; }
+
 struct GateDesc { u32 kind, selector_index, group_begin, group_end, p0, p1, p2; };
 
 GL_HD bool gate_supported(u32 kind) {
-    return kind <= GATE_POSEIDON_MDS || kind == GATE_INTERPOLATION_HIGH_DEGREE || kind == GATE_INTERPOLATION_LOW_DEGREE;
+    return kind <= GATE_POSEIDON_MDS || (kind >= GATE_INTERPOLATION_HIGH_DEGREE && kind <= GATE_COMPARISON);
 }
 
 // Gate::num_constraints() of standard_recursion_config instances (host and device)
@@ -72,6 +88,11 @@ GL_HD u32 gate_num_constraints(u32 kind, u32 num_routed, u32 num_gate_consts, u3
         case GATE_POSEIDON_MDS: return 12 * D;
         case GATE_INTERPOLATION_HIGH_DEGREE: return D * ((1u << p0) + 1);
         case GATE_INTERPOLATION_LOW_DEGREE: return 5 * (1u << p0) - 4;
+        case GATE_U32_ARITHMETIC: return 36 * p0;
+        case GATE_U32_ADD_MANY: return 21 * p1;
+        case GATE_U32_SUBTRACTION: return 19 * p0;
+        case GATE_U32_RANGE_CHECK: return 17 * p0;
+        case GATE_COMPARISON: return 6 + 5 * p1 + comparison_chunk_bits(p0, p1);
         default: return 0;
     }
 }
@@ -87,6 +108,11 @@ GL_HD u32 gate_num_wires(u32 kind, u32 num_routed, u32 p0, u32 p1, u32 p2) {
         case GATE_POSEIDON: return 135;
         case GATE_INTERPOLATION_HIGH_DEGREE: return 5 + 4 * (1u << p0);
         case GATE_INTERPOLATION_LOW_DEGREE: return 7 * (1u << p0) - 1;
+        case GATE_U32_ARITHMETIC: return 38 * p0;
+        case GATE_U32_ADD_MANY: return (p0 + 21) * p1;
+        case GATE_U32_SUBTRACTION: return 21 * p0;
+        case GATE_U32_RANGE_CHECK: return 17 * p0;
+        case GATE_COMPARISON: return 5 + 5 * p1 + comparison_chunk_bits(p0, p1);
         default: return num_routed;
     }
 }
@@ -157,6 +183,9 @@ GL_FN u64 root_of_unity(u32 bits) {
     for (u32 k = bits; k < 32; k++) g = gl::mul(g, g);
     return g;
 }
+
+// prod_{v < 4} (x - v): the range check of a two-bit limb
+GL_FN u64 limb_range(u64 x) { return gl::mul(gl::mul(x, gl::sub(x, 1)), gl::mul(gl::sub(x, 2), gl::sub(x, 3))); }
 
 // running sums of one gate's constraints, one per challenge
 struct Fold {
@@ -481,6 +510,101 @@ GL_FN void quotient_point(const Params& p, u64 t) {
                 }
                 const E2 r = e2_sub(ext(3 + D * m), v);
                 f.add(r.a); f.add(r.b);
+                break;
+            }
+            case GATE_U32_ARITHMETIC:
+            case GATE_U32_ADD_MANY:
+            case GATE_U32_SUBTRACTION: {                              // plonky2_u32 gates/{arithmetic,add_many,subtraction}_u32.rs
+                // per op: the word equation (U32Arithmetic: the canonicity check first), the range of every limb from the top
+                // one down, the limbs below 16 combined minus the low word, then the limbs above minus the high word
+                // (U32Subtraction: borrow_out is a bit instead).  Limbs are read where they are used, never held.
+                const u32 kind = gd.kind, a = gd.p0;
+                const u32 ops = kind == GATE_U32_ADD_MANY ? gd.p1 : gd.p0;
+                const u32 per = kind == GATE_U32_ARITHMETIC ? 6 : kind == GATE_U32_ADD_MANY ? a + 3 : 5;
+                const u32 limbs = kind == GATE_U32_ARITHMETIC ? 2 * U32_LIMBS_PER_WORD : kind == GATE_U32_ADD_MANY ? U32_LIMBS_PER_WORD + 2 : U32_LIMBS_PER_WORD;
+                const u64 two32 = (u64)1 << 32;
+#pragma unroll 1
+                for (u32 op = 0; op < ops; op++) {
+                    const u32 w0 = per * op, l0 = per * ops + limbs * op;
+                    u64 lo, hi;
+                    if (kind == GATE_U32_ARITHMETIC) {
+                        lo = wire(w0 + 3); hi = wire(w0 + 4);
+                        f.add(gl::mul(gl::sub(gl::mul(wire(w0 + 5), gl::sub(0xFFFFFFFFull, hi)), 1), lo));
+                        f.add(gl::sub(gl::add(gl::mul(hi, two32), lo), gl::add(gl::mul(wire(w0), wire(w0 + 1)), wire(w0 + 2))));
+                    } else if (kind == GATE_U32_ADD_MANY) {
+                        lo = wire(w0 + a + 1); hi = wire(w0 + a + 2);
+                        u64 sum = wire(w0 + a);
+#pragma unroll 1
+                        for (u32 j = 0; j < a; j++) sum = gl::add(sum, wire(w0 + j));
+                        f.add(gl::sub(gl::add(gl::mul(hi, two32), lo), sum));
+                    } else {
+                        lo = wire(w0 + 3); hi = wire(w0 + 4);
+                        f.add(gl::sub(lo, gl::add(gl::sub(gl::sub(wire(w0), wire(w0 + 1)), wire(w0 + 2)), gl::mul(hi, two32))));
+                    }
+                    u64 comb_lo = 0, comb_hi = 0;
+#pragma unroll 1
+                    for (u32 j = limbs; j-- > 0;) {
+                        const u64 l = wire(l0 + j);
+                        f.add(limb_range(l));
+                        if (j < U32_LIMBS_PER_WORD) comb_lo = gl::add(gl::mul(comb_lo, 4), l);
+                        else comb_hi = gl::add(gl::mul(comb_hi, 4), l);
+                    }
+                    f.add(gl::sub(comb_lo, lo));
+                    f.add(kind == GATE_U32_SUBTRACTION ? gl::mul(hi, gl::sub(1, hi)) : gl::sub(comb_hi, hi));
+                }
+                break;
+            }
+            case GATE_U32_RANGE_CHECK: {                              // plonky2_u32 gates/range_check_u32.rs
+                const u32 nl = gd.p0;
+#pragma unroll 1
+                for (u32 q = 0; q < nl; q++) {
+                    const u32 l0 = nl + U32_LIMBS_PER_WORD * q;
+                    u64 comb = 0;
+#pragma unroll 1
+                    for (u32 j = U32_LIMBS_PER_WORD; j-- > 0;) comb = gl::add(gl::mul(comb, 4), wire(l0 + j));
+                    f.add(gl::sub(comb, wire(q)));
+#pragma unroll 1
+                    for (u32 j = 0; j < U32_LIMBS_PER_WORD; j++) f.add(limb_range(wire(l0 + j)));
+                }
+                break;
+            }
+            case GATE_COMPARISON: {                                   // plonky2_u32 gates/comparison.rs
+                const u32 nc = gd.p1, cb = comparison_chunk_bits(gd.p0, gd.p1);
+                const u64 chunk_size = (u64)1 << cb;
+                u64 first = 0, second = 0;
+#pragma unroll 1
+                for (u32 c = nc; c-- > 0;) {
+                    first = gl::add(gl::mul(first, chunk_size), wire(4 + c));
+                    second = gl::add(gl::mul(second, chunk_size), wire(4 + nc + c));
+                }
+                f.add(gl::sub(first, wire(0)));
+                f.add(gl::sub(second, wire(1)));
+                u64 msd = 0;                                          // the most significant difference so far
+#pragma unroll 1
+                for (u32 c = 0; c < nc; c++) {
+                    const u64 x = wire(4 + c), y = wire(4 + nc + c);
+                    u64 px = 1, py = 1;
+#pragma unroll 1
+                    for (u64 v = 0; v < chunk_size; v++) { px = gl::mul(px, gl::sub(x, v)); py = gl::mul(py, gl::sub(y, v)); }
+                    f.add(px);
+                    f.add(py);
+                    const u64 diff = gl::sub(y, x), eq = wire(4 + 3 * nc + c), inter = wire(4 + 4 * nc + c);
+                    f.add(gl::sub(gl::mul(diff, wire(4 + 2 * nc + c)), gl::sub(1, eq)));
+                    f.add(gl::mul(eq, diff));
+                    f.add(gl::sub(inter, gl::mul(eq, msd)));
+                    msd = gl::add(inter, gl::mul(gl::sub(1, eq), diff));
+                }
+                const u64 msd_wire = wire(3);
+                f.add(gl::sub(msd_wire, msd));
+                u64 bits = 0;
+#pragma unroll 1
+                for (u32 b = 0; b <= cb; b++) {
+                    const u64 bit = wire(4 + 5 * nc + b);
+                    f.add(gl::mul(bit, gl::sub(1, bit)));
+                    bits = gl::add(bits, gl::mul(bit, (u64)1 << b));
+                }
+                f.add(gl::sub(gl::add(chunk_size, msd_wire), bits));
+                f.add(gl::sub(wire(2), wire(4 + 5 * nc + cb)));
                 break;
             }
             default: break;

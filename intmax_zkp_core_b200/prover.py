@@ -176,7 +176,8 @@ GATE_NOOP, GATE_CONSTANT, GATE_PUBLIC_INPUT, GATE_ARITHMETIC, GATE_POSEIDON = ra
 (GATE_ARITHMETIC_EXTENSION, GATE_MUL_EXTENSION, GATE_BASE_SUM, GATE_REDUCING, GATE_REDUCING_EXTENSION, GATE_RANDOM_ACCESS,
  GATE_EXPONENTIATION, GATE_POSEIDON_MDS) = range(5, 13)
 GATE_INTERPOLATION_HIGH_DEGREE, GATE_INTERPOLATION_LOW_DEGREE = 14, 15         # (13 is not assigned)
-MAX_GATES = 16
+GATE_U32_ARITHMETIC, GATE_U32_ADD_MANY, GATE_U32_SUBTRACTION, GATE_U32_RANGE_CHECK, GATE_COMPARISON = range(16, 21)
+MAX_GATES = 32
 
 
 class _VanishingDesc(C.Structure):
@@ -196,8 +197,11 @@ class CommonCircuitData:
     gates: [(kind, selector_index, (group_begin, group_end)[, params]), ...]; params: the gate's own parameters
     (BaseSum (B, num_limbs), Reducing / ReducingExtension (num_coeffs,), RandomAccess (bits, num_copies, num_extra_constants),
     Exponentiation (num_power_bits,), HighDegreeInterpolation (subgroup_bits,) with subgroup_bits 1..5,
-    LowDegreeInterpolation (subgroup_bits,) with subgroup_bits 1..4).  The u32 and comparison gates are refused
-    (B200ZkpError with code -4); the interpolation layouts are restated from memory as for the other gates (include/b200zkp.h)"""
+    LowDegreeInterpolation (subgroup_bits,) with subgroup_bits 1..4, and plonky2_u32's U32Arithmetic (num_ops,),
+    U32AddMany (num_addends, num_ops) with num_addends 1..16, U32Subtraction (num_ops,), U32RangeCheck (num_input_limbs,),
+    Comparison (num_bits, num_chunks) with num_bits 1..63 and chunks of at most 3 bits).  Parameters out of range, or a gate
+    reading more than 135 wires, are B200ZkpError with code -1; a kind the device does not evaluate (13) has code -4.  At
+    most MAX_GATES gates.  The layouts are restated from memory as for the other gates (include/b200zkp.h)"""
 
     def __init__(self, degree_bits: int, gates, num_selectors: int, quotient_degree_factor: int = 8, num_routed_wires: int = 80,
                  k_is=None):

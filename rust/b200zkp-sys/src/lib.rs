@@ -12,7 +12,7 @@ use std::os::raw::{c_char, c_int, c_void};
 
 pub const B200ZKP_COMM_ID_BYTES: usize = 128;
 pub const B200ZKP_SALT_SIZE: u32 = 4; // plonky2 fri/oracle.rs SALT_SIZE
-pub const B200ZKP_MAX_GATES: usize = 16;
+pub const B200ZKP_MAX_GATES: usize = 32; // 16 before the plonky2_u32 gates (b200zkp_vanishing_desc layout changed)
 /// gate kinds of `b200zkp_vanishing_desc::gate_kind` (include/b200zkp.h B200ZKP_GATE_*); parameters in `gate_params`
 pub const B200ZKP_GATE_NOOP: u32 = 0;
 pub const B200ZKP_GATE_CONSTANT: u32 = 1;
@@ -30,6 +30,12 @@ pub const B200ZKP_GATE_POSEIDON_MDS: u32 = 12;
 // 13 is not assigned
 pub const B200ZKP_GATE_INTERPOLATION_HIGH_DEGREE: u32 = 14;
 pub const B200ZKP_GATE_INTERPOLATION_LOW_DEGREE: u32 = 15;
+// plonky2_u32 / plonky2_ecdsa gates
+pub const B200ZKP_GATE_U32_ARITHMETIC: u32 = 16; // { num_ops }
+pub const B200ZKP_GATE_U32_ADD_MANY: u32 = 17; // { num_addends, num_ops }
+pub const B200ZKP_GATE_U32_SUBTRACTION: u32 = 18; // { num_ops }
+pub const B200ZKP_GATE_U32_RANGE_CHECK: u32 = 19; // { num_input_limbs }
+pub const B200ZKP_GATE_COMPARISON: u32 = 20; // { num_bits, num_chunks }
 
 /// include/b200zkp.h `b200zkp_vanishing_desc` (row N1b: what compute_quotient_polys reads of CommonCircuitData)
 #[repr(C)]

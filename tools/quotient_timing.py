@@ -2,11 +2,13 @@
 """Row N1b timing: compute_quotient_values_device (vanish::quotient_values_kernel plus its small table upload) on random
 device-resident LDEs, 2 challenges, quotient_degree_factor 8, for two gate sets:
   five       Noop / Constant / PublicInput / Arithmetic / Poseidon, the set bench.py's prove_chain_latency uses;
-  recursion  the 14 gates of a standard_recursion_config verifier circuit (the 13 other kinds + LowDegreeInterpolation(4)).
+  recursion  the 14 gates of a standard_recursion_config verifier circuit (the 13 other kinds + LowDegreeInterpolation(4));
+  ecdsa      those 14 plus the plonky2_u32 gates of a circuit built with the ecdsa feature (U32AddMany at two arities): 20.
 The kernel's work does not depend on the values, so the matrices are random.  CUDA events, median of --reps calls after
 --warmup calls; one JSON line per (set, size), with the card's name and power limit.  B200ZKP_LIB selects another build of the
-library, so two builds can be timed alternately in one session (a build that refuses a gate set reports it as unsupported).
-GPU only.   python tools/quotient_timing.py [--sizes 12 14 16] [--sets five recursion] [--label NAME]"""
+library of the same `b200zkp_vanishing_desc` layout, so two builds can be timed alternately in one session (a build that
+refuses a gate set reports it as unsupported).
+GPU only.   python tools/quotient_timing.py [--sizes 12 14 16] [--sets five recursion ecdsa] [--label NAME]"""
 import argparse
 import json
 import os
@@ -33,7 +35,15 @@ def gate_sets():
     groups = [(0, 6), (6, 11), (11, 13), (13, 14)]
     selector = [0] * 6 + [1] * 5 + [2] * 2 + [3]
     rec = [(k, s, groups[s], pr) for (k, pr), s in zip(kinds, selector)]
-    return {"five": (five, 2), "recursion": (rec, len(groups))}
+    # tests/u32_ref.py's ecdsa_circuit: the degree-4 u32 gates after ExponentiationGate; degrees 0 1 1 1 2 2 | 2 2 3 3 3 |
+    # 4 4 4 4 | 4 4 4 | 5 | 7
+    u32 = [(zp.GATE_U32_ARITHMETIC, (3,)), (zp.GATE_U32_ADD_MANY, (3, 5)), (zp.GATE_U32_ADD_MANY, (16, 3)),
+           (zp.GATE_U32_SUBTRACTION, (6,)), (zp.GATE_U32_RANGE_CHECK, (4,)), (zp.GATE_COMPARISON, (32, 16))]
+    kinds = kinds[:12] + u32 + kinds[12:]
+    groups = [(0, 6), (6, 11), (11, 15), (15, 18), (18, 19), (19, 20)]
+    selector = [0] * 6 + [1] * 5 + [2] * 4 + [3] * 3 + [4, 5]
+    ecdsa = [(k, s, groups[s], pr) for (k, pr), s in zip(kinds, selector)]
+    return {"five": (five, 2), "recursion": (rec, 4), "ecdsa": (ecdsa, len(groups))}
 
 
 def card():
